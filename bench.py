@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""bench.py — the judged benchmark of the B200 signal path (contract in the task prompt).
+"""bench.py — the benchmark of the B200 signal path: one JSON result line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload at N=1 = BASELINE.json configs[1] ("c2"): 256 streams x 1080p, CHROM_GREEN ROI sampling,
 [DETREND_LINEAR, FILTER_FIR], Welch HR, W=300, T=64 frames per stream resident in HBM per step (102 GB of the
@@ -14,9 +14,11 @@ N>1: every rank owns S streams (weak scaling, no data-path collective); the 24-b
 all-gathered over NCCL inside the timed region, one step behind the compute (bpv.dist.RecordGather).
 
 `--impl reference` times the UNMODIFIED reference (`baseline/_ref`, a git-ignored copy of the reference's own
-modules made by `__graft_entry__.build()` in the build container; it travels to the GPU box with the snapshot):
+modules that `__graft_entry__.build()` makes where the upstream project is checked out at `__graft_entry__.REFERENCE`):
 `SignalProcessor.process` per frame, one process per host core, one stream each.  The oracle port
 (`oracle/bpv_oracle.py`) is the fallback when that copy is missing, and is reported beside it.
+
+`--dump-outputs DIR` writes what the last timed step returned (`dump_outputs`), for comparing two builds output for output.
 """
 from __future__ import annotations
 
@@ -63,6 +65,9 @@ OTHER_SHAPES = {
                desc='configs[4]: 65536 streams x 10 s windows over all GPUs, ROI -> Butterworth -> Lomb-Scargle -> HR -> PTT + NCCL record gather'),
 }
 METRIC, UNIT = 'roi_sampled_frames_per_s', 'frames/s'
+# --dump-outputs: the StepResult fields a caller of BatchedSignalProcessor.step receives
+DUMP_FIELDS = ('samples', 'peak_freq', 'peak_idx', 'peak_mag', 'lag_sec', 'lag_idx', 'lag_corr', 'status')
+DUMP_MAX_BYTES = 64 << 20
 # dram__bytes_read.sum + dram__bytes_write.sum of one c2 F1 launch of 16 384 frames (ncu --set full; profiles/r2y_c2_summary.md:
 # 664.3 + 4.0 and 664.4 + 5.9 MB for the two captured launches, same boxes); 337.2 MB for the 8192-frame launch of round 1
 ROI_NCU_TRAFFIC_BYTES = 669.3e6
@@ -551,6 +556,30 @@ def run_latency_c1(torch, dev, frames_n=60):
             'how': 'drop-in SignalProcessor.process (S=1 engine, store_arrays=True): host BGR frame in, deep-copied SignalStore out'}
 
 
+def dump_outputs(res, out_dir):
+    """Write the StepResult `res` as out_dir/<field>.npy, float64 (the int32 bins and status convert exactly).  The inputs
+    of a run are fixed by its arguments, so two builds of the project run with the same arguments compare file for file.
+    Every file holds finite values: the path reports "none" as NaN (a missed detection or a box outside the frame gives a
+    NaN ROI sample, a window without a peak NaN bpm), so each floating-point field is written with its non-finite entries
+    as 0 beside <field>_nonfinite.npy, which holds 1 where the value was NaN, 2 for +inf, 3 for -inf and 0 elsewhere.
+    All of it is written: at c2 it is 2.8 MB, and the frames in HBM bound any shape far below DUMP_MAX_BYTES."""
+    arrays = {}
+    for k in DUMP_FIELDS:
+        t = getattr(res, k)
+        a = t.double().cpu().numpy()
+        if t.is_floating_point():
+            bad = ~np.isfinite(a)
+            arrays[f'{k}_nonfinite'] = np.select([np.isnan(a), a > 0], [1.0, 2.0], 3.0) * bad
+            a = np.where(bad, 0.0, a)
+        arrays[k] = a
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError(f'--dump-outputs: {total} bytes of outputs, more than {DUMP_MAX_BYTES}')
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f'{k}.npy'), a)
+
+
 def run_gpu(args, wl):
     import torch
     from bpv import _cabi, dist as bdist, synth
@@ -626,6 +655,8 @@ def run_gpu(args, wl):
     barrier()
     for k, fn in orig.items():
         setattr(ops, k, fn)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(res, args.dump_outputs)              # before the profile pass below reuses the result buffers
     ms = start.elapsed_time(stop)
     launches_per_step = eng.launches_per_step + 1            # of the timed steps: the engine's own count + pack_records32
     clk = clocks.stop() if rank == 0 else None
@@ -888,7 +919,7 @@ def _shutdown():
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=200)
+    ap.add_argument('--steps', type=int, default=200, help='timed steps (>= 1)')
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--impl', default='bpv', choices=['bpv', 'reference'])
     ap.add_argument('--workload', default='c2', choices=list(WORKLOADS))
@@ -902,7 +933,13 @@ def main():
     ap.add_argument('--bind-numa', dest='numa', action='store_true', help='N > 1: bind each rank to the CPUs of its GPU\'s NUMA node')
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-other', action='store_true', help='skip the other_shapes / latency blocks')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the results of the last timed step as DIR/<name>.npy '
+                                                          '(rank 0\'s streams when N > 1)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'bpv':
+        ap.error('--dump-outputs writes the results of the GPU path (--impl bpv)')
     wl = dict(WORKLOADS[args.workload])
     if args.frames_per_step > 0:
         wl['T'] = args.frames_per_step

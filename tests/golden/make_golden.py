@@ -1,5 +1,5 @@
-"""Generate golden vectors by running the UNMODIFIED reference (`/root/reference`) in the build
-container.  Run:  python tests/golden/make_golden.py   (writes tests/golden/*.npz)
+"""Generate golden vectors by running the UNMODIFIED reference, the checkout of the upstream bp-from-video project at
+__graft_entry__.REFERENCE.  Run:  python tests/golden/make_golden.py   (writes tests/golden/*.npz)
 
 The reference has no tests/golden vectors of its own, so these fixtures are the parity pin for
 `oracle/bpv_oracle.py` (tests/test_oracle_golden.py demands exact equality) and, through the
@@ -17,8 +17,6 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, os.path.join(ROOT, 'bp-from-video_b200'))
 from bpv import synth  # noqa: E402
-
-REF = '/root/reference'
 
 
 def load_reference():
@@ -89,7 +87,7 @@ def sig_arrays(group):
 
 
 sys.path.insert(0, ROOT)
-from tests.helpers import CASES, LIVE_CASES, SEEDS, IMG_H as H, IMG_W as W  # noqa: E402  (single source of the case tables)
+from tests.helpers import CASES, LIVE_CASES, SEEDS, IMG_H as H, IMG_W as W, REFERENCE as REF  # noqa: E402  (single source of the case tables)
 
 
 
@@ -143,6 +141,8 @@ def roi_case(sp, seed=7):
 
 def main():
     warnings.simplefilter('ignore')
+    if not os.path.isdir(REF):
+        sys.exit(f'no checkout of the upstream bp-from-video project at {REF}')
     sp = load_reference()
     if len(sys.argv) == 3 and sys.argv[1] == '--live':     # the non-committed differential cases, into a scratch directory
         for k, name in enumerate(LIVE_CASES):

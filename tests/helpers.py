@@ -3,9 +3,11 @@ import os
 
 import numpy as np
 
+from __graft_entry__ import REFERENCE   # the upstream checkout build() stages from; live-reference tests skip without it
 from oracle import bpv_oracle as orc
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
+NO_REFERENCE = f'no checkout of the reference at {REFERENCE}'
 METHOD = dict(DIFF_1=orc.DIFF_1, DIFF_2=orc.DIFF_2, INTERP_LINEAR=orc.INTERP_LINEAR, INTERP_CUBIC=orc.INTERP_CUBIC,
               DETREND_CONST=orc.DETREND_CONST, DETREND_LINEAR=orc.DETREND_LINEAR, FILTER_BUTTER=orc.FILTER_BUTTER,
               FILTER_FIR=orc.FILTER_FIR)
@@ -39,7 +41,7 @@ CASES.update({
 SEEDS = {name: 100 + k for k, name in enumerate(list(CASES)[:10])}
 SEEDS.update(diff1_butter4_welch=500, cubic_lin_fir31_ls=501, const_dft_smooth3=502, lin_diff2_butter8_ls=503)
 # cases that are NOT committed as fixtures: tests/test_oracle_golden.py::test_live_differential_vs_reference runs the
-# reference on them in a subprocess (build container only) and demands exact equality with the oracle, so the pin does
+# reference on them in a subprocess (where REFERENCE exists) and demands exact equality with the oracle, so the pin does
 # not rest on the frozen files alone
 LIVE_CASES = {
     'live_diff2_butter2_dft':       ('GREEN', ['DIFF_2', 'FILTER_BUTTER'], 'DFT_RFFT', 38, 54, 30, True, 0.03, 1, dict(butter_order=2)),

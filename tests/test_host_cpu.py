@@ -12,7 +12,7 @@ from oracle import bpv_oracle as orc
 from tests import helpers as h
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = '/root/reference'
+REF = h.REFERENCE
 
 
 def test_cabi_exports_every_declared_symbol():
@@ -124,7 +124,7 @@ def _eq(a, b):
     return a.shape == b.shape and np.array_equal(a, b, equal_nan=True)
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason='reference not mounted (GPU box)')
+@pytest.mark.skipif(not os.path.isdir(REF), reason=h.NO_REFERENCE)
 def test_signal_data_differential_vs_reference():
     """Random operation sequences on our Signal/SignalGroup and the reference's must agree on everything."""
     import warnings
@@ -221,14 +221,14 @@ def test_signal_processor_surface_matches_reference_signature():
     pickle.loads(pickle.dumps(st.snapshot()))
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason='reference not mounted (GPU box)')
+@pytest.mark.skipif(not os.path.isdir(REF), reason=h.NO_REFERENCE)
 def test_reference_modules_import_on_top_of_the_drop_in():
     """PYTHONPATH=<ours>:<reference>: the reference's own video_reader must import against OUR profiler/exceptions,
     and `signal_processor` / `roi` / `signal_data` must resolve to the drop-in (INTEGRATION.md §1)."""
     import subprocess
     code = ("import sys, video_reader, signal_processor, roi, signal_data, profiler, exceptions;"
             "assert 'bp-from-video_b200' in signal_processor.__file__ and 'bp-from-video_b200' in roi.__file__;"
-            "assert 'bp-from-video_b200' in profiler.__file__ and video_reader.__file__.startswith('/root/reference');"
+            f"assert 'bp-from-video_b200' in profiler.__file__ and video_reader.__file__.startswith({REF!r});"
             "assert issubclass(exceptions.CaptureError, RuntimeError);"
             "p = signal_processor.SignalProcessor(); assert p.num_signals == 2 and p.store.sg_corr.num_signals == 1;"
             "print('ok')")

@@ -14,7 +14,7 @@ def test_process_matches_reference(name):
     _replay(h.CASES[name], h.load_case(name), name)
 
 
-@pytest.mark.skipif(not os.path.exists('/root/reference'), reason='reference not mounted (GPU box)')
+@pytest.mark.skipif(not os.path.isdir(h.REFERENCE), reason=h.NO_REFERENCE)
 def test_live_differential_vs_reference(tmp_path):
     """Beyond the frozen fixtures: run the UNMODIFIED reference now, in a subprocess, on cases that are not committed
     (other method chains, filter orders, tap counts, frame rates, ROI smoothing lengths) and demand exact equality."""
