@@ -23,7 +23,17 @@ Overlap (`overlap`, bit mask; default from the environment variable BPV_OVERLAP,
   2  F4 (cross-correlation) runs on a side stream beside F3 (spectrum): both only read the processed windows
   4  F3 + F4 as ONE grid of interleaved Welch / xcorr CTAs (PGRAM_WELCH, windows up to 320 samples, >= 2 ROIs; takes precedence
      over 2 where it applies).  Measured SLOWER than bit 2 (profiles/r4g: 272.9 against 227.5 us for the pair, step 0.7255 against
-     0.6840 ms) although the two kernels are bound by different things: not in the default mask, kept as a measurement switch
+     0.6840 ms) although the two kernels are bound by different things: not in the default mask, kept as a measurement switch.
+     It has no band-limited peak search: with `freq_band` or `lag_band` set, the step runs the two kernels of bit 2 instead.
+
+Peak search ranges (`freq_band`, `lag_band`; default None).  process() searches the heart-rate peak over EVERY spectrum bin
+and the PTT lag over EVERY correlation lag: SignalGroup resets the ranges that transform_signal / correlate_signal_pair set
+(signal_processor.py:272, 294; signal_data.py:82-86), and None keeps that behaviour bit for bit.  A (lo, hi) pair limits the
+search as Signal.get_peak(lo, hi) does (signal_data.py:65-70): the peak is the first maximum over the bins (lags) whose
+reported frequency in Hz (lag in seconds) lies in [lo, hi]; fewer than two such entries give no peak (NaN, index -1).  The
+ranges the reference configures are freq_band=(min_freq, max_freq) and lag_band=(-0.5, 0.5).  Spectra, correlations and
+the stored arrays do not depend on the bands; peak_idx / lag_idx still index the full arrays, and the running means and
+packed records take the band-limited peaks.  Both are plain attributes: assign a new pair (or None) between steps.
 """
 from __future__ import annotations
 
@@ -81,7 +91,8 @@ class BatchedSignalProcessor:
                  fir_taps: int = 127, fir_df: float = 0.3, min_freq: float = 0.8, max_freq: float = 4.0,
                  ls_num_freqs: int | None = None, windows: str = EVERY_FRAME, store_arrays: bool = False,
                  device: str | torch.device = 'cuda', roi_pixels_hint: int = 0, peak_max_samples: int = 0,
-                 result_buffers: int = 2, overlap: int | None = None, design_cache: bool | None = None):
+                 result_buffers: int = 2, overlap: int | None = None, design_cache: bool | None = None,
+                 freq_band: tuple[float, float] | None = None, lag_band: tuple[float, float] | None = None):
         _cabi.lib()  # fail loudly if the CUDA library is missing: there is no CPU fallback
         if not torch.cuda.is_available():
             raise _cabi.BpvError('BatchedSignalProcessor needs a CUDA device (no CPU fallback)')
@@ -101,6 +112,9 @@ class BatchedSignalProcessor:
         self.kw = dict(butter_order=butter_order, butter_min_bw=butter_min_bw, fir_taps=fir_taps, fir_df=fir_df,
                        min_freq=min_freq, max_freq=max_freq, ls_num_freqs=int(ls_num_freqs or 0))
         self.windows, self.store_arrays = windows, bool(store_arrays)
+        # peak search ranges (module docstring): None = every bin / lag, as process()
+        self.freq_band = ops.peak_band(freq_band, 'freq_band')
+        self.lag_band = ops.peak_band(lag_band, 'lag_band')
         self.roi_pixels_hint = int(roi_pixels_hint)
         self.device = torch.device(device)
         if self.device.type != 'cuda':
@@ -323,7 +337,9 @@ class BatchedSignalProcessor:
         spo = None if spo is None or spo['peak_idx'].shape[0] != J else spo
         xco = None if xco is None or xco['lag_idx'].shape[0] != J else xco
         # (windows over 320 samples: the entry point itself runs the two stand-alone launches, on this stream)
-        fused = bool(self.overlap & OVERLAP_FUSED) and self.P > 0 and self.transform == _cabi.PGRAM_WELCH
+        fb, lb = ops.peak_band(self.freq_band, 'freq_band'), ops.peak_band(self.lag_band, 'lag_band')
+        fused = (bool(self.overlap & OVERLAP_FUSED) and self.P > 0 and self.transform == _cabi.PGRAM_WELCH
+                 and fb is None and lb is None)       # the fused grid has no band: two kernels instead
         if fused:
             sp, xc = ops.window_welch_xcorr(px, py, p, store=self.store_arrays, out_spectrum=spo, out_xcorr=xco)
         elif (self.overlap & OVERLAP_XCORR) and self.P:
@@ -336,16 +352,16 @@ class BatchedSignalProcessor:
             side.wait_event(ev['pre'])
             xc_first = os.environ.get('BPV_XC_FIRST', '') == '1'
             if not xc_first:
-                sp = ops.window_spectrum(px, py, p, store=self.store_arrays, workspace=self._ws_spec, out=spo)
+                sp = ops.window_spectrum(px, py, p, store=self.store_arrays, workspace=self._ws_spec, out=spo, band=fb)
             with torch.cuda.stream(side):
-                xc = ops.window_xcorr(px, py, p, store=self.store_arrays, out=xco)
+                xc = ops.window_xcorr(px, py, p, store=self.store_arrays, out=xco, band=lb)
                 ev['xc'].record(side)
             if xc_first:
-                sp = ops.window_spectrum(px, py, p, store=self.store_arrays, workspace=self._ws_spec, out=spo)
+                sp = ops.window_spectrum(px, py, p, store=self.store_arrays, workspace=self._ws_spec, out=spo, band=fb)
             main.wait_event(ev['xc'])
         else:
-            sp = ops.window_spectrum(px, py, p, store=self.store_arrays, workspace=self._ws_spec, out=spo)
-            xc = ops.window_xcorr(px, py, p, store=self.store_arrays, out=xco)
+            sp = ops.window_spectrum(px, py, p, store=self.store_arrays, workspace=self._ws_spec, out=spo, band=fb)
+            xc = ops.window_xcorr(px, py, p, store=self.store_arrays, out=xco, band=lb)
         self._spec[turn], self._xc[turn] = sp, xc
         if not self.store_arrays and self.discard_scratch:
             # the processed windows are dead now: drop their dirty L2 lines instead of letting the next step's ROI sampling

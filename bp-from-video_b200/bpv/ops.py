@@ -246,9 +246,27 @@ def window_welch_xcorr(proc_x, proc_y, p: WindowParams, store: bool = True, out_
     return sp, xc
 
 
-def window_spectrum(proc_x, proc_y, p: WindowParams, store: bool = True, out=None, workspace=None):
+def peak_band(band, name: str = 'band'):
+    """None, or (lo, hi) as two floats: the search range of a band-limited peak (Signal.get_peak(lo, hi), signal_data.py:65-70).
+    Infinite bounds are allowed and lo > hi gives no peak, as get_peak does; NaN bounds are rejected."""
+    if band is None:
+        return None
+    try:
+        lo, hi = (float(v) for v in band)
+    except (TypeError, ValueError):
+        raise ValueError(f'{name} must be None or a (lo, hi) pair of numbers, not {band!r}') from None
+    if lo != lo or hi != hi:
+        raise ValueError(f'{name} has a NaN bound: {band!r}')
+    return lo, hi
+
+
+def window_spectrum(proc_x, proc_y, p: WindowParams, store: bool = True, out=None, workspace=None, band=None):
     """F3 + HR peak (signal_processor.py:248-277, 310).  Returns dict(freqs, mags f32 [J,R,max_bins] | None,
-    num_bins i32, peak_idx i32, peak_freq f64, peak_mag f64 [J,R])."""
+    num_bins i32, peak_idx i32, peak_freq f64, peak_mag f64 [J,R]).
+    band = (min_freq, max_freq): the peak is the first maximum over the bins whose frequency lies in the band, as a single
+    transform_signal(s).get_peak() finds it (include/bpv.h bpv_window_spectrum_band); the spectrum itself does not change.
+    None searches every bin, as process() does."""
+    band = peak_band(band)
     dev = proc_y.device
     mb = max_bins(p)
     o = _spectrum_out(p, store, out, dev)
@@ -258,19 +276,30 @@ def window_spectrum(proc_x, proc_y, p: WindowParams, store: bool = True, out=Non
     need = lib().bpv_spectrum_workspace_bytes(C.byref(p), mb) if (not store or p.transform == _cabi.DFT_RFFT) else 0
     if need and (workspace is None or workspace.numel() < need):
         workspace = torch.zeros(need, dtype=torch.uint8, device=dev)
-    _run(proc_y.device, 'bpv_window_spectrum', ptr(proc_x), ptr(proc_y), C.byref(p), mb, ptr(workspace) if need else None, need,
-                                    ptr(o['freqs']), ptr(o['mags']),
-                                    ptr(o['num_bins']), ptr(o['peak_idx']), ptr(o['peak_freq']), ptr(o['peak_mag']))
+    args = (ptr(proc_x), ptr(proc_y), C.byref(p), mb, ptr(workspace) if need else None, need, ptr(o['freqs']), ptr(o['mags']),
+            ptr(o['num_bins']), ptr(o['peak_idx']), ptr(o['peak_freq']), ptr(o['peak_mag']))
+    if band is None:
+        _run(proc_y.device, 'bpv_window_spectrum', *args)
+    else:
+        _run(proc_y.device, 'bpv_window_spectrum_band', *args, *band)
     return o
 
 
-def window_xcorr(proc_x, proc_y, p: WindowParams, store: bool = True, out=None):
-    """F4 pairwise xcorr + lag peak (signal_processor.py:280-299, 312)."""
+def window_xcorr(proc_x, proc_y, p: WindowParams, store: bool = True, out=None, band=None):
+    """F4 pairwise xcorr + lag peak (signal_processor.py:280-299, 312).
+    band = (min_lag, max_lag) in seconds: the peak is the first maximum over the lags inside the band, as a single
+    correlate_signal_pair(a, b).get_peak() finds it (include/bpv.h bpv_window_xcorr_band); the correlation does not change.
+    None searches every lag, as process() does."""
+    band = peak_band(band)
     P = p.R * (p.R - 1) // 2
     o = _xcorr_out(p, store, out, proc_y.device)
     if P > 0:
-        _run(proc_y.device, 'bpv_window_xcorr', ptr(proc_x), ptr(proc_y), C.byref(p), ptr(o['lags']), ptr(o['corr']),
-                                     ptr(o['num_lags']), ptr(o['lag_idx']), ptr(o['lag_sec']), ptr(o['lag_corr']))
+        args = (ptr(proc_x), ptr(proc_y), C.byref(p), ptr(o['lags']), ptr(o['corr']), ptr(o['num_lags']), ptr(o['lag_idx']),
+                ptr(o['lag_sec']), ptr(o['lag_corr']))
+        if band is None:
+            _run(proc_y.device, 'bpv_window_xcorr', *args)
+        else:
+            _run(proc_y.device, 'bpv_window_xcorr_band', *args, *band)
     return o
 
 

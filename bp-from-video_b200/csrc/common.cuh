@@ -31,6 +31,16 @@ inline int check_launch(const char* what) {
 
 __device__ __forceinline__ double nan_f64() { return __longlong_as_double(0x7ff8000000000000LL); }
 
+// Search range of a peak: Signal.get_peak(min_x, max_x) (signal_data.py:65-70) with explicit bounds.  A bin or lag is
+// eligible iff lo <= x <= hi for the float64 x the kernel reports for it.  The peak kernels take it as a template switch
+// BAND: the BAND = false instantiations are the unbanded search of process() and never read the bounds.
+struct PeakBand {
+  double lo, hi;
+  __device__ __forceinline__ bool in(double x) const { return lo <= x && x <= hi; }
+};
+// (-inf, +inf) selects the unbanded kernels; the entry points reject NaN bounds before calling this
+inline bool band_limits(double lo, double hi) { return !(lo == -INFINITY && hi == INFINITY); }
+
 template <typename T>
 __device__ __forceinline__ T warp_sum(T v) {
 #pragma unroll

@@ -386,12 +386,15 @@ __global__ void __launch_bounds__(DTC_THREADS, 1) dft_tc_kernel(const double* __
   tc_teardown(tmem);
 }
 
-// warp per signal; smem: double2 tw[W] shared by the CTA's warps
+// warp per signal; smem: double2 tw[W] shared by the CTA's warps.
+// BAND: the peak is searched over the bins with band.lo <= k * fval <= band.hi; their fp32 maximum and count are taken over those
+// bins alone.  The float64 values written back into the spectrum are those of the unbanded candidates, whatever the band.
+template <bool BAND>
 __global__ void __launch_bounds__(128) dft_peak_kernel(const double* __restrict__ proc_x, const double* __restrict__ proc_y, int W,
                                                        long long nsig, int max_bins, float* __restrict__ spec_f,
                                                        float* __restrict__ mags, int32_t* __restrict__ num_bins,
                                                        int32_t* __restrict__ peak_idx, double* __restrict__ peak_freq,
-                                                       double* __restrict__ peak_mag) {
+                                                       double* __restrict__ peak_mag, const PeakBand band) {
   extern __shared__ __align__(16) uint8_t psm[];
   double2* tw = reinterpret_cast<double2*>(psm);
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
@@ -423,21 +426,31 @@ __global__ void __launch_bounds__(128) dft_peak_kernel(const double* __restrict_
   const double fval = 1.0 / ((double)n * (1.0 / fs));      // rfftfreq(n, d=1/fs)[k] = k * (1/(n*d))
   float* row = mags + sig * max_bins;
   float cmax = -INFINITY; int cnt = 0;
+  float bmax = -INFINITY; int cb = 0;                      // BAND: over the finite in-band bins
   for (int k = lane; k < F; k += 32) {
     const float v = row[k];
-    if (isfinite(v)) { ++cnt; cmax = fmaxf(cmax, v); }
+    if (isfinite(v)) { ++cnt; cmax = fmaxf(cmax, v); if (BAND && band.in((double)k * fval)) { ++cb; bmax = fmaxf(bmax, v); } }
     if (spec_f) spec_f[sig * max_bins + k] = (float)((double)k * fval);
   }
   for (int o = 16; o > 0; o >>= 1) { cmax = fmaxf(cmax, __shfl_xor_sync(0xffffffffu, cmax, o)); cnt += __shfl_xor_sync(0xffffffffu, cnt, o); }
+  if (BAND)
+    for (int o = 16; o > 0; o >>= 1) { bmax = fmaxf(bmax, __shfl_xor_sync(0xffffffffu, bmax, o)); cb += __shfl_xor_sync(0xffffffffu, cb, o); }
   const float thr = cmax - DFT_TC_BAND * fabsf(cmax);
+  const float thr_b = bmax - DFT_TC_BAND * fabsf(bmax);
   double best = -INFINITY; int bi = 0x7fffffff;
   for (int kk0 = 0; kk0 < F; kk0 += 32) {
     const int k = kk0 + lane;
-    bool cand = false;
-    if (k < F) { const float v = row[k]; cand = cnt >= 2 ? (isfinite(v) && v >= thr) : true; }
-    unsigned mk = __ballot_sync(0xffffffffu, cand);
+    bool cand = false, cand_b = false;
+    if (k < F) {
+      const float v = row[k];
+      cand = cnt >= 2 ? (isfinite(v) && v >= thr) : true;
+      if (BAND) cand_b = band.in((double)k * fval) && (cb >= 2 ? (isfinite(v) && v >= thr_b) : true);
+    }
+    // BAND: mw = bins whose float64 value is written back (the unbanded candidates), mb = in-band candidates
+    unsigned mk = __ballot_sync(0xffffffffu, cand || cand_b);
+    const unsigned mw = BAND ? __ballot_sync(0xffffffffu, cand) : 0u, mb = BAND ? __ballot_sync(0xffffffffu, cand_b) : 0u;
     while (mk) {
-      const int kc = kk0 + __ffs(mk) - 1;
+      const int b = __ffs(mk) - 1, kc = kk0 + b;
       mk &= mk - 1;
       double re = 0.0, im = 0.0;
       int idx = (int)(((long long)lane * kc) % n);
@@ -450,13 +463,13 @@ __global__ void __launch_bounds__(128) dft_peak_kernel(const double* __restrict_
       }
       re = warp_sum(re); im = warp_sum(im);
       const double mg = 2.0 * hypot(re, im) / (double)n;
-      if (lane == 0) row[kc] = (float)mg;
-      if (isfinite(mg) && (mg > best || (mg == best && kc < bi))) { best = mg; bi = kc; }
+      if (lane == 0 && (!BAND || ((mw >> b) & 1u))) row[kc] = (float)mg;
+      if ((!BAND || ((mb >> b) & 1u)) && isfinite(mg) && (mg > best || (mg == best && kc < bi))) { best = mg; bi = kc; }
     }
   }
   if (lane == 0) {
     num_bins[sig] = F;
-    if (cnt >= 2 && bi != 0x7fffffff) { peak_idx[sig] = bi; peak_freq[sig] = (double)bi * fval; peak_mag[sig] = best; }
+    if ((BAND ? cb : cnt) >= 2 && bi != 0x7fffffff) { peak_idx[sig] = bi; peak_freq[sig] = (double)bi * fval; peak_mag[sig] = best; }
     else { peak_idx[sig] = -1; peak_freq[sig] = nan_f64(); peak_mag[sig] = nan_f64(); }
   }
 }
@@ -872,9 +885,9 @@ long long dft_tc_image_bytes(int W) { return dtc_image_bytes(W); }
 // kernel, or NULL for the kernel that generates its operands itself.  BPV_DFT_TMA=0 forces the latter (measurement switch).
 int launch_dft_tc(const double* proc_x, const double* proc_y, int W, long long nsig, int max_bins, float* spec_f, float* mags,
                   int32_t* num_bins, int32_t* peak_idx, double* peak_freq, double* peak_mag, void* image_ws, void* split_ws,
-                  cudaStream_t st) {
+                  bool banded, PeakBand band, cudaStream_t st) {
   const int smem = dtc_smem(W), smem_p = W * 16;
-  if (int rc = ensure_dyn_smem((const void*)dft_peak_kernel, smem_p)) return rc;
+  if (int rc = ensure_dyn_smem(banded ? (const void*)dft_peak_kernel<true> : (const void*)dft_peak_kernel<false>, smem_p)) return rc;
   const int F = W / 2 + 1;
   dim3 grid((unsigned)((nsig + TC_M - 1) / TC_M), (unsigned)((F + 127) / 128));
   const char* env = getenv("BPV_DFT_TMA");
@@ -928,8 +941,12 @@ int launch_dft_tc(const double* proc_x, const double* proc_y, int W, long long n
     dft_tc_kernel<<<grid, DTC_THREADS, smem, st>>>(proc_y, W, nsig, max_bins, mags, num_bins);
     if (int rc = check_launch("dft_tc_kernel")) return rc;
   }
-  dft_peak_kernel<<<(unsigned)((nsig + 3) / 4), 128, smem_p, st>>>(proc_x, proc_y, W, nsig, max_bins, spec_f, mags, num_bins, peak_idx,
-                                                                 peak_freq, peak_mag);
+  if (banded)
+    dft_peak_kernel<true><<<(unsigned)((nsig + 3) / 4), 128, smem_p, st>>>(proc_x, proc_y, W, nsig, max_bins, spec_f, mags, num_bins,
+                                                                           peak_idx, peak_freq, peak_mag, band);
+  else
+    dft_peak_kernel<false><<<(unsigned)((nsig + 3) / 4), 128, smem_p, st>>>(proc_x, proc_y, W, nsig, max_bins, spec_f, mags, num_bins,
+                                                                            peak_idx, peak_freq, peak_mag, band);
   return check_launch("dft_peak_kernel");
 }
 

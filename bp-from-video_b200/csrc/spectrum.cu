@@ -22,7 +22,7 @@ long long dft_tc_image_bytes(int W);
 long long dft_tc_split_bytes(int W, long long nsig);
 int launch_dft_tc(const double* proc_x, const double* proc_y, int W, long long nsig, int max_bins, float* spec_f, float* mags,
                   int32_t* num_bins, int32_t* peak_idx, double* peak_freq, double* peak_mag, void* image_ws, void* split_ws,
-                  cudaStream_t st);
+                  bool banded, PeakBand band, cudaStream_t st);
 
 constexpr float LS_DELTA = 1.0e-4f;     // candidate band below the fp32 maximum (PSD is in [0, 1])
 constexpr int LS_SMALL_N = 24;          // below this every bin is evaluated in float64
@@ -70,14 +70,15 @@ __device__ SigInfo gather_signal(const double* __restrict__ px, const double* __
 }
 
 // Block argmax with numpy's first-max rule over finite values; also counts finite entries.
-// vals in shared/global memory (double).  Result broadcast through smem.
+// vals in shared/global memory (double).  Result broadcast through smem.  BAND: only bins with band.lo <= k * fval <= band.hi.
 struct Peak { int idx; double val; int nfinite; };
-__device__ Peak block_argmax(const double* vals, int F, double* s_val, int* s_idx) {
+template <bool BAND>
+__device__ Peak block_argmax(const double* vals, int F, double* s_val, int* s_idx, double fval, const PeakBand band) {
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5, nw = (blockDim.x + 31) >> 5;
   double bv = -INFINITY; int bi = 0x7fffffff, cnt = 0;
   for (int k = tid; k < F; k += blockDim.x) {
     const double v = vals[k];
-    if (isfinite(v)) { ++cnt; if (v > bv || (v == bv && k < bi)) { bv = v; bi = k; } }
+    if (isfinite(v) && (!BAND || band.in((double)k * fval))) { ++cnt; if (v > bv || (v == bv && k < bi)) { bv = v; bi = k; } }
   }
   for (int o = 16; o > 0; o >>= 1) {
     const double ov = __shfl_xor_sync(0xffffffffu, bv, o);
@@ -105,12 +106,14 @@ __device__ Peak block_argmax(const double* vals, int F, double* s_val, int* s_id
 // DFT_RFFT and PGRAM_WELCH: one CTA per signal.
 // smem doubles: ys[W] | tw_c[N] | tw_s[N] | z[N] | mags[F]   (N = n or nperseg <= W, F <= W/2+1)
 // ---------------------------------------------------------------------------------------------
+template <bool BAND>
 __global__ void __launch_bounds__(128) spectrum_dense_kernel(const double* __restrict__ proc_x,
                                                              const double* __restrict__ proc_y,
                                                              const bpv_window_params p, int max_bins, int only_flagged,
                                                              float* __restrict__ spec_f, float* __restrict__ spec_mag,
                                                              int32_t* __restrict__ num_bins, int32_t* __restrict__ peak_idx,
-                                                             double* __restrict__ peak_freq, double* __restrict__ peak_mag) {
+                                                             double* __restrict__ peak_freq, double* __restrict__ peak_mag,
+                                                             const PeakBand band) {
   extern __shared__ __align__(16) double sm[];
   __shared__ int s_cnt[4];
   if (only_flagged && num_bins[blockIdx.x] != -2) return;   // second pass behind dft_tc_kernel (CTA uniform)
@@ -229,7 +232,7 @@ __global__ void __launch_bounds__(128) spectrum_dense_kernel(const double* __res
       spec_mag[sig * max_bins + k] = (float)mags[k];
     }
   }
-  const Peak pk = block_argmax(mags, F, s_val, s_idx);
+  const Peak pk = block_argmax<BAND>(mags, F, s_val, s_idx, fval, band);
   if (tid == 0) {
     num_bins[sig] = F;
     if (pk.nfinite >= 2) { peak_idx[sig] = pk.idx; peak_freq[sig] = (double)pk.idx * fval; peak_mag[sig] = pk.val; }
@@ -238,14 +241,17 @@ __global__ void __launch_bounds__(128) spectrum_dense_kernel(const double* __res
 }
 
 // PGRAM_WELCH: the warp-per-signal kernel lives in welch.cuh (welch_warp_body)
+template <bool BAND>
 __global__ void __launch_bounds__(32 * WELCH_WPB, WELCH_MINB) welch_warp_kernel(const double* __restrict__ proc_x,
                                                                     const double* __restrict__ proc_y,
                                                                     const bpv_window_params p, int max_bins, long long nsig,
                                                                     int only_flagged, float* __restrict__ spec_f, float* __restrict__ spec_mag,
                                                                     int32_t* __restrict__ num_bins, int32_t* __restrict__ peak_idx,
-                                                                    double* __restrict__ peak_freq, double* __restrict__ peak_mag) {
+                                                                    double* __restrict__ peak_freq, double* __restrict__ peak_mag,
+                                                                    const PeakBand band) {
   extern __shared__ __align__(16) double sm[];
-  welch_warp_body(blockIdx.x, sm, proc_x, proc_y, p, max_bins, nsig, only_flagged, spec_f, spec_mag, num_bins, peak_idx, peak_freq, peak_mag);
+  welch_warp_body<BAND>(blockIdx.x, sm, proc_x, proc_y, p, max_bins, nsig, only_flagged, spec_f, spec_mag, num_bins, peak_idx, peak_freq,
+                        peak_mag, band);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -403,11 +409,18 @@ __global__ void __launch_bounds__(128) ls_coarse_kernel(const double* __restrict
 
 // Peak pass: one CTA (128 threads) per signal.  smem doubles: ts[W] | ys[W] | cand_val[max_bins];
 // ints: cand_idx[max_bins].
+// BAND: the peak is searched over the bins with band.lo <= ls_freq(k) <= band.hi.  Their fp32 maximum and count are taken over
+// those bins alone (an out-of-band maximum would set a threshold that excludes every in-band bin).  The bins re-evaluated for the
+// unbanded search are still the ones whose float64 values are written back, so the stored spectrum does not depend on the band:
+// a candidate carries bit 30 (write back) and bit 29 (in-band candidate) above its bin index.
+template <bool BAND>
 __global__ void __launch_bounds__(128) ls_peak_kernel(const double* __restrict__ proc_x, const double* __restrict__ proc_y,
                                                       const bpv_window_params p, int max_bins,
                                                       float* __restrict__ spec_f, float* __restrict__ psd,
                                                       int32_t* __restrict__ num_bins, int32_t* __restrict__ peak_idx,
-                                                      double* __restrict__ peak_freq, double* __restrict__ peak_mag) {
+                                                      double* __restrict__ peak_freq, double* __restrict__ peak_mag,
+                                                      const PeakBand band) {
+  constexpr int WB = 1 << 30, CB = 1 << 29, KM = CB - 1;
   extern __shared__ __align__(16) double sm[];
   __shared__ int s_cnt[4];
   __shared__ double s_d[2];
@@ -428,15 +441,28 @@ __global__ void __launch_bounds__(128) ls_peak_kernel(const double* __restrict__
   }
   const int F = p.ls_num_freqs > 0 ? p.ls_num_freqs : n;
   float* row = psd + sig * max_bins;
-  // fp32 maximum over finite bins
+  // fp32 maximum over finite bins (BAND: also over the finite in-band bins, bb / cb)
   float bv = -INFINITY; int cnt = 0;
-  for (int k = tid; k < F; k += blockDim.x) { const float v = row[k]; if (isfinite(v)) { ++cnt; bv = fmaxf(bv, v); } }
+  float bb = -INFINITY; int cb = 0;
+  for (int k = tid; k < F; k += blockDim.x) {
+    const float v = row[k];
+    if (isfinite(v)) {
+      ++cnt; bv = fmaxf(bv, v);
+      if (BAND && band.in(ls_freq(k, F, p.min_freq, p.max_freq))) { ++cb; bb = fmaxf(bb, v); }
+    }
+  }
   for (int o = 16; o > 0; o >>= 1) { bv = fmaxf(bv, __shfl_xor_sync(0xffffffffu, bv, o)); cnt += __shfl_xor_sync(0xffffffffu, cnt, o); }
-  if (lane == 0) { s_val[wid] = bv; s_idx[wid] = cnt; }
+  if (BAND)
+    for (int o = 16; o > 0; o >>= 1) { bb = fmaxf(bb, __shfl_xor_sync(0xffffffffu, bb, o)); cb += __shfl_xor_sync(0xffffffffu, cb, o); }
+  if (lane == 0) { s_val[wid] = bv; s_idx[wid] = cnt; if (BAND) { s_val[16 + wid] = bb; s_idx[16 + wid] = cb; } }
   if (tid == 0) s_nc = 0;
   __syncthreads();
   bv = s_val[0]; cnt = s_idx[0];
   for (int w2 = 1; w2 < nw; ++w2) { bv = fmaxf(bv, s_val[w2]); cnt += s_idx[w2]; }
+  if (BAND) {
+    bb = s_val[16]; cb = s_idx[16];
+    for (int w2 = 1; w2 < nw; ++w2) { bb = fmaxf(bb, s_val[16 + w2]); cb += s_idx[16 + w2]; }
+  }
   __syncthreads();
   // moments for the float64 evaluation (relative time; Y, YY as scipy Eq. 7 / 10)
   const double t0 = xs[0];
@@ -455,32 +481,37 @@ __global__ void __launch_bounds__(128) ls_peak_kernel(const double* __restrict__
   __syncthreads();
   // candidate list: every bin for small problems, else bins within LS_DELTA of the fp32 maximum
   const bool all = n < LS_SMALL_N || cnt < 2;
+  const bool all_b = BAND ? (n < LS_SMALL_N || cb < 2) : all;
   for (int k = tid; k < F; k += blockDim.x) {
     const float v = row[k];
-    if (all || (isfinite(v) && v >= bv - LS_DELTA)) cidx[atomicAdd(&s_nc, 1)] = k;
+    const bool cw = all || (isfinite(v) && v >= bv - LS_DELTA);
+    bool cbd = false;
+    if (BAND) cbd = band.in(ls_freq(k, F, p.min_freq, p.max_freq)) && (all_b || (isfinite(v) && v >= bb - LS_DELTA));
+    if (cw || cbd) cidx[atomicAdd(&s_nc, 1)] = BAND ? (k | (cw ? WB : 0) | (cbd ? CB : 0)) : k;
   }
   __syncthreads();
   const int nc = s_nc;
   for (int c = wid; c < nc; c += nw) {
-    const int k = cidx[c];
+    const int k = BAND ? (cidx[c] & KM) : cidx[c];
     const double v = ls_eval_f64(xs, ys, n, ls_freq(k, F, p.min_freq, p.max_freq), Y, YY);
-    if (lane == 0) { cval[c] = v; row[k] = (float)v; }
+    if (lane == 0) { cval[c] = v; if (!BAND || (cidx[c] & WB)) row[k] = (float)v; }
   }
   __syncthreads();
-  if (all && tid == 0) {   // recount finite bins from the float64 values
+  if (all_b && tid == 0) {   // recount finite bins from the float64 values
     int c2 = 0;
-    for (int c = 0; c < nc; ++c) c2 += isfinite(cval[c]);
+    for (int c = 0; c < nc; ++c) c2 += isfinite(cval[c]) && (!BAND || (cidx[c] & CB));
     s_idx[0] = c2;
   }
   __syncthreads();
-  const int nfinite = all ? s_idx[0] : cnt;
+  const int nfinite = all_b ? s_idx[0] : (BAND ? cb : cnt);
   __syncthreads();
   // first-max rule in float64 over the candidates (ties -> smallest bin index)
   double best = -INFINITY; int bi = 0x7fffffff;
   if (tid == 0) {
     for (int c = 0; c < nc; ++c) {
       const double v = cval[c];
-      if (isfinite(v) && (v > best || (v == best && cidx[c] < bi))) { best = v; bi = cidx[c]; }
+      const int k = BAND ? (cidx[c] & KM) : cidx[c];
+      if ((!BAND || (cidx[c] & CB)) && isfinite(v) && (v > best || (v == best && k < bi))) { best = v; bi = k; }
     }
     num_bins[sig] = F;
     if (nfinite >= 2 && bi != 0x7fffffff) {
@@ -494,13 +525,15 @@ __global__ void __launch_bounds__(128) ls_peak_kernel(const double* __restrict__
 
 // Warp-per-signal version of the Lomb-Scargle peak pass (default): the CTA-per-signal kernel above spends most of its time
 // in __syncthreads between short phases (gather, three block reductions, candidate list); here every phase is warp-local.
-// smem per warp: doubles ts[W] | ys[W].
+// smem per warp: doubles ts[W] | ys[W].  BAND as ls_peak_kernel.
 constexpr int LSP_WPB = 4;
+template <bool BAND>
 __global__ void __launch_bounds__(32 * LSP_WPB) ls_peak_warp_kernel(const double* __restrict__ proc_x, const double* __restrict__ proc_y,
                                                                     const bpv_window_params p, int max_bins, long long nsig,
                                                                     float* __restrict__ spec_f, float* __restrict__ psd,
                                                                     int32_t* __restrict__ num_bins, int32_t* __restrict__ peak_idx,
-                                                                    double* __restrict__ peak_freq, double* __restrict__ peak_mag) {
+                                                                    double* __restrict__ peak_freq, double* __restrict__ peak_mag,
+                                                                    const PeakBand band) {
   extern __shared__ __align__(16) double sm[];
   const int W = p.window, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const long long sig = (long long)blockIdx.x * LSP_WPB + wid;
@@ -538,8 +571,17 @@ __global__ void __launch_bounds__(32 * LSP_WPB) ls_peak_warp_kernel(const double
   const int F = p.ls_num_freqs > 0 ? p.ls_num_freqs : n;
   float* row = psd + sig * max_bins;
   float bv = -INFINITY; int cnt = 0;
-  for (int k = lane; k < F; k += 32) { const float v = row[k]; if (isfinite(v)) { ++cnt; bv = fmaxf(bv, v); } }
+  float bb = -INFINITY; int cb = 0;              // BAND: over the finite in-band bins
+  for (int k = lane; k < F; k += 32) {
+    const float v = row[k];
+    if (isfinite(v)) {
+      ++cnt; bv = fmaxf(bv, v);
+      if (BAND && band.in(ls_freq(k, F, p.min_freq, p.max_freq))) { ++cb; bb = fmaxf(bb, v); }
+    }
+  }
   for (int o = 16; o > 0; o >>= 1) { bv = fmaxf(bv, __shfl_xor_sync(0xffffffffu, bv, o)); cnt += __shfl_xor_sync(0xffffffffu, cnt, o); }
+  if (BAND)
+    for (int o = 16; o > 0; o >>= 1) { bb = fmaxf(bb, __shfl_xor_sync(0xffffffffu, bb, o)); cb += __shfl_xor_sync(0xffffffffu, cb, o); }
   // moments for the float64 evaluation (relative time; Y, YY as scipy Eq. 7 / 10; centred second moment)
   const double t0 = xs[0];
   double a = 0.0;
@@ -551,21 +593,28 @@ __global__ void __launch_bounds__(32 * LSP_WPB) ls_peak_warp_kernel(const double
   for (int j = lane; j < n; j += 32) xs[j] -= t0;
   __syncwarp();
   const bool all = n < LS_SMALL_N || cnt < 2;
+  const bool all_b = BAND ? (n < LS_SMALL_N || cb < 2) : all;
   double best = -INFINITY; int bi = 0x7fffffff, nf64 = 0;
   for (int k0 = 0; k0 < F; k0 += 32) {
     const int k = k0 + lane;
-    bool cand = false;
-    if (k < F) { const float v = row[k]; cand = all || (isfinite(v) && v >= bv - LS_DELTA); }
-    unsigned mk = __ballot_sync(0xffffffffu, cand);
+    bool cand = false, cand_b = false;
+    if (k < F) {
+      const float v = row[k];
+      cand = all || (isfinite(v) && v >= bv - LS_DELTA);
+      if (BAND) cand_b = band.in(ls_freq(k, F, p.min_freq, p.max_freq)) && (all_b || (isfinite(v) && v >= bb - LS_DELTA));
+    }
+    // BAND: mw = bins whose float64 value is written back (the unbanded candidates), mb = in-band candidates
+    unsigned mk = __ballot_sync(0xffffffffu, cand || cand_b);
+    const unsigned mw = BAND ? __ballot_sync(0xffffffffu, cand) : 0u, mb = BAND ? __ballot_sync(0xffffffffu, cand_b) : 0u;
     while (mk) {
-      const int kc = k0 + __ffs(mk) - 1;
+      const int b = __ffs(mk) - 1, kc = k0 + b;
       mk &= mk - 1;
       const double v = ls_eval_f64(xs, ys, n, ls_freq(kc, F, p.min_freq, p.max_freq), Y, YY);
-      if (lane == 0) row[kc] = (float)v;
-      if (isfinite(v)) { ++nf64; if (v > best || (v == best && kc < bi)) { best = v; bi = kc; } }
+      if (lane == 0 && (!BAND || ((mw >> b) & 1u))) row[kc] = (float)v;
+      if ((!BAND || ((mb >> b) & 1u)) && isfinite(v)) { ++nf64; if (v > best || (v == best && kc < bi)) { best = v; bi = kc; } }
     }
   }
-  const int nfinite = all ? nf64 : cnt;
+  const int nfinite = all_b ? nf64 : (BAND ? cb : cnt);
   if (lane == 0) {
     num_bins[sig] = F;
     if (nfinite >= 2 && bi != 0x7fffffff) {
@@ -596,7 +645,19 @@ extern "C" int bpv_window_spectrum(const double* proc_x, const double* proc_y, c
                                    int32_t max_bins, void* workspace, int64_t workspace_bytes,
                                    float* spec_f, float* spec_mag, int32_t* num_bins,
                                    int32_t* peak_idx, double* peak_freq, double* peak_mag, void* stream) {
+  return bpv_window_spectrum_band(proc_x, proc_y, p, max_bins, workspace, workspace_bytes, spec_f, spec_mag, num_bins, peak_idx, peak_freq,
+                                  peak_mag, -INFINITY, INFINITY, stream);
+}
+
+extern "C" int bpv_window_spectrum_band(const double* proc_x, const double* proc_y, const bpv_window_params* p,
+                                        int32_t max_bins, void* workspace, int64_t workspace_bytes,
+                                        float* spec_f, float* spec_mag, int32_t* num_bins,
+                                        int32_t* peak_idx, double* peak_freq, double* peak_mag,
+                                        double min_freq, double max_freq, void* stream) {
   using namespace bpv;
+  BPV_REQUIRE(!isnan(min_freq) && !isnan(max_freq), BPV_E_INVALID, "bpv_window_spectrum: NaN frequency band (%g, %g)", min_freq, max_freq);
+  const bool banded = band_limits(min_freq, max_freq);
+  const PeakBand band{min_freq, max_freq};
   BPV_REQUIRE(p && proc_x && proc_y && num_bins && peak_idx && peak_freq && peak_mag, BPV_E_INVALID,
               "bpv_window_spectrum: NULL pointer");
   BPV_REQUIRE((spec_f == nullptr) == (spec_mag == nullptr), BPV_E_INVALID, "bpv_window_spectrum: spec_f/spec_mag must both be set or both NULL");
@@ -611,15 +672,22 @@ extern "C" int bpv_window_spectrum(const double* proc_x, const double* proc_y, c
     BPV_REQUIRE(!spec_mag || max_bins >= need, BPV_E_INVALID, "bpv_window_spectrum: max_bins %d < %d", max_bins, need);
     if (p->transform == BPV_PGRAM_WELCH && W <= 512) {   // warp per signal (x staging needs W <= 512 doubles)
       const size_t smw = (size_t)(512 + WELCH_WPB * welch_warp_doubles(W)) * sizeof(double);
-      if (int rc = ensure_dyn_smem((const void*)welch_warp_kernel, smw)) return rc;
       const int only_flagged = 0;
-      welch_warp_kernel<<<(unsigned)((nsig + WELCH_WPB - 1) / WELCH_WPB), 32 * WELCH_WPB, smw, st>>>(
-          proc_x, proc_y, *p, max_bins, nsig, only_flagged, spec_f, spec_mag, num_bins, peak_idx, peak_freq, peak_mag);
+      const unsigned grid = (unsigned)((nsig + WELCH_WPB - 1) / WELCH_WPB);
+      const void* kfn = banded ? (const void*)welch_warp_kernel<true> : (const void*)welch_warp_kernel<false>;
+      if (int rc = ensure_dyn_smem(kfn, smw)) return rc;
+      if (banded)
+        welch_warp_kernel<true><<<grid, 32 * WELCH_WPB, smw, st>>>(proc_x, proc_y, *p, max_bins, nsig, only_flagged, spec_f, spec_mag,
+                                                                   num_bins, peak_idx, peak_freq, peak_mag, band);
+      else
+        welch_warp_kernel<false><<<grid, 32 * WELCH_WPB, smw, st>>>(proc_x, proc_y, *p, max_bins, nsig, only_flagged, spec_f, spec_mag,
+                                                                    num_bins, peak_idx, peak_freq, peak_mag, band);
       return check_launch("welch_warp_kernel");
     }
     const size_t smem = (size_t)(4 * W + W / 2 + 2 + 256) * sizeof(double);
     BPV_REQUIRE(smem <= 200 * 1024, BPV_E_TOO_LARGE, "bpv_window_spectrum: window %d too large for the dense spectrum kernel", W);
-    if (int rc = ensure_dyn_smem((const void*)spectrum_dense_kernel, smem)) return rc;
+    if (int rc = ensure_dyn_smem(banded ? (const void*)spectrum_dense_kernel<true> : (const void*)spectrum_dense_kernel<false>, smem))
+      return rc;
     // DFT_RFFT as one dense contraction on the tensor cores (dft_tc.cu) when the windows of the launch share n = W: by
     // default for pipelines that resample (INTERP_*: valid = block, so every warmed-up window is full), or forced /
     // disabled with BPV_DFT_TC=1 / 0.  Windows with a non-finite sample are flagged and taken by the float64 kernel.
@@ -642,12 +710,18 @@ extern "C" int bpv_window_spectrum(const double* proc_x, const double* proc_y, c
         const int64_t ib = (dft_tc_image_bytes(W) + 255) / 256 * 256;
         void* images = (workspace && workspace_bytes >= cb + ib) ? (void*)((unsigned char*)workspace + cb) : nullptr;
         void* split = (images && workspace_bytes >= cb + ib + dft_tc_split_bytes(W, nsig)) ? (void*)((unsigned char*)workspace + cb + ib) : nullptr;
-        if (int rc = launch_dft_tc(proc_x, proc_y, W, nsig, max_bins, spec_f, coarse, num_bins, peak_idx, peak_freq, peak_mag, images, split, st)) return rc;
+        if (int rc = launch_dft_tc(proc_x, proc_y, W, nsig, max_bins, spec_f, coarse, num_bins, peak_idx, peak_freq, peak_mag, images, split,
+                                   banded, band, st))
+          return rc;
         only_flagged = 1;
       }
     }
-    spectrum_dense_kernel<<<(unsigned)nsig, 128, smem, st>>>(proc_x, proc_y, *p, max_bins, only_flagged, spec_f, spec_mag, num_bins,
-                                                            peak_idx, peak_freq, peak_mag);
+    if (banded)
+      spectrum_dense_kernel<true><<<(unsigned)nsig, 128, smem, st>>>(proc_x, proc_y, *p, max_bins, only_flagged, spec_f, spec_mag, num_bins,
+                                                                     peak_idx, peak_freq, peak_mag, band);
+    else
+      spectrum_dense_kernel<false><<<(unsigned)nsig, 128, smem, st>>>(proc_x, proc_y, *p, max_bins, only_flagged, spec_f, spec_mag,
+                                                                      num_bins, peak_idx, peak_freq, peak_mag, band);
     return check_launch("spectrum_dense_kernel");
   }
   const int Fmax = p->ls_num_freqs > 0 ? p->ls_num_freqs : W;
@@ -687,12 +761,23 @@ extern "C" int bpv_window_spectrum(const double* proc_x, const double* proc_y, c
   if (int rc = check_launch("ls_coarse_kernel")) return rc;
   const size_t smem_w = (size_t)LSP_WPB * 2 * W * sizeof(double);
   if (smem_w <= 200 * 1024) {          // warp per signal
-    if (int rc = ensure_dyn_smem((const void*)ls_peak_warp_kernel, smem_w)) return rc;
-    ls_peak_warp_kernel<<<(unsigned)((nsig + LSP_WPB - 1) / LSP_WPB), 32 * LSP_WPB, smem_w, st>>>(proc_x, proc_y, *p, max_bins, nsig, spec_f,
-                                                                                                 psd, num_bins, peak_idx, peak_freq, peak_mag);
+    const unsigned grid = (unsigned)((nsig + LSP_WPB - 1) / LSP_WPB);
+    if (int rc = ensure_dyn_smem(banded ? (const void*)ls_peak_warp_kernel<true> : (const void*)ls_peak_warp_kernel<false>, smem_w))
+      return rc;
+    if (banded)
+      ls_peak_warp_kernel<true><<<grid, 32 * LSP_WPB, smem_w, st>>>(proc_x, proc_y, *p, max_bins, nsig, spec_f, psd, num_bins, peak_idx,
+                                                                    peak_freq, peak_mag, band);
+    else
+      ls_peak_warp_kernel<false><<<grid, 32 * LSP_WPB, smem_w, st>>>(proc_x, proc_y, *p, max_bins, nsig, spec_f, psd, num_bins, peak_idx,
+                                                                     peak_freq, peak_mag, band);
     return check_launch("ls_peak_warp_kernel");
   }
-  if (int rc = ensure_dyn_smem((const void*)ls_peak_kernel, smem_p)) return rc;
-  ls_peak_kernel<<<(unsigned)nsig, 128, smem_p, st>>>(proc_x, proc_y, *p, max_bins, spec_f, psd, num_bins, peak_idx, peak_freq, peak_mag);
+  if (int rc = ensure_dyn_smem(banded ? (const void*)ls_peak_kernel<true> : (const void*)ls_peak_kernel<false>, smem_p)) return rc;
+  if (banded)
+    ls_peak_kernel<true><<<(unsigned)nsig, 128, smem_p, st>>>(proc_x, proc_y, *p, max_bins, spec_f, psd, num_bins, peak_idx, peak_freq,
+                                                              peak_mag, band);
+  else
+    ls_peak_kernel<false><<<(unsigned)nsig, 128, smem_p, st>>>(proc_x, proc_y, *p, max_bins, spec_f, psd, num_bins, peak_idx, peak_freq,
+                                                               peak_mag, band);
   return check_launch("ls_peak_kernel");
 }

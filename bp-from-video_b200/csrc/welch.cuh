@@ -65,12 +65,14 @@ __device__ __forceinline__ void welch_fft_pass(double2* __restrict__ fz, const d
 
 // The kernel's body as a device function of (CTA index, shared memory): welch_warp_kernel (spectrum.cu) is a CTA of four such
 // warps; welch_xcorr_kernel (welch_xcorr.cu) interleaves CTAs of this role with cross-correlation CTAs in one grid.
+// BAND: the peak is searched over the bins with band.lo <= k * fval <= band.hi only (common.cuh PeakBand).
+template <bool BAND = false>
 __device__ __forceinline__ void welch_warp_body(unsigned blk, double* __restrict__ sm, const double* __restrict__ proc_x,
                                                 const double* __restrict__ proc_y, const bpv_window_params& p, int max_bins,
                                                 long long nsig, int only_flagged, float* __restrict__ spec_f,
                                                 float* __restrict__ spec_mag, int32_t* __restrict__ num_bins,
                                                 int32_t* __restrict__ peak_idx, double* __restrict__ peak_freq,
-                                                double* __restrict__ peak_mag) {
+                                                double* __restrict__ peak_mag, const PeakBand band = PeakBand{}) {
   const int W = p.window, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   double2* tw = reinterpret_cast<double2*>(sm);                 // [256] exp(+2*pi*i*k/256) as (cos, sin)
   const long long sig = (long long)blk * WELCH_WPB + wid;
@@ -212,7 +214,8 @@ __device__ __forceinline__ void welch_warp_body(unsigned blk, double* __restrict
       __syncwarp();
     }
   }
-  // rfftfreq(N, d=1/fs)[k] = k * (1/(N*d)); mean over segments; argmax with numpy's first-max rule over finite bins
+  // rfftfreq(N, d=1/fs)[k] = k * (1/(N*d)); mean over segments; argmax with numpy's first-max rule over finite (BAND: and
+  // in-band) bins
   const double fval = 1.0 / ((double)N * (1.0 / fs));
   double bv = -INFINITY; int bi = 0x7fffffff, cnt = 0;
   if (fft) {
@@ -225,7 +228,7 @@ __device__ __forceinline__ void welch_warp_body(unsigned blk, double* __restrict
           spec_f[sig * max_bins + k] = (float)((double)k * fval);
           spec_mag[sig * max_bins + k] = (float)v;
         }
-        if (isfinite(v)) { ++cnt; if (v > bv || (v == bv && k < bi)) { bv = v; bi = k; } }
+        if (isfinite(v) && (!BAND || band.in((double)k * fval))) { ++cnt; if (v > bv || (v == bv && k < bi)) { bv = v; bi = k; } }
       }
     }
   } else {
@@ -238,7 +241,7 @@ __device__ __forceinline__ void welch_warp_body(unsigned blk, double* __restrict
           spec_f[sig * max_bins + k] = (float)((double)k * fval);
           spec_mag[sig * max_bins + k] = (float)v;
         }
-        if (isfinite(v)) { ++cnt; if (v > bv) { bv = v; bi = k; } }
+        if (isfinite(v) && (!BAND || band.in((double)k * fval))) { ++cnt; if (v > bv) { bv = v; bi = k; } }
       }
     }
   }

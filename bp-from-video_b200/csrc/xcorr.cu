@@ -8,11 +8,13 @@
 
 namespace bpv {
 
+// BAND: the peak is searched over the lags whose lag in seconds lies in [band.lo, band.hi] (as xcorr_warp_body)
+template <bool BAND>
 __global__ void __launch_bounds__(128) xcorr_kernel(const double* __restrict__ proc_x, const double* __restrict__ proc_y,
                                                     const bpv_window_params p, float* __restrict__ corr_lag,
                                                     float* __restrict__ corr_val, int32_t* __restrict__ num_lags,
                                                     int32_t* __restrict__ lag_idx, double* __restrict__ lag_sec,
-                                                    double* __restrict__ lag_corr) {
+                                                    double* __restrict__ lag_corr, const PeakBand band) {
   extern __shared__ __align__(16) double sm[];
   __shared__ double s_val[33];
   __shared__ int s_idx[64];
@@ -125,21 +127,32 @@ __global__ void __launch_bounds__(128) xcorr_kernel(const double* __restrict__ p
   __syncthreads();
   // PEAK in float64: every lag whose coarse value is within XC_DELTA of the coarse maximum is re-evaluated as a
   // float64 dot product; the first maximum among those decides (Signal.get_peak after the range reset).
-  float cmax = -INFINITY; int cnt = 0;
-  for (int li = tid; li < L; li += blockDim.x) { const float v = cv[li]; if (isfinite(v)) { ++cnt; cmax = fmaxf(cmax, v); } }
+  auto in_band = [&](int li) {
+    const int k = li - (n - 1), ak = k < 0 ? -k : k;
+    return band.in((xa[n - 1] - xa[n - 1 - ak]) * (k > 0 ? 1.0 : (k < 0 ? -1.0 : 0.0)));
+  };
+  float cmax = -INFINITY; int cnt = 0, nin = 0;   // BAND: nin = lags inside the band
+  for (int li = tid; li < L; li += blockDim.x) {
+    const float v = cv[li];
+    const bool inb = !BAND || in_band(li);
+    if (BAND && inb) ++nin;
+    if (isfinite(v) && inb) { ++cnt; cmax = fmaxf(cmax, v); }
+  }
   for (int o = 16; o > 0; o >>= 1) { cmax = fmaxf(cmax, __shfl_xor_sync(0xffffffffu, cmax, o)); cnt += __shfl_xor_sync(0xffffffffu, cnt, o); }
+  if (BAND) nin = warp_sum(nin);
   {
     const int wid = tid >> 5, nw = blockDim.x >> 5;
-    if (lane == 0) { s_val[wid] = cmax; s_idx[wid] = cnt; }
+    if (lane == 0) { s_val[wid] = cmax; s_idx[wid] = cnt; if (BAND) s_idx[16 + wid] = nin; }
     __syncthreads();
     cmax = s_val[0]; cnt = s_idx[0];
-    for (int w2 = 1; w2 < nw; ++w2) { cmax = fmaxf(cmax, (float)s_val[w2]); cnt += s_idx[w2]; }
+    if (BAND) nin = s_idx[16];
+    for (int w2 = 1; w2 < nw; ++w2) { cmax = fmaxf(cmax, (float)s_val[w2]); cnt += s_idx[w2]; if (BAND) nin += s_idx[16 + w2]; }
     __syncthreads();
   }
   double bv = -INFINITY; int bi = 0x7fffffff;
   for (int li = tid; li < L; li += blockDim.x) {
     const float v = cv[li];
-    if (cnt >= 2 ? (isfinite(v) && v >= cmax - XC_DELTA) : true) {
+    if ((cnt >= 2 ? (isfinite(v) && v >= cmax - XC_DELTA) : true) && (!BAND || in_band(li))) {
       const int k = li - (n - 1);
       const int l0 = k < 0 ? -k : 0, l1 = k > 0 ? n - k : n;
       double acc = 0.0;
@@ -160,10 +173,11 @@ __global__ void __launch_bounds__(128) xcorr_kernel(const double* __restrict__ p
     if (tid == 0) {
       for (int w2 = 1; w2 < nw; ++w2)
         if (s_val[w2] > bv || (s_val[w2] == bv && s_idx[w2] < bi)) { bv = s_val[w2]; bi = s_idx[w2]; }
-      // finite-lag count in float64 terms: den == 0 or non-finite makes every lag non-finite (NaN / inf)
+      // finite-lag count in float64 terms: den == 0 or non-finite makes every lag non-finite (NaN / inf); BAND: of the lags
+      // inside the band
       const bool any = isfinite(den) && den != 0.0 && bi != 0x7fffffff;
       num_lags[jp] = L;
-      if (any && L >= 2) {
+      if (any && (BAND ? nin : L) >= 2) {
         const int k = bi - (n - 1), ak = k < 0 ? -k : k;
         lag_idx[jp] = bi;
         lag_sec[jp] = (xa[n - 1] - xa[n - 1 - ak]) * (k > 0 ? 1.0 : (k < 0 ? -1.0 : 0.0));
@@ -175,14 +189,16 @@ __global__ void __launch_bounds__(128) xcorr_kernel(const double* __restrict__ p
 
 
 // warp-per-pair kernel (default): body in xcorr_warp.cuh
-template <int LDC, bool ONE>
+template <int LDC, bool ONE, bool BAND>
 __global__ void __launch_bounds__(128, ONE ? 5 : 1) xcorr_warp_kernel(const double* __restrict__ proc_x, const double* __restrict__ proc_y,
                                                          const bpv_window_params p, const XwLayout Lw, long long npairs,
                                                          float* __restrict__ corr_lag, float* __restrict__ corr_val,
                                                          int32_t* __restrict__ num_lags, int32_t* __restrict__ lag_idx,
-                                                         double* __restrict__ lag_sec, double* __restrict__ lag_corr) {
+                                                         double* __restrict__ lag_sec, double* __restrict__ lag_corr,
+                                                         const PeakBand band) {
   extern __shared__ __align__(16) unsigned char xsm[];
-  xcorr_warp_body<LDC, ONE>(blockIdx.x, xsm, proc_x, proc_y, p, Lw, npairs, corr_lag, corr_val, num_lags, lag_idx, lag_sec, lag_corr);
+  xcorr_warp_body<LDC, ONE, BAND>(blockIdx.x, xsm, proc_x, proc_y, p, Lw, npairs, corr_lag, corr_val, num_lags, lag_idx, lag_sec, lag_corr,
+                                  band);
 }
 
 }  // namespace bpv
@@ -190,7 +206,17 @@ __global__ void __launch_bounds__(128, ONE ? 5 : 1) xcorr_warp_kernel(const doub
 extern "C" int bpv_window_xcorr(const double* proc_x, const double* proc_y, const bpv_window_params* p,
                                 float* corr_lag, float* corr_val, int32_t* num_lags,
                                 int32_t* lag_idx, double* lag_sec, double* lag_corr, void* stream) {
+  return bpv_window_xcorr_band(proc_x, proc_y, p, corr_lag, corr_val, num_lags, lag_idx, lag_sec, lag_corr, -INFINITY, INFINITY, stream);
+}
+
+extern "C" int bpv_window_xcorr_band(const double* proc_x, const double* proc_y, const bpv_window_params* p,
+                                     float* corr_lag, float* corr_val, int32_t* num_lags,
+                                     int32_t* lag_idx, double* lag_sec, double* lag_corr,
+                                     double min_lag, double max_lag, void* stream) {
   using namespace bpv;
+  BPV_REQUIRE(!isnan(min_lag) && !isnan(max_lag), BPV_E_INVALID, "bpv_window_xcorr: NaN lag band (%g, %g)", min_lag, max_lag);
+  const bool banded = band_limits(min_lag, max_lag);
+  const PeakBand band{min_lag, max_lag};
   BPV_REQUIRE(p && proc_x && proc_y && num_lags && lag_idx && lag_sec && lag_corr, BPV_E_INVALID, "bpv_window_xcorr: NULL pointer");
   BPV_REQUIRE((corr_lag == nullptr) == (corr_val == nullptr), BPV_E_INVALID, "bpv_window_xcorr: corr_lag/corr_val must both be set or both NULL");
   const int W = p->window, P = p->R * (p->R - 1) / 2;
@@ -206,11 +232,16 @@ extern "C" int bpv_window_xcorr(const double* proc_x, const double* proc_y, cons
     if (wpb >= 1) {
       const size_t smw = (size_t)wpb * Lw.total;
       const unsigned grid = (unsigned)((n + wpb - 1) / wpb);
+#define BPV_XW1(LDC, ONE, BAND)                                                                                       \
+  do {                                                                                                                \
+    if (int rc = ensure_dyn_smem((const void*)xcorr_warp_kernel<LDC, ONE, BAND>, smw)) return rc;                     \
+    xcorr_warp_kernel<LDC, ONE, BAND><<<grid, wpb * 32, smw, (cudaStream_t)stream>>>(proc_x, proc_y, *p, Lw, n, corr_lag, \
+                                                                 corr_val, num_lags, lag_idx, lag_sec, lag_corr, band); \
+  } while (0)
 #define BPV_XW(LDC, ONE)                                                                                              \
   do {                                                                                                                \
-    if (int rc = ensure_dyn_smem((const void*)xcorr_warp_kernel<LDC, ONE>, smw)) return rc;                           \
-    xcorr_warp_kernel<LDC, ONE><<<grid, wpb * 32, smw, (cudaStream_t)stream>>>(proc_x, proc_y, *p, Lw, n, corr_lag,  \
-                                                                              corr_val, num_lags, lag_idx, lag_sec, lag_corr); \
+    if (banded) BPV_XW1(LDC, ONE, true);                                                                              \
+    else BPV_XW1(LDC, ONE, false);                                                                                    \
   } while (0)
       if (Lw.LD == 63 && Lw.one_round) BPV_XW(63, true);      // windows of 291..300 samples (the 10 s window at 30 fps)
       else if (Lw.LD == 53 && Lw.one_round) BPV_XW(53, true); // 241..250 (the reference's default signal_max_samples)
@@ -218,13 +249,19 @@ extern "C" int bpv_window_xcorr(const double* proc_x, const double* proc_y, cons
       else if (Lw.one_round) BPV_XW(0, true);
       else BPV_XW(0, false);
 #undef BPV_XW
+#undef BPV_XW1
       return check_launch("bpv_window_xcorr");
     }
   }
   const int Kw = (W + 7) / 8 * 8;
   const size_t smem = (size_t)(3 * W) * sizeof(double) + (size_t)(2 * W + Kw + 8 * ((Kw + 3 * W + 16) / 8 + 1)) * sizeof(float);
   BPV_REQUIRE(smem <= 200 * 1024, BPV_E_TOO_LARGE, "bpv_window_xcorr: window %d too large for shared memory", W);
-  if (int rc = ensure_dyn_smem((const void*)xcorr_kernel, smem)) return rc;
-  xcorr_kernel<<<(unsigned)n, 128, smem, (cudaStream_t)stream>>>(proc_x, proc_y, *p, corr_lag, corr_val, num_lags, lag_idx, lag_sec, lag_corr);
+  if (int rc = ensure_dyn_smem(banded ? (const void*)xcorr_kernel<true> : (const void*)xcorr_kernel<false>, smem)) return rc;
+  if (banded)
+    xcorr_kernel<true><<<(unsigned)n, 128, smem, (cudaStream_t)stream>>>(proc_x, proc_y, *p, corr_lag, corr_val, num_lags, lag_idx, lag_sec,
+                                                                         lag_corr, band);
+  else
+    xcorr_kernel<false><<<(unsigned)n, 128, smem, (cudaStream_t)stream>>>(proc_x, proc_y, *p, corr_lag, corr_val, num_lags, lag_idx, lag_sec,
+                                                                          lag_corr, band);
   return check_launch("bpv_window_xcorr");
 }

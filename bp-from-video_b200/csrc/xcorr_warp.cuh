@@ -46,12 +46,16 @@ __host__ __device__ inline XwLayout xw_layout(int W, bool force_cv = false) {
 // 88 registers keep the packed tile loop free of spills (ptxas settles on 72 without it and pays 60 register moves per 10 taps).
 // The kernel's body as a device function of (CTA index, shared memory): xcorr_warp_kernel (xcorr.cu) is a CTA of up to four
 // such warps; welch_xcorr_kernel (welch_xcorr.cu) interleaves CTAs of this role with Welch CTAs in one grid.
-template <int LDC, bool ONE>
+// BAND: the peak is searched over the lags whose lag in seconds (the float64 value reported as lag_sec) lies in [band.lo, band.hi],
+// evaluated lag by lag (the timestamps need not be monotone); the coarse maximum and the finite count are taken over those lags
+// alone, so that an out-of-band maximum cannot set a threshold that excludes every in-band lag.
+template <int LDC, bool ONE, bool BAND = false>
 __device__ __forceinline__ void xcorr_warp_body(unsigned blk, unsigned char* __restrict__ xsm, const double* __restrict__ proc_x,
                                                 const double* __restrict__ proc_y, const bpv_window_params& p, const XwLayout& Lw,
                                                 long long npairs, float* __restrict__ corr_lag, float* __restrict__ corr_val,
                                                 int32_t* __restrict__ num_lags, int32_t* __restrict__ lag_idx,
-                                                double* __restrict__ lag_sec, double* __restrict__ lag_corr) {
+                                                double* __restrict__ lag_sec, double* __restrict__ lag_corr,
+                                                const PeakBand band = PeakBand{}) {
   constexpr int RT = XW_RT;
   const int W = p.window, R = p.R, P = R * (R - 1) / 2, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const long long jp = (long long)blk * (blockDim.x >> 5) + wid;          // job * P + pair
@@ -134,9 +138,14 @@ __device__ __forceinline__ void xcorr_warp_body(unsigned blk, unsigned char* __r
   const int L = 2 * n - 1;
   const long long ob = jp * (2LL * W - 1);
   const double x_last = xa_g[pos[n - 1]];
+  auto in_band = [&](int li) {                  // BAND: lag index li -> is its lag in seconds inside the band
+    const int k = li - (n - 1), ak = k < 0 ? -k : k;
+    return band.in((x_last - xa_g[pos[n - 1 - ak]]) * (k > 0 ? 1.0 : (k < 0 ? -1.0 : 0.0)));
+  };
   float cmax = -INFINITY; int cnt = 0;          // coarse maximum / finite count, gathered while the tiles are written
+  int nin = 0;                                  // BAND, cv[] path: lags inside the band (ONE: the bits of okm)
   const int tiles = K / RT;
-  unsigned okm = 0;                             // ONE: bit r = first lag of pair r is a lag of this window, bit RT + r = second lag
+  unsigned okm = 0;                             // ONE: bit r = first lag of pair r is a lag of this window (BAND: in band), bit RT + r = second lag
   float acc[RT], first[RT];                     // ONE: after the tile, the lane's scaled coarse values (second | first lags)
   for (int tile = lane; tile < tiles; tile += 32) {
 #pragma unroll
@@ -152,8 +161,10 @@ __device__ __forceinline__ void xcorr_warp_body(unsigned blk, unsigned char* __r
         const bool ok = h ? (la <= n - 2) : (la >= 0 && la <= n - 2);
         if (ok) {
           const float cc = h ? acc[r] : first[r];
-          if (ONE) okm |= 1u << (h * RT + r); else cv[li] = cc;
-          if (isfinite(cc)) { ++cnt; cmax = fmaxf(cmax, cc); }
+          bool inb = true;
+          if (BAND) inb = in_band(li);
+          if (ONE) { if (inb) okm |= 1u << (h * RT + r); } else { cv[li] = cc; if (BAND && inb) ++nin; }
+          if (isfinite(cc) && inb) { ++cnt; cmax = fmaxf(cmax, cc); }
           if (corr_val) {
             const int k = li - (n - 1), ak = k < 0 ? -k : k;
             const double lag = (x_last - xa_g[pos[n - 1 - ak]]) * (k > 0 ? 1.0 : (k < 0 ? -1.0 : 0.0));
@@ -206,7 +217,10 @@ __device__ __forceinline__ void xcorr_warp_body(unsigned blk, unsigned char* __r
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
         const int li = lb + e;
-        if (li < L) { const float v = cv[li]; if (cnt >= 2 ? (isfinite(v) && v >= thr) : true) flags |= 1u << e; }
+        if (li < L) {
+          const float v = cv[li];
+          if ((cnt >= 2 ? (isfinite(v) && v >= thr) : true) && (!BAND || in_band(li))) flags |= 1u << e;
+        }
       }
       unsigned m = __ballot_sync(0xffffffffu, flags != 0);
       while (m) {                                  // lanes in increasing lag order, lags of a lane in increasing order
@@ -221,11 +235,14 @@ __device__ __forceinline__ void xcorr_warp_body(unsigned blk, unsigned char* __r
       }
     }
   }
+  // eligible lags (BAND: inside the band) in float64 terms: den == 0 or non-finite makes every lag non-finite (NaN / inf),
+  // any other den every lag finite
+  int neligible = L;
+  if (BAND) neligible = warp_sum(ONE ? __popc(okm) : nin);
   if (lane == 0) {
-    // finite-lag count in float64 terms: den == 0 or non-finite makes every lag non-finite (NaN / inf)
     const bool any = isfinite(den) && den != 0.0 && bi != 0x7fffffff;
     num_lags[jp] = L;
-    if (any && L >= 2) {
+    if (any && neligible >= 2) {
       const int k = bi - (n - 1), ak = k < 0 ? -k : k;
       lag_idx[jp] = bi;
       lag_sec[jp] = (x_last - xa_g[pos[n - 1 - ak]]) * (k > 0 ? 1.0 : (k < 0 ? -1.0 : 0.0));

@@ -232,6 +232,19 @@ int bpv_window_spectrum(const double* proc_x, const double* proc_y, const bpv_wi
                         int32_t max_bins, void* workspace, int64_t workspace_bytes,
                         float* spec_f, float* spec_mag, int32_t* num_bins,
                         int32_t* peak_idx, double* peak_freq, double* peak_mag, void* stream);
+/* Band-limited HR peak — what a single transform_signal(s).get_peak() searches (signal_processor.py:272 sets the range to
+ *     (min_freq, max_freq); signal_data.py:65-70), where process() searches every bin.  Same arguments and spectra as
+ * bpv_window_spectrum; the peak is the first maximum over the bins k with a finite magnitude and
+ * min_freq <= x_k <= max_freq, x_k being the float64 frequency the kernel reports for the bin (k * fval for DFT_RFFT /
+ * PGRAM_WELCH, the linspace value for PGRAM_LS).  Fewer than two such bins: no peak (-1 / NaN).  peak_idx still indexes
+ * the full spectrum, and spec_f / spec_mag / num_bins do not depend on the band.  (-INFINITY, INFINITY) is
+ * bpv_window_spectrum bit for bit (which forwards here); min_freq > max_freq gives no peak; a NaN bound returns
+ * BPV_E_INVALID before anything is enqueued. */
+int bpv_window_spectrum_band(const double* proc_x, const double* proc_y, const bpv_window_params* p,
+                             int32_t max_bins, void* workspace, int64_t workspace_bytes,
+                             float* spec_f, float* spec_mag, int32_t* num_bins,
+                             int32_t* peak_idx, double* peak_freq, double* peak_mag,
+                             double min_freq, double max_freq, void* stream);
 
 /* F4(b) pairwise cross-correlation lag search — replaces correlate_signal_pair / correlate_signals
  *     + get_peaks on sg_corr (signal_processor.py:280-299, 312).  Pairs in
@@ -242,8 +255,19 @@ int bpv_window_spectrum(const double* proc_x, const double* proc_y, const bpv_wi
 int bpv_window_xcorr(const double* proc_x, const double* proc_y, const bpv_window_params* p,
                      float* corr_lag, float* corr_val, int32_t* num_lags,
                      int32_t* lag_idx, double* lag_sec, double* lag_corr, void* stream);
+/* Band-limited PTT lag — what a single correlate_signal_pair(a, b).get_peak() searches (signal_processor.py:294 sets the
+ *     range to (min_lag, max_lag) = (-0.5, 0.5) s).  Same arguments and correlations as bpv_window_xcorr; the peak is the
+ * first maximum over the lags with a finite correlation and min_lag <= x_k <= max_lag, x_k = (x_last - x[pos[n-1-|k|]]) *
+ * sign(k) being the float64 lag in seconds reported as lag_sec, evaluated lag by lag (timestamps need not be monotone).
+ * Fewer than two such lags: no peak.  lag_idx still indexes the 2n-1 lags.  (-INFINITY, INFINITY) is bpv_window_xcorr bit
+ * for bit (which forwards here); min_lag > max_lag gives no peak; a NaN bound returns BPV_E_INVALID before anything is
+ * enqueued. */
+int bpv_window_xcorr_band(const double* proc_x, const double* proc_y, const bpv_window_params* p,
+                          float* corr_lag, float* corr_val, int32_t* num_lags,
+                          int32_t* lag_idx, double* lag_sec, double* lag_corr,
+                          double min_lag, double max_lag, void* stream);
 
-/* F3 + F4 of the same window jobs in ONE grid (PGRAM_WELCH only): CTAs of the Welch kernel and of the cross-correlation
+/* F3 + F4 of the same window jobs in ONE grid (PGRAM_WELCH only; unbanded peaks): CTAs of the Welch kernel and of the cross-correlation
  *     kernel interleaved in the ratio of their counts, so that every SM holds both for the whole launch (the two are bound
  *     by different things — shared-memory wavefronts vs FP32 issue — and mix poorly when launched as two kernels).
  *     Same arguments and results, bit for bit, as bpv_window_spectrum followed by bpv_window_xcorr; shapes the fused grid
