@@ -51,11 +51,18 @@ _SIGS = {
     'bpv_scratch_discard': (C.c_int, [_P, C.c_int64, _P]),
     'bpv_dft256_tc': (C.c_int, [_P, C.c_int32, _P, _P]),
     'bpv_ring_push': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int32, _P, _P, _P]),
+    'bpv_ring_push_ragged': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P, C.c_int32, _P, _P, _P]),
+    'bpv_stream_jobs': (C.c_int, [C.c_int32, _P, _P, C.c_int32, C.c_int64, _P, _P, _P, _P, _P]),
+    'bpv_running_mean_jobs': (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, C.c_double, _P, _P, _P]),
     'bpv_window_workspace_bytes': (C.c_int64, [C.POINTER(WindowParams)]),
     'bpv_window_preprocess': (C.c_int, [_P, _P, C.POINTER(WindowParams), _P, C.c_int64, _P, _P, _P, _P]),
     'bpv_design_cache_bytes': (C.c_int64, []),
     'bpv_window_design': (C.c_int, [_P, C.POINTER(WindowParams), _P, C.c_int64, _P, C.c_int64, _P]),
     'bpv_window_filter': (C.c_int, [_P, _P, C.POINTER(WindowParams), _P, C.c_int64, _P, C.c_int64, _P, _P, _P, _P]),
+    'bpv_window_design_jobs': (C.c_int, [_P, C.POINTER(WindowParams), _P, C.c_int64, _P, C.c_int64, _P, _P, C.c_int64, _P]),
+    'bpv_window_filter_jobs': (C.c_int, [_P, _P, C.POINTER(WindowParams), _P, C.c_int64, _P, C.c_int64, _P, _P, _P, _P, _P,
+                                         C.c_int64, _P]),
+    'bpv_window_preprocess_jobs': (C.c_int, [_P, _P, C.POINTER(WindowParams), _P, C.c_int64, _P, _P, _P, _P, _P, C.c_int64, _P]),
     'bpv_probe_fma': (C.c_int64, [C.c_int32, C.c_int64, C.c_int32, _P, _P]),
     'bpv_spectrum_workspace_bytes': (C.c_int64, [C.POINTER(WindowParams), C.c_int32]),
     'bpv_window_spectrum': (C.c_int, [_P, _P, C.POINTER(WindowParams), C.c_int32, _P, C.c_int64, _P, _P, _P, _P, _P, _P, _P]),

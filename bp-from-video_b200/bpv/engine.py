@@ -34,6 +34,19 @@ reported frequency in Hz (lag in seconds) lies in [lo, hi]; fewer than two such 
 ranges the reference configures are freq_band=(min_freq, max_freq) and lag_band=(-0.5, 0.5).  Spectra, correlations and
 the stored arrays do not depend on the bands; peak_idx / lag_idx still index the full arrays, and the running means and
 packed records take the band-limited peaks.  Both are plain attributes: assign a new pair (or None) between steps.
+
+Ragged steps (`frame_counts` of step / step_signals): real streams do not advance in lockstep — cameras join and leave, run
+at different frame rates, drop frames.  frame_counts = n_s in 0..T per stream (host sequence, numpy array or CPU tensor):
+stream s takes rows [:n_s] of its T input rows and behaves exactly like its own BatchedSignalProcessor(1, R, ...) fed only
+those frames (one reference SignalProcessor per camera).  It contributes n_s window jobs ('every_frame') or one job when
+n_s > 0 ('last'); jobs are laid out stream-major and in frame order (StepResult.job_offsets / job_stream), which with every
+n_s = T is the lockstep layout.  Sample counts, running-mean history lengths and ROI smoothing rows are per stream
+(`counts`; `count` is their common value), and reset(streams=[...]) empties chosen streams only.  A step with every
+n_s = T from level counts runs the lockstep kernels unchanged; any other step builds a job map on the device
+(bpv_stream_jobs) and runs the job-map instantiations of the push, design and filter kernels, F3 / F4 over the J jobs
+(every overlap schedule, the fused grid of bit 4 included, works unchanged: F3 / F4 only see J processed windows).  A step
+with J = 0 enqueues nothing.  step_detections stays lockstep.  BPV_FORCE_JOBMAP=1 (attribute `force_jobmap`) sends level
+steps through the job-map path too: a measurement switch (tools/bench_ragged.py).
 """
 from __future__ import annotations
 
@@ -41,6 +54,7 @@ import math
 import os
 from dataclasses import dataclass, field
 
+import numpy as np
 import torch
 
 from . import _cabi, ops
@@ -48,13 +62,15 @@ from . import _cabi, ops
 EVERY_FRAME, LAST = 'every_frame', 'last'
 OVERLAP_DESIGN, OVERLAP_XCORR, OVERLAP_FUSED = 1, 2, 4
 OVERLAP_DEFAULT = OVERLAP_DESIGN | OVERLAP_XCORR    # measured on c2 (profiles/r2k_overlap_ab.txt): 0.474 ms serial, 0.467 xcorr only, 0.461 both
-STATE_VERSION = 1
+STATE_VERSION = 2          # 2: per-stream sample / running-mean counts (version 1 states hold one level count)
 
 
 @dataclass
 class StepResult:
-    """Device tensors for the J = S * jobs_per_stream window jobs of one step (job = s*jobs_per_stream + j)."""
-    jobs_per_stream: int
+    """Device tensors for the J window jobs of one step.  A lockstep step has J = S * jobs_per_stream (job =
+    s*jobs_per_stream + j); a ragged step (module docstring) has jobs_per_stream = None and the jobs of stream s in rows
+    job_offsets[s]:job_offsets[s+1], in frame order."""
+    jobs_per_stream: int | None
     samples: torch.Tensor | None          # f64 [S, T, R]   raw ROI samples of this step
     peak_freq: torch.Tensor               # f64 [J, R]      Hz (NaN = none)
     peak_idx: torch.Tensor                # i32 [J, R]
@@ -65,6 +81,25 @@ class StepResult:
     status: torch.Tensor                  # i32 [J, R]
     arrays: dict = field(default_factory=dict)   # proc_x/proc_y/freqs/mags/lags/corr/num_bins/num_lags when stored
     means: dict = field(default_factory=dict)    # mean_bpm, mean_bpm_int [J, R], mean_ptt, mean_ptt_int [J, P] when tracked
+    _job_offsets: np.ndarray | None = field(default=None, repr=False)   # host int64 [S+1] of a ragged step
+    _job_stream: torch.Tensor | None = field(default=None, repr=False)  # device int32 [J] of a ragged step
+
+    @property
+    def job_offsets(self) -> np.ndarray:
+        """Host int64 [S+1]: the jobs of stream s are rows job_offsets[s]:job_offsets[s+1]."""
+        if self._job_offsets is None:
+            S = self.peak_freq.shape[0] // self.jobs_per_stream
+            self._job_offsets = np.arange(S + 1, dtype=np.int64) * self.jobs_per_stream
+        return self._job_offsets
+
+    @property
+    def job_stream(self) -> torch.Tensor:
+        """Device int32 [J]: the stream of each job (built on first use for a lockstep step)."""
+        if self._job_stream is None:
+            off = self.job_offsets
+            rows = np.repeat(np.arange(len(off) - 1, dtype=np.int32), np.diff(off))
+            self._job_stream = torch.from_numpy(rows).to(self.peak_freq.device)
+        return self._job_stream
 
     @property
     def bpm(self):                        # signal_processor.py:310  f * 60
@@ -128,7 +163,21 @@ class BatchedSignalProcessor:
         dev, f64 = self.device, torch.float64
         self.ring_t = torch.full((self.S, self.cap), float('nan'), dtype=f64, device=dev)
         self.ring_y = torch.full((self.S, self.R, self.cap), float('nan'), dtype=f64, device=dev)
-        self.count = 0  # samples pushed per stream so far (global index of the next sample)
+        # samples pushed per stream so far (global index of the next sample) and bpm / ptt history lengths: an int while every
+        # stream holds the same count (the lockstep path), else a host int64 [S] array (the `counts` property)
+        self._cnt = self._mcnt = 0
+        # device copies for the job-map path: the sample counts (ping-pong: bpv_stream_jobs writes the advanced ones), valid
+        # while _g0_ok; the history counts are uploaded for every ragged step that tracks running means
+        self._g0 = [torch.zeros(self.S, dtype=torch.int64, device=dev) for _ in range(2)]
+        self._g0_ok = True
+        self._mg0 = torch.zeros(self.S, dtype=torch.int64, device=dev) if int(peak_max_samples) else None
+        self._ndev = torch.zeros(self.S, dtype=torch.int32, device=dev)
+        self._jobmap = [None] * int(result_buffers)          # per result buffer: job_stream i32 [Jmax], job_head i64, stream_job0 i32
+        # per result buffer: pinned staging of the host counts a job-map step uploads, and an event after those copies (the
+        # host waits on it before refilling the buffer: a fresh pinned allocation per step would call cudaHostAlloc)
+        self._staging = [None] * int(result_buffers)
+        # measurement switch: level counts take the job-map path too (tools/bench_ragged.py)
+        self.force_jobmap = os.environ.get('BPV_FORCE_JOBMAP', '0') == '1'
         Jmax = self.S * (self.Tmax if windows == EVERY_FRAME else 1)
         self._Jmax = Jmax
         self._nbuf = int(result_buffers)
@@ -138,8 +187,7 @@ class BatchedSignalProcessor:
         nproc = self._nbuf if self.store_arrays else 1
         self._proc = [torch.empty((2, Jmax, self.R, self.W), dtype=f64, device=dev) for _ in range(nproc)]   # [x | y]
         self._status = [torch.empty((Jmax, self.R), dtype=torch.int32, device=dev) for _ in range(self._nbuf)]
-        self._spec = [None] * self._nbuf
-        self._xc = [None] * self._nbuf
+        self._out = [None] * self._nbuf          # per result buffer: F3 / F4 outputs of Jmax jobs, sliced to each step's J
         p = self._params(0, 1, self.Tmax if windows == EVERY_FRAME else 1)
         self._mb = ops.max_bins(p)
         need = max(_cabi.lib().bpv_window_workspace_bytes(p), 16)
@@ -162,7 +210,6 @@ class BatchedSignalProcessor:
         self._ev = None
         # SURVEY.md §8(f) row 3: sg_bpm / sg_ptt histories and their running means on the device (0 = off)
         self.peak_max_samples = int(peak_max_samples)
-        self._mean_count = 0
         self._bpm_ring = self._ptt_ring = None
         if self.peak_max_samples:
             self._bpm_ring = torch.full((self.S, self.R, self.peak_max_samples), float('nan'), dtype=f64, device=dev)
@@ -188,6 +235,91 @@ class BatchedSignalProcessor:
                 self._ev = {k: torch.cuda.Event() for k in ('ts', 'design', 'pre', 'xc')}
         return self._side, self._ev
 
+    # per-stream counts (module docstring: ragged steps)
+    @property
+    def counts(self) -> np.ndarray:
+        """Host int64 [S]: samples pushed so far per stream."""
+        return np.full(self.S, self._cnt, dtype=np.int64) if isinstance(self._cnt, int) else self._cnt.copy()
+
+    @property
+    def count(self) -> int:
+        """The samples pushed per stream while every stream holds the same count; raises ValueError otherwise (see
+        `counts`).  Assigning it sets every stream's count."""
+        if not isinstance(self._cnt, int):
+            raise ValueError('count: the streams hold different sample counts; read `counts`')
+        return self._cnt
+
+    @count.setter
+    def count(self, value: int) -> None:
+        self._cnt = int(value)
+        self._g0_ok = False
+
+    def _level(self, a: np.ndarray):
+        """a as one int when every stream holds the same value (the lockstep path's form), else as the array."""
+        return int(a[0]) if (a == a[0]).all() else a
+
+    def _frame_counts(self, frame_counts, T: int):
+        """frame_counts (host sequence / numpy array / CPU int tensor of S values in 0..T) as int64 [S], or None."""
+        if frame_counts is None:
+            return None
+        if torch.is_tensor(frame_counts):
+            if frame_counts.device.type != 'cpu':
+                raise ValueError('frame_counts must live on the host (a sequence, numpy array or CPU tensor): the engine '
+                                 'needs the job count without synchronising with the device')
+            frame_counts = frame_counts.numpy()
+        a = np.asarray(frame_counts)
+        if a.shape != (self.S,):
+            raise ValueError(f'frame_counts must hold {self.S} values, got shape {a.shape}')
+        if a.dtype.kind not in 'iu' and not (a.dtype.kind == 'f' and np.array_equal(a, np.floor(a))):
+            raise ValueError(f'frame_counts must be integers, got {a.dtype}')
+        a = a.astype(np.int64)
+        if a.size and (a.min() < 0 or a.max() > T):
+            raise ValueError(f'frame_counts must lie in [0, {T}]')
+        return a
+
+    def _lockstep(self, n, T: int) -> bool:
+        """The lockstep path serves a step in which every stream takes T frames from the same counts."""
+        return ((n is None or bool((n == T).all())) and isinstance(self._cnt, int) and isinstance(self._mcnt, int)
+                and not self.force_jobmap)
+
+    def _plan(self, n, T: int) -> dict:
+        """Host side of a job-map step: the per-stream frame counts, job counts, offsets and J."""
+        n = np.full(self.S, T, dtype=np.int64) if n is None else n
+        jobs = n if self.windows == EVERY_FRAME else (n > 0).astype(np.int64)
+        off = np.zeros(self.S + 1, dtype=np.int64)
+        np.cumsum(jobs, out=off[1:])
+        return dict(n=n, jobs=jobs, off=off, J=int(off[-1]), T=T, mapped=False)
+
+    def _map_jobs(self, plan: dict, turn: int) -> None:
+        """Upload the step's frame counts (and the sample counts when the device copy is stale) and build the job map of
+        the plan on the device (bpv_stream_jobs), into the buffers of result turn `turn`."""
+        dev = self.device
+        if self._jobmap[turn] is None:
+            self._jobmap[turn] = (torch.empty(self._Jmax, dtype=torch.int32, device=dev),
+                                  torch.empty(self._Jmax, dtype=torch.int64, device=dev),
+                                  torch.empty(self.S + 1, dtype=torch.int32, device=dev))
+        pin = self._pinned(turn)
+        pin['n'].numpy()[:] = plan['n']
+        self._ndev.copy_(pin['n'], non_blocking=True)
+        if not self._g0_ok:
+            pin['g0'].numpy()[:] = self.counts
+            self._g0[0].copy_(pin['g0'], non_blocking=True)
+            self._g0_ok = True
+        js, jh, sj0 = self._jobmap[turn]
+        ops.stream_jobs(self._g0[0], self._ndev, self.windows == LAST, plan['J'], js, jh, sj0, self._g0[1])
+        plan['mapped'] = True
+
+    def _pinned(self, turn: int) -> dict:
+        """Pinned staging buffers of result turn `turn`, once the device has consumed their previous contents."""
+        if self._staging[turn] is None:
+            mk = lambda dt: torch.empty(self.S, dtype=dt).pin_memory()
+            self._staging[turn] = dict(n=mk(torch.int32), g0=mk(torch.int64), m0=mk(torch.int64), ev=torch.cuda.Event(), used=False)
+        pin = self._staging[turn]
+        if pin['used']:
+            pin['ev'].synchronize()
+            pin['used'] = False
+        return pin
+
     def _check_step(self, S, T, boxes=None):
         if S != self.S or not 1 <= T <= self.Tmax:
             raise ValueError(f'step: expected {self.S} streams and 1..{self.Tmax} frames per stream, got {S} x {T}')
@@ -195,7 +327,7 @@ class BatchedSignalProcessor:
             raise ValueError(f'step: boxes must be int32 [{S}, {T}, {self.R}, 4], got {tuple(boxes.shape)}')
 
     def step(self, frames: torch.Tensor, boxes: torch.Tensor, timestamps: torch.Tensor, view=None, nv12_size=None,
-             resize_to=None, masks: torch.Tensor | None = None, mask_category=0) -> StepResult:
+             resize_to=None, masks: torch.Tensor | None = None, mask_category=0, frame_counts=None) -> StepResult:
         """frames uint8 [S, T, H, W, 3] (HBM, or pinned host memory: the ROI kernel then reads the ROI rows
         straight over PCIe), boxes int32 [S, T, R, 4] (device), timestamps float64 [S, T] (device).
         view = (view_w, view_h, left, flip_horizontally): the boxes are expressed in the reference VideoReader's
@@ -204,9 +336,15 @@ class BatchedSignalProcessor:
         nv12_size = (H, W): frames are NV12 decoder buffers uint8 [S, T, 3H/2, pitch]; the ROI is sampled from the planes
         with OpenCV's integer BT.601 conversion, i.e. as from the BGR frame cv2.VideoCapture would have produced.
         masks uint8 [S, T, H, W] + mask_category (one int, or one per ROI): only ROI pixels whose segmentation category
-        matches contribute (SURVEY.md §8(f) row 4; category masks as InferenceResults.person_segmenter, inference_runner.py:154-166)."""
+        matches contribute (SURVEY.md §8(f) row 4; category masks as InferenceResults.person_segmenter, inference_runner.py:154-166).
+        frame_counts: S values n_s in 0..T on the host (module docstring, ragged steps): stream s takes rows [:n_s] of its T
+        frames.  F1 still samples all S x T rows; the rows a stream does not take cost next to nothing when their boxes
+        are BPV_NO_BOX (x0 = NO_BOX).  A step in which no stream takes a frame enqueues nothing (samples = None)."""
         S, T = frames.shape[:2]
         self._check_step(S, T, boxes)
+        n = self._frame_counts(frame_counts, T)
+        if n is not None and not n.any():
+            return self._empty_step(None)
         self._extra_launches = 0
         with torch.cuda.device(self.device):
             if view is not None:
@@ -218,26 +356,29 @@ class BatchedSignalProcessor:
                 dst_h, dst_w = resize_to
                 val, _ = ops.roi_sample_resized(frames.view(S * T, *frames.shape[2:]), dst_h, dst_w,
                                                 boxes.reshape(S * T, self.R, 4).contiguous(), self.color_channel)
-                return self.step_signals(val.view(S, T, self.R), timestamps, _count_roi=True)
+                return self.step_signals(val.view(S, T, self.R), timestamps, _count_roi=True, frame_counts=n)
             if nv12_size is not None:
                 H, W = nv12_size
                 val, _ = ops.roi_sample_nv12(frames.view(S * T, *frames.shape[2:]), H, W,
                                              boxes.reshape(S * T, self.R, 4).contiguous(), self.color_channel)
-                return self.step_signals(val.view(S, T, self.R), timestamps, _count_roi=True)
+                return self.step_signals(val.view(S, T, self.R), timestamps, _count_roi=True, frame_counts=n)
             if masks is not None:
                 val, _ = ops.roi_sample_masked(frames.view(S * T, *frames.shape[2:]), masks.view(S * T, *masks.shape[2:]),
                                                mask_category, boxes.reshape(S * T, self.R, 4).contiguous(),
                                                self.color_channel)
-                return self.step_signals(val.view(S, T, self.R), timestamps, _count_roi=True)
+                return self.step_signals(val.view(S, T, self.R), timestamps, _count_roi=True, frame_counts=n)
             samples = self._samples[self._turn][:, :T]
             if T != self.Tmax:
                 samples = torch.empty((S, T, self.R), dtype=torch.float64, device=self.device)
             design_ahead = bool(self.overlap & OVERLAP_DESIGN) and any(m in (_cabi.FILTER_BUTTER, _cabi.FILTER_FIR) for m in self.methods)
-            if design_ahead:
+            plan = None if self._lockstep(n, T) else self._plan(n, T)
+            if design_ahead and plan is None:
                 self._design_ahead(timestamps, T)
+            elif design_ahead:
+                self._design_ahead_jobs(timestamps, plan)
             ops.roi_sample(frames.view(S * T, *frames.shape[2:]), boxes.view(S * T, self.R, 4), self.color_channel,
                            roi_pixels_hint=self.roi_pixels_hint, out_value=samples.view(S * T, self.R))
-            return self.step_signals(samples, timestamps, _count_roi=True, _designed=design_ahead)
+            return self.step_signals(samples, timestamps, _count_roi=True, _designed=design_ahead, frame_counts=n, _plan=plan)
 
     def _design_ahead(self, timestamps: torch.Tensor, T: int) -> None:
         """Push the step's timestamps and start the filter design of its window jobs on the side stream: make_filter
@@ -245,14 +386,29 @@ class BatchedSignalProcessor:
         _, ev = self._streams()
         side = self._side_hi
         main = torch.cuda.current_stream(self.device)
-        ops.ring_push(self.ring_t, self.ring_y, self.count, timestamps.contiguous(), None)
+        ops.ring_push(self.ring_t, self.ring_y, self._cnt, timestamps.contiguous(), None)
         ev['ts'].record(main)
         jobs = T if self.windows == EVERY_FRAME else 1
-        head0 = self.count if self.windows == EVERY_FRAME else self.count + T - 1
+        head0 = self._cnt if self.windows == EVERY_FRAME else self._cnt + T - 1
         p = self._params(head0, 1, jobs)
         side.wait_event(ev['ts'])
         with torch.cuda.stream(side):
             ops.window_design(self.ring_t, p, self._ws, self._cache())
+            ev['design'].record(side)
+
+    def _design_ahead_jobs(self, timestamps: torch.Tensor, plan: dict) -> None:
+        """_design_ahead for a job-map step: ragged timestamp push, job map, then the design of the mapped jobs on the
+        side stream."""
+        _, ev = self._streams()
+        side = self._side_hi
+        main = torch.cuda.current_stream(self.device)
+        self._map_jobs(plan, self._turn)
+        ops.ring_push_ragged(self.ring_t, self.ring_y, self._g0[0], self._ndev, timestamps.contiguous(), None)
+        ev['ts'].record(main)
+        js, jh, _ = self._jobmap[self._turn]
+        side.wait_event(ev['ts'])
+        with torch.cuda.stream(side):
+            ops.window_design_jobs(self.ring_t, self._params(0, 1, 1), self._ws, js, jh, plan['J'], self._cache())
             ev['design'].record(side)
 
     def _cache(self):
@@ -305,37 +461,87 @@ class BatchedSignalProcessor:
         return out
 
     def step_signals(self, samples: torch.Tensor, timestamps: torch.Tensor, _count_roi: bool = False,
-                     _designed: bool = False) -> StepResult:
-        """Signals-only entry: samples float64 [S, T, R] (already ROI-sampled), timestamps float64 [S, T]."""
+                     _designed: bool = False, frame_counts=None, _plan: dict | None = None) -> StepResult:
+        """Signals-only entry: samples float64 [S, T, R] (already ROI-sampled), timestamps float64 [S, T].
+        frame_counts: as in `step`; stream s takes rows [:n_s] of its samples and timestamps, the others are not read."""
         S, T, R = samples.shape
         self._check_step(S, T)
         if R != self.R or tuple(timestamps.shape) != (S, T):
             raise ValueError(f'step_signals: samples must be [S, T, {self.R}] and timestamps [S, T]')
+        n = self._frame_counts(frame_counts, T)
+        if n is not None and not n.any():
+            return self._empty_step(samples)
+        if _plan is None and not self._lockstep(n, T):
+            _plan = self._plan(n, T)
         with torch.cuda.device(self.device):
-            return self._step_signals(samples, timestamps, S, T, _count_roi, _designed)
+            return self._step_signals(samples, timestamps, S, T, _count_roi, _designed, _plan)
 
-    def _step_signals(self, samples, timestamps, S, T, _count_roi, _designed) -> StepResult:
+    def _empty_step(self, samples) -> StepResult:
+        """The result of a step in which no stream takes a frame: zero jobs, nothing enqueued, no state changed."""
+        dev, f64, f32, i32 = self.device, torch.float64, torch.float32, torch.int32
+        R, P, W = self.R, self.P, self.W
+        e = lambda *shape, dt=f64: torch.empty(shape, dtype=dt, device=dev)
+        arrays, means = {}, {}
+        if self.store_arrays:
+            arrays = dict(proc_x=e(0, R, W), proc_y=e(0, R, W), freqs=e(0, R, self._mb, dt=f32), mags=e(0, R, self._mb, dt=f32),
+                          num_bins=e(0, R, dt=i32), lags=e(0, P, 2 * W - 1, dt=f32), corr=e(0, P, 2 * W - 1, dt=f32),
+                          num_lags=e(0, P, dt=i32))
+        if self.peak_max_samples:
+            means = dict(mean_bpm=e(0, R), mean_bpm_int=e(0, R))
+            if P:
+                means.update(mean_ptt=e(0, P), mean_ptt_int=e(0, P))
+        self.launches_per_step = 0
+        return StepResult(None, samples, e(0, R), e(0, R, dt=i32), e(0, R), e(0, P), e(0, P, dt=i32), e(0, P), e(0, R, dt=i32),
+                          arrays, means, _job_offsets=np.zeros(self.S + 1, dtype=np.int64), _job_stream=e(0, dt=i32))
+
+    def _outputs(self, turn: int, J: int):
+        """F3 / F4 output dicts of a step: views of the first J rows of result turn `turn`'s Jmax-row buffers."""
+        if self._out[turn] is None:
+            pm = ops.jobs_params(self._params(0, 1, 1), self._Jmax)
+            self._out[turn] = (ops._spectrum_out(pm, self.store_arrays, None, self.device),
+                               ops._xcorr_out(pm, self.store_arrays, None, self.device))
+        return [{k: None if v is None else v[:J] for k, v in d.items()} for d in self._out[turn]]
+
+    def _step_signals(self, samples, timestamps, S, T, _count_roi, _designed, plan=None) -> StepResult:
         main = torch.cuda.current_stream(self.device)
         turn = self._turn
         self._turn = (turn + 1) % self._nbuf
-        ops.ring_push(self.ring_t, self.ring_y, self.count, None if _designed else timestamps.contiguous(), samples.contiguous())
-        g0 = self.count
-        self.count += T
-        jobs = T if self.windows == EVERY_FRAME else 1
-        head0 = g0 if self.windows == EVERY_FRAME else g0 + T - 1
-        p = self._params(head0, 1, jobs)
-        J = S * jobs
+        has_filter = any(m in (_cabi.FILTER_BUTTER, _cabi.FILTER_FIR) for m in self.methods)
+        if plan is None:
+            ops.ring_push(self.ring_t, self.ring_y, self._cnt, None if _designed else timestamps.contiguous(), samples.contiguous())
+            g0 = self._cnt
+            self._cnt += T
+            self._g0_ok = False
+            jobs = T if self.windows == EVERY_FRAME else 1
+            head0 = g0 if self.windows == EVERY_FRAME else g0 + T - 1
+            p = self._params(head0, 1, jobs)
+            pj, J = p, S * jobs
+        else:
+            # job-map path: stream s pushes n_s frames and owns jobs job_offsets[s]:job_offsets[s+1]; F3 / F4 see the J jobs
+            # as J streams of one job (include/bpv.h)
+            if not plan['mapped']:
+                self._map_jobs(plan, turn)
+            ops.ring_push_ragged(self.ring_t, self.ring_y, self._g0[0], self._ndev, None if _designed else timestamps.contiguous(),
+                                 samples.contiguous())
+            jobs, J = None, plan['J']
+            p = self._params(0, 1, 1)
+            pj = ops.jobs_params(p, J)
+            js, jh, sj0 = self._jobmap[turn]
         proc = self._proc[turn % len(self._proc)]
         px, py, st = proc[0, :J], proc[1, :J], self._status[turn][:J]
-        has_filter = any(m in (_cabi.FILTER_BUTTER, _cabi.FILTER_FIR) for m in self.methods)
         if _designed:
             main.wait_event(self._ev['design'])
-        elif has_filter:
+        elif has_filter and plan is None:
             ops.window_design(self.ring_t, p, self._ws, self._cache())
-        ops.window_filter(self.ring_t, self.ring_y, p, self._ws, px, py, st, cache=self._dcache if has_filter else None)
-        spo, xco = self._spec[turn], self._xc[turn]
-        spo = None if spo is None or spo['peak_idx'].shape[0] != J else spo
-        xco = None if xco is None or xco['lag_idx'].shape[0] != J else xco
+        elif has_filter:
+            ops.window_design_jobs(self.ring_t, p, self._ws, js, jh, J, self._cache())
+        if plan is None:
+            ops.window_filter(self.ring_t, self.ring_y, p, self._ws, px, py, st, cache=self._dcache if has_filter else None)
+        else:
+            ops.window_filter_jobs(self.ring_t, self.ring_y, p, self._ws, js, jh, J, px, py, st,
+                                   cache=self._dcache if has_filter else None)
+        spo, xco = self._outputs(turn, J)
+        p = pj
         # (windows over 320 samples: the entry point itself runs the two stand-alone launches, on this stream)
         fb, lb = ops.peak_band(self.freq_band, 'freq_band'), ops.peak_band(self.lag_band, 'lag_band')
         fused = (bool(self.overlap & OVERLAP_FUSED) and self.P > 0 and self.transform == _cabi.PGRAM_WELCH
@@ -362,7 +568,6 @@ class BatchedSignalProcessor:
         else:
             sp = ops.window_spectrum(px, py, p, store=self.store_arrays, workspace=self._ws_spec, out=spo, band=fb)
             xc = ops.window_xcorr(px, py, p, store=self.store_arrays, out=xco, band=lb)
-        self._spec[turn], self._xc[turn] = sp, xc
         if not self.store_arrays and self.discard_scratch:
             # the processed windows are dead now: drop their dirty L2 lines instead of letting the next step's ROI sampling
             # push them out to DRAM (F1 64.5 -> 69.7 us with 80 MB of dirty scratch in L2, profiles/r2p_f1_dirty.txt)
@@ -378,7 +583,7 @@ class BatchedSignalProcessor:
             interp = any(m in (_cabi.INTERP_LINEAR, _cabi.INTERP_CUBIC) for m in self.methods)
             if (env[:1] == '1') if env is not None else interp:
                 n_spec = 6              # dft_image + seal + dft_split + dft_tc_tma2 + dft_peak kernels + spectrum_dense_kernel for the flagged windows
-        n_push = 2 if _designed else 1
+        n_push = (2 if _designed else 1) + (0 if plan is None else 1)          # (+ the job map)
         self.launches_per_step = (1 + self._extra_launches if _count_roi else 0) + n_push + n_pre + n_spec + (1 if self.P and not (fused and self.W <= 320) else 0)
         if not self.store_arrays and self.discard_scratch:
             self.launches_per_step += 1 if J == self._Jmax else 2
@@ -387,16 +592,35 @@ class BatchedSignalProcessor:
             arrays = dict(proc_x=px, proc_y=py, freqs=sp['freqs'], mags=sp['mags'], num_bins=sp['num_bins'],
                           lags=xc['lags'], corr=xc['corr'], num_lags=xc['num_lags'])
         means = {}
-        if self.peak_max_samples:
-            mb, mbi = ops.running_mean(self._bpm_ring, self._mean_count, sp['peak_freq'].view(S, jobs, self.R), 60.0)
+        if self.peak_max_samples and plan is None:
+            mb, mbi = ops.running_mean(self._bpm_ring, self._mcnt, sp['peak_freq'].view(S, jobs, self.R), 60.0)
             means = dict(mean_bpm=mb.view(J, self.R), mean_bpm_int=mbi.view(J, self.R))
             if self.P:
-                mp, mpi = ops.running_mean(self._ptt_ring, self._mean_count, xc['lag_sec'].view(S, jobs, self.P), 1000.0)
+                mp, mpi = ops.running_mean(self._ptt_ring, self._mcnt, xc['lag_sec'].view(S, jobs, self.P), 1000.0)
                 means.update(mean_ptt=mp.view(J, self.P), mean_ptt_int=mpi.view(J, self.P))
-            self._mean_count += jobs
+            self._mcnt += jobs
             self.launches_per_step += 2 if self.P else 1
-        return StepResult(jobs, samples, sp['peak_freq'], sp['peak_idx'], sp['peak_mag'], xc['lag_sec'], xc['lag_idx'],
-                          xc['lag_corr'], st, arrays, means)
+        elif self.peak_max_samples:
+            mcnt = np.full(self.S, self._mcnt, dtype=np.int64) if isinstance(self._mcnt, int) else self._mcnt
+            pin = self._pinned(turn)
+            pin['m0'].numpy()[:] = mcnt
+            self._mg0.copy_(pin['m0'], non_blocking=True)
+            mb, mbi = ops.running_mean_jobs(self._bpm_ring, self._mg0, sj0, sp['peak_freq'], 60.0)
+            means = dict(mean_bpm=mb, mean_bpm_int=mbi)
+            if self.P:
+                mp, mpi = ops.running_mean_jobs(self._ptt_ring, self._mg0, sj0, xc['lag_sec'], 1000.0)
+                means.update(mean_ptt=mp, mean_ptt_int=mpi)
+            self._mcnt = self._level(mcnt + plan['jobs'])
+            self.launches_per_step += 2 if self.P else 1
+        if plan is None:
+            return StepResult(jobs, samples, sp['peak_freq'], sp['peak_idx'], sp['peak_mag'], xc['lag_sec'], xc['lag_idx'],
+                              xc['lag_corr'], st, arrays, means)
+        self._staging[turn]['ev'].record(main)
+        self._staging[turn]['used'] = True
+        self._cnt = self._level(self.counts + plan['n'])
+        self._g0.reverse()                      # bpv_stream_jobs left the advanced counts in the other buffer
+        return StepResult(None, samples, sp['peak_freq'], sp['peak_idx'], sp['peak_mag'], xc['lag_sec'], xc['lag_idx'],
+                          xc['lag_corr'], st, arrays, means, _job_offsets=plan['off'], _job_stream=js[:J])
 
     # ------------------------------------------------------------------------------------------
     # SURVEY.md §8(f) row 3: snapshot / resume of the per-stream state (the reference's deepcopy(store), :313, is the
@@ -406,18 +630,28 @@ class BatchedSignalProcessor:
                     roi_max_samples=0 if self._roi_hist is None else int(self._roi_hist.shape[2]))
 
     def state_dict(self) -> dict:
-        """Everything a run needs to continue bit-for-bit: raw-sample rings and their count, the bpm / ptt histories of
-        the running means, the ROI smoothing history.  Tensors are copied to the host."""
+        """Everything a run needs to continue bit-for-bit: raw-sample rings and their per-stream counts, the bpm / ptt
+        histories of the running means and their per-stream lengths, the ROI smoothing history.  Tensors and counts are
+        copied to the host."""
         torch.cuda.synchronize(self.device)
         cpu = lambda t: None if t is None else t.detach().to('cpu', copy=True)
-        return dict(version=STATE_VERSION, signature=self._signature(), count=int(self.count),
+        mcnt = np.full(self.S, self._mcnt, dtype=np.int64) if isinstance(self._mcnt, int) else self._mcnt.copy()
+        return dict(version=STATE_VERSION, signature=self._signature(), counts=self.counts,
                     ring_t=cpu(self.ring_t), ring_y=cpu(self.ring_y),
-                    mean_count=int(self._mean_count), bpm_ring=cpu(self._bpm_ring), ptt_ring=cpu(self._ptt_ring),
+                    mean_counts=mcnt, bpm_ring=cpu(self._bpm_ring), ptt_ring=cpu(self._ptt_ring),
                     roi_count=int(self._roi_count), roi_hist=cpu(self._roi_hist))
 
     def load_state_dict(self, state: dict) -> None:
-        if state.get('version') != STATE_VERSION:
-            raise ValueError(f"load_state_dict: unsupported state version {state.get('version')!r}")
+        """Load a state_dict() of an engine of the same geometry; version 1 states (one count for every stream) load too."""
+        version = state.get('version')
+        if version not in (1, STATE_VERSION):
+            raise ValueError(f"load_state_dict: unsupported state version {version!r}")
+        if version == 1:
+            counts, mcnt = np.full(self.S, int(state['count']), np.int64), np.full(self.S, int(state['mean_count']), np.int64)
+        else:
+            counts, mcnt = np.asarray(state['counts'], dtype=np.int64), np.asarray(state['mean_counts'], dtype=np.int64)
+            if counts.shape != (self.S,) or mcnt.shape != (self.S,):
+                raise ValueError(f'load_state_dict: counts of {counts.shape} / {mcnt.shape} streams, expected ({self.S},)')
         if state['signature'] != self._signature():
             raise ValueError(f"load_state_dict: state of a different engine geometry {state['signature']} != {self._signature()}")
 
@@ -433,15 +667,36 @@ class BatchedSignalProcessor:
         put(self._bpm_ring, state['bpm_ring'], 'bpm_ring')
         put(self._ptt_ring, state['ptt_ring'], 'ptt_ring')
         put(self._roi_hist, state['roi_hist'], 'roi_hist')
-        self.count, self._mean_count, self._roi_count = int(state['count']), int(state['mean_count']), int(state['roi_count'])
+        self._cnt, self._mcnt, self._roi_count = self._level(counts), self._level(mcnt), int(state['roi_count'])
+        self._g0_ok = False
 
-    def reset(self):
-        """Back to the state of a freshly constructed engine: empty rings AND empty bpm / ptt / ROI histories."""
+    def reset(self, streams=None):
+        """Back to the state of a freshly constructed engine: empty rings AND empty bpm / ptt / ROI histories.
+        streams = indices of some streams (e.g. cameras that disconnected): only their ring rows, bpm / ptt history rows and
+        ROI smoothing rows are emptied and their counts zeroed; every other stream keeps its state bit for bit."""
         nan = float('nan')
-        self.ring_t.fill_(nan)
-        self.ring_y.fill_(nan)
-        self.count = 0
-        for t in (self._bpm_ring, self._ptt_ring, self._roi_hist):
+        if streams is None:
+            self.ring_t.fill_(nan)
+            self.ring_y.fill_(nan)
+            self.count = 0
+            for t in (self._bpm_ring, self._ptt_ring, self._roi_hist):
+                if t is not None:
+                    t.fill_(nan)
+            self._mcnt = self._roi_count = 0
+            return
+        idx = np.unique(np.asarray(streams, dtype=np.int64).reshape(-1))
+        if idx.size and (idx[0] < 0 or idx[-1] >= self.S):
+            raise ValueError(f'reset: stream indices must lie in [0, {self.S})')
+        if not idx.size:
+            return
+        rows = torch.from_numpy(idx).to(self.device)
+        for t in (self.ring_t, self.ring_y, self._bpm_ring, self._ptt_ring, self._roi_hist):
             if t is not None:
-                t.fill_(nan)
-        self._mean_count = self._roi_count = 0
+                t.index_fill_(0, rows, nan)
+        counts = self.counts
+        counts[idx] = 0
+        self._cnt = self._level(counts)
+        mcnt = np.full(self.S, self._mcnt, dtype=np.int64) if isinstance(self._mcnt, int) else self._mcnt.copy()
+        mcnt[idx] = 0
+        self._mcnt = self._level(mcnt)
+        self._g0_ok = False

@@ -112,6 +112,44 @@ def ring_push(ring_t: torch.Tensor, ring_y: torch.Tensor, g0: int, ts: torch.Ten
     _run(ring_y.device, 'bpv_ring_push', ptr(ring_t), ptr(ring_y), S, R, cap, int(g0), T, ptr(ts), ptr(values))
 
 
+def ring_push_ragged(ring_t, ring_y, g0: torch.Tensor, n: torch.Tensor, ts: torch.Tensor | None, values: torch.Tensor | None):
+    """Ragged push (include/bpv.h bpv_ring_push_ragged): stream s appends its first n[s] rows of ts f64 [S,T] / values
+    f64 [S,T,R] at global indices g0[s] ...  g0 int64 [S], n int32 [S] on the device; g0 is not advanced."""
+    S, R, cap = ring_y.shape
+    if ts is None and values is None:
+        raise ValueError('ring_push_ragged: nothing to push')
+    T = ts.shape[1] if ts is not None else values.shape[1]
+    _require(ts is None or (tuple(ts.shape) == (S, T) and ts.is_contiguous()), 'ring_push_ragged: ts must be a contiguous [S, T] tensor')
+    _require(values is None or (tuple(values.shape) == (S, T, R) and values.is_contiguous()),
+             'ring_push_ragged: values must be a contiguous [S, T, R] tensor')
+    _require(g0.dtype == torch.int64 and n.dtype == torch.int32 and g0.numel() == n.numel() == S, 'ring_push_ragged: g0 int64 [S], n int32 [S]')
+    _run(ring_y.device, 'bpv_ring_push_ragged', ptr(ring_t), ptr(ring_y), S, R, cap, ptr(g0), ptr(n), T, ptr(ts), ptr(values))
+
+
+def stream_jobs(g0: torch.Tensor, n: torch.Tensor, last_only: bool, num_jobs: int, job_stream: torch.Tensor,
+                job_head: torch.Tensor, stream_job0: torch.Tensor, g0_next: torch.Tensor) -> None:
+    """Job map of a ragged step on the device (include/bpv.h bpv_stream_jobs): job_stream i32 / job_head i64 [>= num_jobs],
+    stream_job0 i32 [S+1], g0_next i64 [S] = g0 + n.  num_jobs must be the sum of the job counts."""
+    S = g0.numel()
+    _require(n.numel() == S and stream_job0.numel() == S + 1 and g0_next.numel() == S, 'stream_jobs: sizes do not match')
+    _require(job_stream.numel() >= num_jobs and job_head.numel() >= num_jobs, 'stream_jobs: job map buffers too small')
+    _run(g0.device, 'bpv_stream_jobs', S, ptr(g0), ptr(n), int(bool(last_only)), int(num_jobs), ptr(job_stream), ptr(job_head),
+         ptr(stream_job0), ptr(g0_next))
+
+
+def running_mean_jobs(ring, g0: torch.Tensor, stream_job0: torch.Tensor, values, scale: float):
+    """running_mean over the job map of a ragged step (include/bpv.h bpv_running_mean_jobs): values [J,C]; returns (mean,
+    mean_int) f64 [J,C].  g0 int64 [S] = the streams' history counts (not advanced)."""
+    S, C_, H = ring.shape
+    J = values.shape[0]
+    _require(values.dim() == 2 and values.shape[1] == C_ and values.is_contiguous(), 'running_mean_jobs: values must be [J, C]')
+    mean = torch.empty((J, C_), dtype=torch.float64, device=ring.device)
+    mean_int = torch.empty((J, C_), dtype=torch.float64, device=ring.device)
+    _run(ring.device, 'bpv_running_mean_jobs', ptr(ring), S, C_, H, ptr(g0), ptr(stream_job0), ptr(values), float(scale),
+         ptr(mean), ptr(mean_int))
+    return mean, mean_int
+
+
 def make_params(S, R, cap, window, head0, head_step, jobs_per_stream, methods, transform, *, butter_order=16,
                 butter_min_bw=0.1, fir_taps=127, fir_df=0.3, min_freq=0.8, max_freq=4.0, ls_num_freqs=0) -> WindowParams:
     p = WindowParams()
@@ -167,6 +205,31 @@ def window_filter(ring_t, ring_y, p: WindowParams, workspace, proc_x=None, proc_
     proc_x, proc_y, status, workspace = _pre_buffers(ring_y, p, proc_x, proc_y, status, workspace)
     _run(ring_y.device, 'bpv_window_filter', ptr(ring_t), ptr(ring_y), C.byref(p), ptr(workspace), workspace.numel(),
          ptr(cache), 0 if cache is None else cache.numel(), ptr(proc_x), ptr(proc_y), ptr(status))
+    return proc_x, proc_y, status
+
+
+def jobs_params(p: WindowParams, num_jobs: int) -> WindowParams:
+    """The params F3 / F4 (and the per-job output shapes) see for the num_jobs jobs of a job map: S = num_jobs,
+    jobs_per_stream = 1 (include/bpv.h: F3 and F4 only use S * jobs_per_stream)."""
+    q = WindowParams.from_buffer_copy(p)
+    q.S, q.jobs_per_stream, q.head0, q.head_step = int(num_jobs), 1, 0, 0
+    return q
+
+
+def window_design_jobs(ring_t, p: WindowParams, workspace, job_stream, job_head, num_jobs: int, cache=None):
+    """window_design over a job map (include/bpv.h bpv_window_design_jobs): p describes the rings."""
+    _run(ring_t.device, 'bpv_window_design_jobs', ptr(ring_t), C.byref(p), ptr(workspace), workspace.numel(),
+         ptr(cache), 0 if cache is None else cache.numel(), ptr(job_stream), ptr(job_head), int(num_jobs))
+
+
+def window_filter_jobs(ring_t, ring_y, p: WindowParams, workspace, job_stream, job_head, num_jobs: int, proc_x=None, proc_y=None,
+                       status=None, cache=None):
+    """window_filter over a job map (include/bpv.h bpv_window_filter_jobs).  Returns proc_x, proc_y f64 [J,R,window],
+    status i32 [J,R] for the J = num_jobs jobs."""
+    proc_x, proc_y, status, workspace = _pre_buffers(ring_y, jobs_params(p, num_jobs), proc_x, proc_y, status, workspace)
+    _run(ring_y.device, 'bpv_window_filter_jobs', ptr(ring_t), ptr(ring_y), C.byref(p), ptr(workspace), workspace.numel(),
+         ptr(cache), 0 if cache is None else cache.numel(), ptr(proc_x), ptr(proc_y), ptr(status), ptr(job_stream), ptr(job_head),
+         int(num_jobs))
     return proc_x, proc_y, status
 
 

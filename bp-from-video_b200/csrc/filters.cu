@@ -282,12 +282,16 @@ __global__ void __launch_bounds__(FIRLS_THREADS) firls_from_fs_kernel(const doub
 }
 
 // ---- per-job design from the ring timestamps (used by the window pipeline) ----------------------
-__global__ void job_butter_kernel(const double* __restrict__ ring_t, bpv_window_params p, double* __restrict__ sos_out) {
+// JMAP: the job's ring row and newest sample come from the job map (filters.cuh JobMap), else from head0 / head_step
+template <bool JMAP>
+__global__ void job_butter_kernel(const double* __restrict__ ring_t, bpv_window_params p, double* __restrict__ sos_out,
+                                  const JobMap jm) {
   const int job = blockIdx.x * blockDim.x + threadIdx.x;
   const int J = p.S * p.jobs_per_stream;
   if (job >= J) return;
-  const int s = job / p.jobs_per_stream, j = job % p.jobs_per_stream;
-  const double fs = job_fs(ring_t + (long long)s * p.cap, p.cap, p.window, p.head0 + (long long)j * p.head_step, nullptr);
+  const int s = JMAP ? jm.stream[job] : job / p.jobs_per_stream, j = JMAP ? 0 : job % p.jobs_per_stream;
+  const long long head = JMAP ? (long long)jm.head[job] : p.head0 + (long long)j * p.head_step;
+  const double fs = job_fs(ring_t + (long long)s * p.cap, p.cap, p.window, head, nullptr);
   double sos[MAX_SOS * 6];
   if (isfinite(fs)) butter_bandpass_sos(fs, p.butter_order, p.min_freq, p.max_freq, p.butter_min_bw, sos);
   else for (int k = 0; k < p.butter_order * 6; ++k) sos[k] = nan_f64();
@@ -296,10 +300,12 @@ __global__ void job_butter_kernel(const double* __restrict__ ring_t, bpv_window_
 
 // fs of a job's window, cooperative over a group of FIRLS_LPD lanes (first / last finite timestamp and their count); every
 // lane of the group returns the same value.  Same arithmetic as job_fs.
-__device__ __forceinline__ double group_job_fs(const double* __restrict__ ring_t, const bpv_window_params& p, int job, int sub) {
-  const int s = job / p.jobs_per_stream, j = job % p.jobs_per_stream;
+template <bool JMAP>
+__device__ __forceinline__ double group_job_fs(const double* __restrict__ ring_t, const bpv_window_params& p, int job, int sub,
+                                               const JobMap& jm) {
+  const int s = JMAP ? jm.stream[job] : job / p.jobs_per_stream, j = JMAP ? 0 : job % p.jobs_per_stream;
   const double* rt = ring_t + (long long)s * p.cap;
-  const long long g0 = p.head0 + (long long)j * p.head_step - p.window + 1;
+  const long long g0 = (JMAP ? (long long)jm.head[job] : p.head0 + (long long)j * p.head_step) - p.window + 1;
   int lo = 0x7fffffff, hi = -1, cnt = 0;
   const int kmin = g0 < 0 ? (int)(-g0 < p.window ? -g0 : p.window) : 0;
   const int slot0 = (int)(((g0 % p.cap) + p.cap) % p.cap);
@@ -326,14 +332,15 @@ __device__ __forceinline__ double group_job_fs(const double* __restrict__ ring_t
   return fs;
 }
 
+template <bool JMAP>
 __global__ void __launch_bounds__(FIRLS_THREADS) job_firls_kernel(const double* __restrict__ ring_t, bpv_window_params p,
-                                                                  double* __restrict__ out) {
+                                                                  double* __restrict__ out, const JobMap jm) {
   extern __shared__ double smem[];
   const int d = threadIdx.x / FIRLS_LPD, sub = threadIdx.x & (FIRLS_LPD - 1);
   const int job = blockIdx.x * FIRLS_DPB + d;
   const bool live = job < p.S * p.jobs_per_stream;
   // padding groups shadow job 0 (warp-uniform control flow), write nothing
-  const double fs = group_job_fs(ring_t, p, live ? job : 0, sub);
+  const double fs = group_job_fs<JMAP>(ring_t, p, live ? job : 0, sub, jm);
   double* o = out + (long long)(live ? job : 0) * FIR_WS_STRIDE;      // taps [128] | lfilter_zi [128] | merged taps [FIR_MERGED_LEN]
   firls_design_group(fs, live, p.fir_taps, p.min_freq, p.max_freq, p.fir_df, o, o + 128, o + 256, smem + firls_smem_offset(d));
 }
@@ -362,13 +369,14 @@ __device__ __forceinline__ unsigned dc_hash(unsigned long long k) {
   return (unsigned)k & (DC_SLOTS - 1);
 }
 
+template <bool JMAP>
 __global__ void __launch_bounds__(256) design_probe_kernel(const double* __restrict__ ring_t, const bpv_window_params p,
                                                            unsigned char* __restrict__ cache, int32_t* __restrict__ ref,
-                                                           DesignMiss* __restrict__ miss) {
+                                                           DesignMiss* __restrict__ miss, const JobMap jm) {
   const int J = p.S * p.jobs_per_stream;
   const int job = (blockIdx.x * blockDim.x + threadIdx.x) / FIRLS_LPD, sub = threadIdx.x & (FIRLS_LPD - 1);
   const bool live = job < J;
-  const double fs = group_job_fs(ring_t, p, live ? job : 0, sub);
+  const double fs = group_job_fs<JMAP>(ring_t, p, live ? job : 0, sub, jm);
   if (!live || sub != 0) return;
   unsigned int* counter = reinterpret_cast<unsigned int*>(cache);
   unsigned long long* keys = reinterpret_cast<unsigned long long*>(cache + DC_HDR_BYTES);
@@ -444,27 +452,32 @@ __global__ void miss_butter_kernel(const bpv_window_params p, unsigned char* __r
 
 constexpr size_t FIRLS_SMEM = (size_t)(firls_smem_offset(FIRLS_DPB - 1) + FIRLS_WS) * sizeof(double);
 
-int launch_job_butter(const double* ring_t, const bpv_window_params& p, double* sos_out, cudaStream_t st) {
+// jm = NULL: the lockstep instantiations (head0 / head_step); else the job-map ones
+int launch_job_butter(const double* ring_t, const bpv_window_params& p, double* sos_out, cudaStream_t st, const JobMap* jm) {
   const int J = p.S * p.jobs_per_stream;
-  job_butter_kernel<<<(J + 63) / 64, 64, 0, st>>>(ring_t, p, sos_out);
+  if (jm) job_butter_kernel<true><<<(J + 63) / 64, 64, 0, st>>>(ring_t, p, sos_out, *jm);
+  else job_butter_kernel<false><<<(J + 63) / 64, 64, 0, st>>>(ring_t, p, sos_out, JobMap{});
   return check_launch("job_butter_kernel");
 }
 
-int launch_job_firls(const double* ring_t, const bpv_window_params& p, double* taps_out, cudaStream_t st) {
+int launch_job_firls(const double* ring_t, const bpv_window_params& p, double* taps_out, cudaStream_t st, const JobMap* jm) {
   const int J = p.S * p.jobs_per_stream;
-  job_firls_kernel<<<(J + FIRLS_DPB - 1) / FIRLS_DPB, FIRLS_THREADS, FIRLS_SMEM, st>>>(ring_t, p, taps_out);
+  if (jm) job_firls_kernel<true><<<(J + FIRLS_DPB - 1) / FIRLS_DPB, FIRLS_THREADS, FIRLS_SMEM, st>>>(ring_t, p, taps_out, *jm);
+  else job_firls_kernel<false><<<(J + FIRLS_DPB - 1) / FIRLS_DPB, FIRLS_THREADS, FIRLS_SMEM, st>>>(ring_t, p, taps_out, JobMap{});
   return check_launch("job_firls_kernel");
 }
 
 // Cached design of every window job: probe + design of the misses.  ref int32 [J] and the miss list live in the caller's
 // workspace (window_pre.cu lays it out); `cache` is the persistent table (zero-initialised by its owner).
 int launch_design_cached(const double* ring_t, const bpv_window_params& p, bool butter, bool fir, unsigned char* cache,
-                         int32_t* ref, void* miss, double* ws_sos, double* ws_fir, cudaStream_t st) {
+                         int32_t* ref, void* miss, double* ws_sos, double* ws_fir, cudaStream_t st, const JobMap* jm) {
   const int J = p.S * p.jobs_per_stream;
   cudaError_t e = cudaMemsetAsync(cache, 0, 4, st);                       // the launch's miss counter
   if (e != cudaSuccess) { set_error("bpv_window_design: cudaMemsetAsync: %s", cudaGetErrorString(e)); return (int)e; }
   const long long threads = (long long)J * FIRLS_LPD;
-  design_probe_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(ring_t, p, cache, ref, (DesignMiss*)miss);
+  const unsigned blocks = (unsigned)((threads + 255) / 256);
+  if (jm) design_probe_kernel<true><<<blocks, 256, 0, st>>>(ring_t, p, cache, ref, (DesignMiss*)miss, *jm);
+  else design_probe_kernel<false><<<blocks, 256, 0, st>>>(ring_t, p, cache, ref, (DesignMiss*)miss, JobMap{});
   if (int rc = check_launch("design_probe_kernel")) return rc;
   if (butter) {
     miss_butter_kernel<<<(J + 63) / 64, 64, 0, st>>>(p, cache, (const DesignMiss*)miss, ws_sos, ws_fir);

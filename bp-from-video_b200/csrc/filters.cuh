@@ -17,6 +17,15 @@ constexpr long long DC_BYTES = DC_HDR_BYTES + (long long)DC_SLOTS * 8 + (long lo
 // status codes written to the per-signal status array
 constexpr int ST_OK = 0, ST_GUARD = 1, ST_CUBIC_X = 2, ST_BAD_BANDS = 3;
 
+// Job map of a ragged step (include/bpv.h bpv_stream_jobs): job k reads ring row stream[k], newest sample head[k].  The
+// window kernels take it behind a template switch JMAP; the JMAP = false instantiations locate job j of stream s at
+// head0 + j * head_step as before and never read the map.  With JMAP the launch's params carry S = number of jobs and
+// jobs_per_stream = 1, so every per-job layout is the lockstep one over the job list.
+struct JobMap {
+  const int32_t* stream;
+  const int64_t* head;
+};
+
 struct cplx { double re, im; };
 __device__ __forceinline__ cplx cmul(cplx a, cplx b) { return {a.re * b.re - a.im * b.im, a.re * b.im + a.im * b.re}; }
 __device__ __forceinline__ cplx cdiv(cplx a, cplx b) {

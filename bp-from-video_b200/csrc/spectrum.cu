@@ -627,8 +627,9 @@ __global__ void __launch_bounds__(32 * LSP_WPB) ls_peak_warp_kernel(const double
 
 }  // namespace bpv
 
-// workspace plan: [coarse magnitudes / LS psd when the spectrum is not stored, rounded up to 256 B] [DFT_RFFT on the tensor
-// cores: the twiddle operand images of dft_tc.cu — persistent across calls, zero-initialised once by the caller]
+// workspace plan: [DFT_RFFT on the tensor cores: the twiddle operand images of dft_tc.cu — persistent across calls,
+// zero-initialised once by the caller; FIRST, so that they stay where they were built whatever the launch's job count]
+// [coarse magnitudes / LS psd when the spectrum is not stored, rounded up to 256 B] [DFT_RFFT: this launch's split samples]
 static int64_t spectrum_coarse_bytes(const bpv_window_params* p, int32_t max_bins) {
   if (p->transform == BPV_PGRAM_WELCH) return 0;
   return ((int64_t)p->S * p->jobs_per_stream * p->R * max_bins * 4 + 255) / 256 * 256;
@@ -698,18 +699,22 @@ extern "C" int bpv_window_spectrum_band(const double* proc_x, const double* proc
       const char* env = getenv("BPV_DFT_TC");
       const bool use_tc = env ? env[0] == '1' : interp;
       if (use_tc) {
-        float* coarse = spec_mag;
+        // the twiddle operand images open the workspace when it has room for them (and for the coarse area, if the spectrum is
+        // not stored): their offset must not depend on the launch's job count, or a launch of another J would find a stale
+        // header over overwritten images.  Behind them the coarse area, then the hi / lo images of this launch's samples
+        // (A operand) when there is room for those too.
         const int64_t cb = spectrum_coarse_bytes(p, max_bins);
+        const int64_t ib = (dft_tc_image_bytes(W) + 255) / 256 * 256;
+        const int64_t need_coarse = spec_mag ? 0 : cb;
+        void* images = (workspace && workspace_bytes >= ib + need_coarse) ? workspace : nullptr;
+        unsigned char* rest = (unsigned char*)workspace + (images ? ib : 0);
+        float* coarse = spec_mag;
         if (!coarse) {
           BPV_REQUIRE(workspace && workspace_bytes >= cb, BPV_E_INVALID,
                       "bpv_window_spectrum: workspace too small (see bpv_spectrum_workspace_bytes)");
-          coarse = (float*)workspace;
+          coarse = (float*)rest;
         }
-        // the twiddle operand images live behind the coarse area when the caller's workspace has room for them
-        // and behind them the hi / lo images of this launch's samples (A operand), when there is room for those too
-        const int64_t ib = (dft_tc_image_bytes(W) + 255) / 256 * 256;
-        void* images = (workspace && workspace_bytes >= cb + ib) ? (void*)((unsigned char*)workspace + cb) : nullptr;
-        void* split = (images && workspace_bytes >= cb + ib + dft_tc_split_bytes(W, nsig)) ? (void*)((unsigned char*)workspace + cb + ib) : nullptr;
+        void* split = (images && workspace_bytes >= ib + need_coarse + dft_tc_split_bytes(W, nsig)) ? (void*)(rest + need_coarse) : nullptr;
         if (int rc = launch_dft_tc(proc_x, proc_y, W, nsig, max_bins, spec_f, coarse, num_bins, peak_idx, peak_freq, peak_mag, images, split,
                                    banded, band, st))
           return rc;

@@ -18,11 +18,11 @@
 
 namespace bpv {
 
-int launch_job_butter(const double* ring_t, const bpv_window_params& p, double* sos_out, cudaStream_t st);
-int launch_job_firls(const double* ring_t, const bpv_window_params& p, double* taps_out, cudaStream_t st);
+int launch_job_butter(const double* ring_t, const bpv_window_params& p, double* sos_out, cudaStream_t st, const JobMap* jm);
+int launch_job_firls(const double* ring_t, const bpv_window_params& p, double* taps_out, cudaStream_t st, const JobMap* jm);
 int check_filter_params(const bpv_window_params* p, const char* who);
 int launch_design_cached(const double* ring_t, const bpv_window_params& p, bool butter, bool fir, unsigned char* cache,
-                         int32_t* ref, void* miss, double* ws_sos, double* ws_fir, cudaStream_t st);
+                         int32_t* ref, void* miss, double* ws_sos, double* ws_fir, cudaStream_t st, const JobMap* jm);
 
 // Where a window job's filter coefficients live: in the design cache (ref[job] = slot) or in the job's own workspace slot.
 struct DesignRef {
@@ -734,10 +734,11 @@ __device__ __forceinline__ bool fs_is_finite(double xfirst, double xlast, int m)
 // Stage one signal's window: ring -> shared memory with ballot / popc compaction of the valid samples (Signal.reset_mask:
 // v = isfinite(x), w = isfinite(y); signal_data.py:43-45), writing the position-preserving pass-through copy on the way.
 // Returns ST_OK, or ST_GUARD when the reference's guard (signal_processor.py:200) leaves the window unprocessed.
-template <int FEAT>
+// JMAP: the job's ring row and newest sample come from the job map (filters.cuh JobMap).
+template <int FEAT, bool JMAP>
 __device__ int gather_window(Warp& w, unsigned char* sm, const PreLayout& L, const bpv_window_params& p,
                              const double* __restrict__ ring_t, const double* __restrict__ ring_y, long long sig,
-                             double* __restrict__ ox, double* __restrict__ oy) {
+                             double* __restrict__ ox, double* __restrict__ oy, const JobMap& jm) {
   // xv / posb exist in the shared-memory plan only when the method list resamples (an instantiation may serve a subset
   // of its stages)
   bool has_interp = false;
@@ -755,8 +756,8 @@ __device__ int gather_window(Warp& w, unsigned char* sm, const PreLayout& L, con
   w.fir_c = L.fir_c; w.fir_gt = L.fir_gt; w.fir_b = L.fir_b;
   const long long job = sig / p.R;
   const int r = (int)(sig % p.R);
-  const int s = (int)(job / p.jobs_per_stream), j = (int)(job % p.jobs_per_stream);
-  const long long head = p.head0 + (long long)j * p.head_step;
+  const int s = JMAP ? jm.stream[job] : (int)(job / p.jobs_per_stream), j = JMAP ? 0 : (int)(job % p.jobs_per_stream);
+  const long long head = JMAP ? (long long)jm.head[job] : p.head0 + (long long)j * p.head_step;
   const double* rt = ring_t + (long long)s * p.cap;
   const double* ry = ring_y + ((long long)s * p.R + r) * p.cap;
   const int W = p.window;
@@ -878,13 +879,13 @@ __device__ __forceinline__ void prefetch_filters(int FEAT, int lane, const bpv_w
 // DUAL = false: one warp per signal.  DUAL = true (every instantiation with FILTER_BUTTER): one warp per PAIR of
 // consecutive signals — the single-signal stages run for one and then the other, the Butterworth cascade for both at once
 // (sos_filtfilt_dual); the warp's shared-memory slice holds two per-signal plans.
-template <int FEAT, int MINB, bool DUAL>
+template <int FEAT, int MINB, bool DUAL, bool JMAP>
 __global__ void __launch_bounds__(128, MINB) window_preprocess_kernel(const double* __restrict__ ring_t,
                                                                       const double* __restrict__ ring_y,
                                                                       const bpv_window_params p, const PreLayout L,
                                                                       const DesignRef dr,
                                                                       double* __restrict__ proc_x, double* __restrict__ proc_y,
-                                                                      int32_t* __restrict__ status) {
+                                                                      int32_t* __restrict__ status, const JobMap jm) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int wib = threadIdx.x >> 5, wpb = blockDim.x >> 5;
   const long long unit = (long long)blockIdx.x * wpb + wib;
@@ -900,7 +901,7 @@ __global__ void __launch_bounds__(128, MINB) window_preprocess_kernel(const doub
     prefetch_filters(FEAT, lane, p, dr, job);
     double* ox = proc_x + sig * W;
     double* oy = proc_y + sig * W;
-    int st = gather_window<FEAT>(w, smem_raw + (size_t)wib * L.total, L, p, ring_t, ring_y, sig, ox, oy);
+    int st = gather_window<FEAT, JMAP>(w, smem_raw + (size_t)wib * L.total, L, p, ring_t, ring_y, sig, ox, oy, jm);
     for (int mi = 0; mi < p.num_methods && st == ST_OK; ++mi) st = apply_method<FEAT>(w, p.methods[mi], p, dr, job);
     scatter_window(w, st, W, ox, oy, status, sig);
   } else {
@@ -915,9 +916,9 @@ __global__ void __launch_bounds__(128, MINB) window_preprocess_kernel(const doub
     unsigned char* sm = smem_raw + (size_t)wib * 2 * L.total;
     double* oxa = proc_x + sa * W; double* oya = proc_y + sa * W;
     double* oxb = proc_x + (hasb ? sb : sa) * W; double* oyb = proc_y + (hasb ? sb : sa) * W;
-    int sta = gather_window<FEAT>(wa, sm, L, p, ring_t, ring_y, sa, oxa, oya);
+    int sta = gather_window<FEAT, JMAP>(wa, sm, L, p, ring_t, ring_y, sa, oxa, oya, jm);
     int stb = ST_GUARD;
-    if (hasb) stb = gather_window<FEAT>(wb, sm + L.total, L, p, ring_t, ring_y, sb, oxb, oyb);
+    if (hasb) stb = gather_window<FEAT, JMAP>(wb, sm + L.total, L, p, ring_t, ring_y, sb, oxb, oyb, jm);
     else { wb = wa; }
     for (int mi = 0; mi < p.num_methods && (sta == ST_OK || stb == ST_OK); ++mi) {
       const int m = p.methods[mi];
@@ -939,7 +940,8 @@ __global__ void __launch_bounds__(128, MINB) window_preprocess_kernel(const doub
 
 template <int FEAT, int MINB, bool DUAL>
 static int launch_preprocess(const double* ring_t, const double* ring_y, const bpv_window_params& p, const PreLayout& L,
-                             const DesignRef& dr, double* proc_x, double* proc_y, int32_t* status, cudaStream_t st) {
+                             const DesignRef& dr, double* proc_x, double* proc_y, int32_t* status, cudaStream_t st,
+                             const JobMap* jm) {
   const int max_smem = 200 * 1024;
   const int per_warp = (DUAL ? 2 : 1) * L.total;                 // a warp holds one signal, or a pair of them
   BPV_REQUIRE(per_warp <= max_smem, BPV_E_TOO_LARGE, "bpv_window_preprocess: window %d needs %d B of shared memory per signal",
@@ -959,11 +961,12 @@ static int launch_preprocess(const double* ring_t, const double* ring_y, const b
     if (warps > best || (warps == best && c < wpb)) { best = warps; wpb = c; }
   }
   const size_t smem = (size_t)wpb * per_warp;
-  auto kern = window_preprocess_kernel<FEAT, MINB, DUAL>;
+  auto kern = jm ? window_preprocess_kernel<FEAT, MINB, DUAL, true> : window_preprocess_kernel<FEAT, MINB, DUAL, false>;
   if (int rc = ensure_dyn_smem((const void*)kern, smem)) return rc;
   const long long nsig = (long long)p.S * p.jobs_per_stream * p.R;
   const long long units = DUAL ? (nsig + 1) / 2 : nsig;
-  kern<<<(unsigned)((units + wpb - 1) / wpb), wpb * 32, smem, st>>>(ring_t, ring_y, p, L, dr, proc_x, proc_y, status);
+  kern<<<(unsigned)((units + wpb - 1) / wpb), wpb * 32, smem, st>>>(ring_t, ring_y, p, L, dr, proc_x, proc_y, status,
+                                                                    jm ? *jm : JobMap{});
   return check_launch("bpv_window_preprocess");
 }
 
@@ -1005,9 +1008,9 @@ extern "C" int64_t bpv_window_workspace_bytes(const bpv_window_params* p) {
 
 extern "C" int64_t bpv_design_cache_bytes(void) { return bpv::DC_BYTES; }
 
-extern "C" int bpv_window_design(const double* ring_t, const bpv_window_params* p, void* workspace, int64_t workspace_bytes,
-                                 void* cache, int64_t cache_bytes, void* stream) {
-  using namespace bpv;
+namespace bpv {
+static int window_design(const double* ring_t, const bpv_window_params* p, void* workspace, int64_t workspace_bytes,
+                         void* cache, int64_t cache_bytes, void* stream, const JobMap* jm) {
   if (int rc = check_filter_params(p, "bpv_window_design")) return rc;
   BPV_REQUIRE(ring_t, BPV_E_INVALID, "bpv_window_design: NULL pointer");
   BPV_REQUIRE(p->S > 0 && p->window > 0 && p->window <= p->cap && p->jobs_per_stream > 0, BPV_E_INVALID, "bpv_window_design: bad sizes");
@@ -1023,16 +1026,15 @@ extern "C" int bpv_window_design(const double* ring_t, const bpv_window_params* 
   double* taps_ws = (double*)(ws + wp.fir);
   cudaStream_t st = (cudaStream_t)stream;
   if (cache)
-    return launch_design_cached(ring_t, *p, butter, fir, (unsigned char*)cache, (int32_t*)(ws + wp.ref), ws + wp.miss, sos_ws, taps_ws, st);
-  if (butter) if (int rc = launch_job_butter(ring_t, *p, sos_ws, st)) return rc;
-  if (fir) if (int rc = launch_job_firls(ring_t, *p, taps_ws, st)) return rc;
+    return launch_design_cached(ring_t, *p, butter, fir, (unsigned char*)cache, (int32_t*)(ws + wp.ref), ws + wp.miss, sos_ws, taps_ws, st, jm);
+  if (butter) if (int rc = launch_job_butter(ring_t, *p, sos_ws, st, jm)) return rc;
+  if (fir) if (int rc = launch_job_firls(ring_t, *p, taps_ws, st, jm)) return rc;
   return 0;
 }
 
-extern "C" int bpv_window_filter(const double* ring_t, const double* ring_y, const bpv_window_params* p,
-                                 const void* workspace, int64_t workspace_bytes, const void* cache, int64_t cache_bytes,
-                                 double* proc_x, double* proc_y, int32_t* status, void* stream) {
-  using namespace bpv;
+static int window_filter(const double* ring_t, const double* ring_y, const bpv_window_params* p,
+                         const void* workspace, int64_t workspace_bytes, const void* cache, int64_t cache_bytes,
+                         double* proc_x, double* proc_y, int32_t* status, void* stream, const JobMap* jm) {
   if (int rc = check_filter_params(p, "bpv_window_preprocess")) return rc;
   BPV_REQUIRE(ring_t && ring_y && proc_x && proc_y && status, BPV_E_INVALID, "bpv_window_preprocess: NULL pointer");
   BPV_REQUIRE(p->S > 0 && p->R > 0 && p->window > 0 && p->window <= p->cap && p->jobs_per_stream > 0, BPV_E_INVALID,
@@ -1060,7 +1062,7 @@ extern "C" int bpv_window_filter(const double* ring_t, const double* ring_y, con
   const bool fir_only = !interp && !butter && fir;
   const PreLayout L = pre_layout(*p, fir_only && taps_global);
   cudaStream_t st = (cudaStream_t)stream;
-#define BPV_PRE(feat, minb, dual) return launch_preprocess<feat, minb, dual>(ring_t, ring_y, *p, L, dr, proc_x, proc_y, status, st)
+#define BPV_PRE(feat, minb, dual) return launch_preprocess<feat, minb, dual>(ring_t, ring_y, *p, L, dr, proc_x, proc_y, status, st, jm)
   // Two signals per warp pay off while enough warps stay resident to hide the stages that run for one signal after the
   // other (the spline's serial Thomas sweep above all): with the 46 KB per signal of a 1200-sample cubic + Butterworth
   // window only two such warps fit an SM and the pair is slower than two single-signal warps (measured on config 4:
@@ -1077,6 +1079,68 @@ extern "C" int bpv_window_filter(const double* ring_t, const double* ring_y, con
   if (!fir) BPV_PRE(F_INTERP | F_BUTTER, 4, true);
   BPV_PRE(F_INTERP | F_BUTTER | F_FIR, 4, true);
 #undef BPV_PRE
+}
+
+// The params of a job-map launch: the window kernels see the job list as S = num_jobs streams of one job each (their
+// per-job layouts, workspace plan and grid are then those of the lockstep path over J jobs); the map supplies each job's
+// ring row and newest sample.  Validates what the lockstep checks cannot see.
+static int jobs_params(const bpv_window_params* p, const int32_t* job_stream, const int64_t* job_head, int64_t num_jobs,
+                       const char* who, bpv_window_params& q) {
+  BPV_REQUIRE(p, BPV_E_INVALID, "%s: NULL params", who);
+  BPV_REQUIRE(job_stream && job_head, BPV_E_INVALID, "%s: NULL job map", who);
+  BPV_REQUIRE(p->S > 0 && num_jobs > 0 && num_jobs <= INT32_MAX / 32, BPV_E_INVALID, "%s: bad sizes", who);
+  q = *p;
+  q.S = (int32_t)num_jobs;
+  q.jobs_per_stream = 1;
+  q.head0 = 0;
+  q.head_step = 0;
+  return 0;
+}
+}  // namespace bpv
+
+extern "C" int bpv_window_design(const double* ring_t, const bpv_window_params* p, void* workspace, int64_t workspace_bytes,
+                                 void* cache, int64_t cache_bytes, void* stream) {
+  return bpv::window_design(ring_t, p, workspace, workspace_bytes, cache, cache_bytes, stream, nullptr);
+}
+
+extern "C" int bpv_window_filter(const double* ring_t, const double* ring_y, const bpv_window_params* p,
+                                 const void* workspace, int64_t workspace_bytes, const void* cache, int64_t cache_bytes,
+                                 double* proc_x, double* proc_y, int32_t* status, void* stream) {
+  return bpv::window_filter(ring_t, ring_y, p, workspace, workspace_bytes, cache, cache_bytes, proc_x, proc_y, status, stream,
+                            nullptr);
+}
+
+extern "C" int bpv_window_design_jobs(const double* ring_t, const bpv_window_params* p, void* workspace, int64_t workspace_bytes,
+                                      void* cache, int64_t cache_bytes, const int32_t* job_stream, const int64_t* job_head,
+                                      int64_t num_jobs, void* stream) {
+  using namespace bpv;
+  if (num_jobs == 0 && p) return 0;
+  bpv_window_params q;
+  if (int rc = jobs_params(p, job_stream, job_head, num_jobs, "bpv_window_design_jobs", q)) return rc;
+  const JobMap jm{job_stream, job_head};
+  return window_design(ring_t, &q, workspace, workspace_bytes, cache, cache_bytes, stream, &jm);
+}
+
+extern "C" int bpv_window_filter_jobs(const double* ring_t, const double* ring_y, const bpv_window_params* p,
+                                      const void* workspace, int64_t workspace_bytes, const void* cache, int64_t cache_bytes,
+                                      double* proc_x, double* proc_y, int32_t* status, const int32_t* job_stream,
+                                      const int64_t* job_head, int64_t num_jobs, void* stream) {
+  using namespace bpv;
+  if (num_jobs == 0 && p) return 0;
+  bpv_window_params q;
+  if (int rc = jobs_params(p, job_stream, job_head, num_jobs, "bpv_window_filter_jobs", q)) return rc;
+  const JobMap jm{job_stream, job_head};
+  return window_filter(ring_t, ring_y, &q, workspace, workspace_bytes, cache, cache_bytes, proc_x, proc_y, status, stream, &jm);
+}
+
+extern "C" int bpv_window_preprocess_jobs(const double* ring_t, const double* ring_y, const bpv_window_params* p,
+                                          void* workspace, int64_t workspace_bytes, double* proc_x, double* proc_y,
+                                          int32_t* status, const int32_t* job_stream, const int64_t* job_head, int64_t num_jobs,
+                                          void* stream) {
+  if (int rc = bpv_window_design_jobs(ring_t, p, workspace, workspace_bytes, nullptr, 0, job_stream, job_head, num_jobs, stream))
+    return rc;
+  return bpv_window_filter_jobs(ring_t, ring_y, p, workspace, workspace_bytes, nullptr, 0, proc_x, proc_y, status, job_stream,
+                                job_head, num_jobs, stream);
 }
 
 extern "C" int bpv_window_preprocess(const double* ring_t, const double* ring_y, const bpv_window_params* p,

@@ -154,6 +154,28 @@ int bpv_view_boxes(const int32_t* boxes, int64_t num_boxes, int32_t view_w, int3
 int bpv_ring_push(double* ring_t, double* ring_y, int32_t S, int32_t R, int32_t cap,
                   int64_t g0, int32_t T, const double* ts, const double* values, void* stream);
 
+/* Ragged steps — streams that advance at their own pace (cameras that join, leave, run at other frame rates or drop
+ * frames).  Stream s of a ragged step takes n[s] frames, 0 <= n[s] <= T, and behaves exactly like its own one-stream
+ * pipeline fed only those frames: one reference SignalProcessor per camera.
+ *
+ * bpv_ring_push_ragged: stream s appends its first n[s] rows of ts [S, T] / values [S, T, R] at global indices
+ *   g0[s] .. g0[s]+n[s]-1 (g0 int64 [S], n int32 [S], device memory); its other rows are not read.  Either of ts /
+ *   values may be NULL, as in bpv_ring_push.  g0 is not advanced (bpv_stream_jobs writes the advanced counts). */
+int bpv_ring_push_ragged(double* ring_t, double* ring_y, int32_t S, int32_t R, int32_t cap, const int64_t* g0,
+                         const int32_t* n, int32_t T, const double* ts, const double* values, void* stream);
+
+/* bpv_stream_jobs: the job map of a ragged step, built on the device (a scan over the counts, one launch; S <= 65 536).
+ *   Stream s contributes n[s] window jobs (last_only = 0: one per pushed frame, as windows='every_frame') or one job when
+ *   n[s] > 0 (last_only = 1: the window after its newest frame).  Jobs are laid out stream-major and, within a stream,
+ *   in frame order; with every n[s] = T this is the lockstep layout job = s*T + t.  Outputs: job_stream int32 [num_jobs]
+ *   (the job's stream), job_head int64 [num_jobs] (global index of the job's newest sample), stream_job0 int32 [S+1]
+ *   (the jobs of stream s are stream_job0[s] .. stream_job0[s+1]-1) and g0_next int64 [S] = g0 + n (a buffer other than g0).
+ *   num_jobs is the caller's sum of the job counts: the kernel always writes stream_job0 (so stream_job0[S] is the
+ *   device's sum) and writes the job map and g0_next only when the two agree.  stream_job0[S] != num_jobs is the error
+ *   status of a mismatch; nothing is written out of bounds.  Counts are expected in 0..T (a negative count reads as 0). */
+int bpv_stream_jobs(int32_t S, const int64_t* g0, const int32_t* n, int32_t last_only, int64_t num_jobs,
+                    int32_t* job_stream, int64_t* job_head, int32_t* stream_job0, int64_t* g0_next, void* stream);
+
 /* Running means of the per-frame results — replaces sg_bpm / sg_ptt (deque(maxlen=peak_max_samples)) and
  * their get_means() (signal_processor.py:49, 83-84, 310, 312; signal_data.py:60-63; read by drawer.py:134-135).
  * ring float64 [S, C, H] (NaN-initialised state, H = peak_max_samples <= 128), values float64 [S, T, C] (e.g.
@@ -163,6 +185,11 @@ int bpv_ring_push(double* ring_t, double* ring_y, int32_t S, int32_t R, int32_t 
  */
 int bpv_running_mean(double* ring, int32_t S, int32_t C, int32_t H, int64_t g0, int32_t T,
                      const double* values, double scale, double* mean, double* mean_int, void* stream);
+/* The running means of a ragged step: stream s pushes the values of its jobs stream_job0[s] .. stream_job0[s+1]-1 (the
+ * map of bpv_stream_jobs) in order, from its own history count g0[s] (int64 [S], device memory; not advanced: it grows
+ * by the stream's job count).  values, mean, mean_int float64 [J, C] over the step's jobs; otherwise as bpv_running_mean. */
+int bpv_running_mean_jobs(double* ring, int32_t S, int32_t C, int32_t H, const int64_t* g0, const int32_t* stream_job0,
+                          const double* values, double scale, double* mean, double* mean_int, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Window jobs.  A window job j of stream s looks at the `window` samples whose newest global
@@ -215,6 +242,24 @@ int bpv_window_design(const double* ring_t, const bpv_window_params* p, void* wo
 int bpv_window_filter(const double* ring_t, const double* ring_y, const bpv_window_params* p,
                       const void* workspace, int64_t workspace_bytes, const void* cache, int64_t cache_bytes,
                       double* proc_x, double* proc_y, int32_t* status, void* stream);
+/* F2 over a job map (ragged steps, bpv_stream_jobs): the same calls with job k reading ring row job_stream[k] and the
+ * window whose newest sample has global index job_head[k].  p->S / R / cap / window describe the rings; head0 /
+ * head_step / jobs_per_stream are ignored.  Outputs (proc_x, proc_y, status, and the per-job filter designs) are laid
+ * out over the num_jobs jobs as the lockstep calls lay them out over J = num_jobs.  The workspace must hold
+ * bpv_window_workspace_bytes() of params with S * jobs_per_stream >= num_jobs (e.g. the engine's largest lockstep step).
+ * job_stream entries must lie in [0, p->S).  num_jobs = 0 enqueues nothing; num_jobs < 0 or a NULL map is BPV_E_INVALID.
+ * The kernels are the lockstep ones compiled with a job-map switch: the results of a job equal those of the lockstep job
+ * with the same stream and head bit for bit. */
+int bpv_window_design_jobs(const double* ring_t, const bpv_window_params* p, void* workspace, int64_t workspace_bytes,
+                           void* cache, int64_t cache_bytes, const int32_t* job_stream, const int64_t* job_head,
+                           int64_t num_jobs, void* stream);
+int bpv_window_filter_jobs(const double* ring_t, const double* ring_y, const bpv_window_params* p,
+                           const void* workspace, int64_t workspace_bytes, const void* cache, int64_t cache_bytes,
+                           double* proc_x, double* proc_y, int32_t* status, const int32_t* job_stream,
+                           const int64_t* job_head, int64_t num_jobs, void* stream);
+int bpv_window_preprocess_jobs(const double* ring_t, const double* ring_y, const bpv_window_params* p,
+                               void* workspace, int64_t workspace_bytes, double* proc_x, double* proc_y, int32_t* status,
+                               const int32_t* job_stream, const int64_t* job_head, int64_t num_jobs, void* stream);
 
 /* F3 + F4(a) spectrum and HR peak — replaces transform_signal(s) + SignalGroup.get_peaks on
  *     sg_spec (signal_processor.py:248-277, 310; signal_data.py:65-70 with the range reset of
@@ -222,11 +267,13 @@ int bpv_window_filter(const double* ring_t, const double* ring_y, const bpv_wind
  * spec_f, spec_mag float32 [J, R, max_bins] (first num_bins[j,r] entries valid; may be NULL to skip
  * storing the spectrum); num_bins int32 [J, R]; peak_idx int32 [J, R] (-1 = none);
  * peak_freq, peak_mag float64 [J, R] (NaN = none).  The peak is decided in float64.
- * workspace: device memory of bpv_spectrum_workspace_bytes() bytes: scratch for the coarse spectrum of PGRAM_LS / DFT_RFFT
- * when it is not stored (spec_mag == NULL), followed — for DFT_RFFT — by the twiddle operand images of the tensor-core
- * kernel.  Zero it once and pass the SAME buffer on every call: the images are built on first use and reused while the
- * window length stays the same.  Without it (NULL / too small) DFT_RFFT generates its operands inside the kernel.
+ * workspace: device memory of bpv_spectrum_workspace_bytes() bytes: for DFT_RFFT first the twiddle operand images of the
+ * tensor-core kernel (at offset 0 whatever the job count of the call), then scratch for the coarse spectrum of PGRAM_LS /
+ * DFT_RFFT when it is not stored (spec_mag == NULL).  Zero it once and pass the SAME buffer on every call: the images are
+ * built on first use and reused while the window length stays the same, by calls of any job count.  Without it (NULL / too small) DFT_RFFT generates its operands inside the kernel.
  */
+/* F3 and F4 only ever use the J = S * jobs_per_stream processed windows, never p->S or a head on its own: the jobs of a
+ * ragged step are passed as params with S = num_jobs, jobs_per_stream = 1. */
 int64_t bpv_spectrum_workspace_bytes(const bpv_window_params* p, int32_t max_bins);
 int bpv_window_spectrum(const double* proc_x, const double* proc_y, const bpv_window_params* p,
                         int32_t max_bins, void* workspace, int64_t workspace_bytes,
