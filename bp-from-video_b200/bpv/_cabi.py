@@ -53,6 +53,7 @@ _SIGS = {
     'bpv_ring_push': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int32, _P, _P, _P]),
     'bpv_ring_push_ragged': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P, C.c_int32, _P, _P, _P]),
     'bpv_stream_jobs': (C.c_int, [C.c_int32, _P, _P, C.c_int32, C.c_int64, _P, _P, _P, _P, _P]),
+    'bpv_stream_jobs_strided': (C.c_int, [C.c_int32, _P, _P, _P, _P, C.c_int64, _P, _P, _P, _P, _P]),
     'bpv_running_mean_jobs': (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, C.c_double, _P, _P, _P]),
     'bpv_window_workspace_bytes': (C.c_int64, [C.POINTER(WindowParams)]),
     'bpv_window_preprocess': (C.c_int, [_P, _P, C.POINTER(WindowParams), _P, C.c_int64, _P, _P, _P, _P]),

@@ -45,8 +45,22 @@ n_s = T is the lockstep layout.  Sample counts, running-mean history lengths and
 n_s = T from level counts runs the lockstep kernels unchanged; any other step builds a job map on the device
 (bpv_stream_jobs) and runs the job-map instantiations of the push, design and filter kernels, F3 / F4 over the J jobs
 (every overlap schedule, the fused grid of bit 4 included, works unchanged: F3 / F4 only see J processed windows).  A step
-with J = 0 enqueues nothing.  step_detections stays lockstep.  BPV_FORCE_JOBMAP=1 (attribute `force_jobmap`) sends level
-steps through the job-map path too: a measurement switch (tools/bench_ragged.py).
+in which no stream takes a frame enqueues nothing.  step_detections stays lockstep.  BPV_FORCE_JOBMAP=1 (attribute
+`force_jobmap`) sends level steps through the job-map path too: a measurement switch (tools/bench_ragged.py).
+
+Cadence (`window_stride` k_s, `window_phase` phi_s; one int, or one per stream; default 1 / 0): a display that updates the
+heart rate and PTT at 1-2 Hz needs no window job for each of 30 frames a second.  Stream s evaluates its window after its
+m-th sample (m = 1, 2, ...) exactly when (m + phi_s) % k_s == 0, with 0 <= phi_s < k_s.  The count is the stream's own, so
+the cadence carries across steps, frame_counts, reassignment of the attributes and state_dict(); reset(streams=...) starts
+it over.  Each job equals, bit for bit, the 'every_frame' row with the same head; the running means push one value per
+evaluated job.  Staggered phases (phi_s = s % k) spread the jobs of equal cadences evenly over the steps: a lower worst step
+for a higher mean, since a step of few jobs runs its launches at their latency floor (profiles/r6b: 4096 streams, k = 30,
+mean 0.156 -> 0.387 ms, worst 0.783 -> 0.478 ms on a B200 at 1000 W).  A step of S x T frames from level counts with one k
+and one phi runs the lockstep kernels with head_step = k; any other strided step builds its job map on the device
+(bpv_stream_jobs_strided).  A step can push frames and have no job (k > T, or between cadence points): it samples and pushes
+its frames and returns a zero-row result.  k = 1 and phi = 0 everywhere is the 'every_frame' step, unchanged; a stride needs
+windows='every_frame' ('last' has its own cadence).  Bad settings raise ValueError at the step, before anything is enqueued.
+`cadence_jobs` is the host planning of both paths.
 """
 from __future__ import annotations
 
@@ -65,11 +79,21 @@ OVERLAP_DEFAULT = OVERLAP_DESIGN | OVERLAP_XCORR    # measured on c2 (profiles/r
 STATE_VERSION = 2          # 2: per-stream sample / running-mean counts (version 1 states hold one level count)
 
 
+def cadence_jobs(counts, n, stride, phase):
+    """Window jobs of a strided step (module docstring, cadence) from host int64 arrays (or ints) of the streams' sample
+    counts c, frames taken n, strides k and phases phi: (jobs per stream, J, first heads).  Stream s takes
+    q = (c + n + phi) // k - b jobs with b = (c + phi) // k; job i has its newest sample at (b + 1 + i) * k - phi - 1."""
+    b = (counts + phase) // stride
+    jobs = (counts + n + phase) // stride - b
+    return jobs, int(np.sum(jobs)), (b + 1) * stride - phase - 1
+
+
 @dataclass
 class StepResult:
     """Device tensors for the J window jobs of one step.  A lockstep step has J = S * jobs_per_stream (job =
-    s*jobs_per_stream + j); a ragged step (module docstring) has jobs_per_stream = None and the jobs of stream s in rows
-    job_offsets[s]:job_offsets[s+1], in frame order."""
+    s*jobs_per_stream + j; 0 jobs per stream for a strided step between cadence points); a ragged or per-stream strided
+    step (module docstring) has jobs_per_stream = None and the jobs of stream s in rows job_offsets[s]:job_offsets[s+1],
+    in frame order."""
     jobs_per_stream: int | None
     samples: torch.Tensor | None          # f64 [S, T, R]   raw ROI samples of this step
     peak_freq: torch.Tensor               # f64 [J, R]      Hz (NaN = none)
@@ -127,7 +151,8 @@ class BatchedSignalProcessor:
                  ls_num_freqs: int | None = None, windows: str = EVERY_FRAME, store_arrays: bool = False,
                  device: str | torch.device = 'cuda', roi_pixels_hint: int = 0, peak_max_samples: int = 0,
                  result_buffers: int = 2, overlap: int | None = None, design_cache: bool | None = None,
-                 freq_band: tuple[float, float] | None = None, lag_band: tuple[float, float] | None = None):
+                 freq_band: tuple[float, float] | None = None, lag_band: tuple[float, float] | None = None,
+                 window_stride=1, window_phase=0):
         _cabi.lib()  # fail loudly if the CUDA library is missing: there is no CPU fallback
         if not torch.cuda.is_available():
             raise _cabi.BpvError('BatchedSignalProcessor needs a CUDA device (no CPU fallback)')
@@ -216,6 +241,11 @@ class BatchedSignalProcessor:
             self._ptt_ring = torch.full((self.S, max(self.P, 1), self.peak_max_samples), float('nan'), dtype=f64, device=dev)
         self._roi_hist = None
         self._roi_count = 0
+        # window cadence (module docstring): plain attributes, checked at every step; the device copies of a strided job-map
+        # step are uploaded when they change
+        self.window_stride, self.window_phase = window_stride, window_phase
+        self._cad_dev = self._cad_host = None
+        self._cadence()
 
     # ------------------------------------------------------------------------------------------
     def _params(self, head0: int, head_step: int, jobs: int) -> _cabi.WindowParams:
@@ -258,37 +288,79 @@ class BatchedSignalProcessor:
         """a as one int when every stream holds the same value (the lockstep path's form), else as the array."""
         return int(a[0]) if (a == a[0]).all() else a
 
+    def _host_ints(self, value, name: str, scalar: bool = False) -> np.ndarray:
+        """value (host sequence / numpy array / CPU int tensor of S integers; one integer for every stream when `scalar`)
+        as int64 [S]."""
+        if torch.is_tensor(value):
+            if value.device.type != 'cpu':
+                raise ValueError(f'{name} must live on the host (a sequence, numpy array or CPU tensor): the engine '
+                                 'needs the job count without synchronising with the device')
+            value = value.numpy()
+        a = np.asarray(value)
+        if scalar and a.shape == ():
+            a = np.full(self.S, a)
+        if a.shape != (self.S,):
+            raise ValueError(f'{name} must hold {self.S} values, got shape {a.shape}')
+        if a.dtype.kind not in 'iu' and not (a.dtype.kind == 'f' and np.array_equal(a, np.floor(a))):
+            raise ValueError(f'{name} must be integers, got {a.dtype}')
+        return a.astype(np.int64)
+
     def _frame_counts(self, frame_counts, T: int):
         """frame_counts (host sequence / numpy array / CPU int tensor of S values in 0..T) as int64 [S], or None."""
         if frame_counts is None:
             return None
-        if torch.is_tensor(frame_counts):
-            if frame_counts.device.type != 'cpu':
-                raise ValueError('frame_counts must live on the host (a sequence, numpy array or CPU tensor): the engine '
-                                 'needs the job count without synchronising with the device')
-            frame_counts = frame_counts.numpy()
-        a = np.asarray(frame_counts)
-        if a.shape != (self.S,):
-            raise ValueError(f'frame_counts must hold {self.S} values, got shape {a.shape}')
-        if a.dtype.kind not in 'iu' and not (a.dtype.kind == 'f' and np.array_equal(a, np.floor(a))):
-            raise ValueError(f'frame_counts must be integers, got {a.dtype}')
-        a = a.astype(np.int64)
+        a = self._host_ints(frame_counts, 'frame_counts')
         if a.size and (a.min() < 0 or a.max() > T):
             raise ValueError(f'frame_counts must lie in [0, {T}]')
         return a
 
-    def _lockstep(self, n, T: int) -> bool:
-        """The lockstep path serves a step in which every stream takes T frames from the same counts."""
-        return ((n is None or bool((n == T).all())) and isinstance(self._cnt, int) and isinstance(self._mcnt, int)
-                and not self.force_jobmap)
+    def _cadence(self):
+        """window_stride / window_phase checked for the coming step: None for the default (a job after every frame), else
+        dict(k=, phase= host int64 [S], uniform= one k and one phase for every stream)."""
+        k, ph = self.window_stride, self.window_phase
+        if type(k) is int and type(ph) is int and k == 1 and ph == 0:
+            return None
+        k, ph = self._host_ints(k, 'window_stride', True), self._host_ints(ph, 'window_phase', True)
+        if k.min() < 1 or k.max() > np.iinfo(np.int32).max:
+            raise ValueError('window_stride must lie in [1, 2^31)')
+        if ph.min() < 0 or (ph >= k).any():
+            raise ValueError('window_phase must lie in [0, window_stride)')
+        if k.max() == 1:
+            return None
+        if self.windows == LAST:
+            raise ValueError("window_stride != 1 needs windows='every_frame' ('last' has its own cadence)")
+        return dict(k=k, phase=ph, uniform=bool((k == k[0]).all() and (ph == ph[0]).all()))
 
-    def _plan(self, n, T: int) -> dict:
-        """Host side of a job-map step: the per-stream frame counts, job counts, offsets and J."""
+    def _lockstep(self, n, T: int, cad) -> bool:
+        """The lockstep path serves a step in which every stream takes T frames from the same counts with the same cadence."""
+        return ((n is None or bool((n == T).all())) and isinstance(self._cnt, int) and isinstance(self._mcnt, int)
+                and (cad is None or cad['uniform']) and not self.force_jobmap)
+
+    def _plan(self, n, T: int, cad) -> dict | None:
+        """Host side of a step: None for a lockstep step at the default cadence; for a strided lockstep step its head0,
+        head_step, jobs per stream and J; for a job-map step the per-stream frame counts, job counts, offsets and J."""
+        if self._lockstep(n, T, cad):
+            if cad is None:
+                return None
+            k, ph = int(cad['k'][0]), int(cad['phase'][0])
+            jobs, _, head0 = cadence_jobs(self._cnt, T, k, ph)
+            return dict(lock=True, head0=head0, head_step=k, jobs=jobs, J=self.S * jobs)
         n = np.full(self.S, T, dtype=np.int64) if n is None else n
-        jobs = n if self.windows == EVERY_FRAME else (n > 0).astype(np.int64)
+        if cad is not None:
+            jobs = cadence_jobs(self.counts, n, cad['k'], cad['phase'])[0]
+        else:
+            jobs = n if self.windows == EVERY_FRAME else (n > 0).astype(np.int64)
         off = np.zeros(self.S + 1, dtype=np.int64)
         np.cumsum(jobs, out=off[1:])
-        return dict(n=n, jobs=jobs, off=off, J=int(off[-1]), T=T, mapped=False)
+        return dict(lock=False, n=n, jobs=jobs, off=off, J=int(off[-1]), T=T, mapped=False, cad=cad)
+
+    def _lock_jobs(self, T: int, plan):
+        """(head0, head_step, jobs per stream) of a lockstep step from the current count."""
+        if plan is not None:
+            return plan['head0'], plan['head_step'], plan['jobs']
+        if self.windows == EVERY_FRAME:
+            return self._cnt, 1, T
+        return self._cnt + T - 1, 1, 1
 
     def _map_jobs(self, plan: dict, turn: int) -> None:
         """Upload the step's frame counts (and the sample counts when the device copy is stale) and build the job map of
@@ -306,14 +378,32 @@ class BatchedSignalProcessor:
             self._g0[0].copy_(pin['g0'], non_blocking=True)
             self._g0_ok = True
         js, jh, sj0 = self._jobmap[turn]
-        ops.stream_jobs(self._g0[0], self._ndev, self.windows == LAST, plan['J'], js, jh, sj0, self._g0[1])
+        if plan['cad'] is None:
+            ops.stream_jobs(self._g0[0], self._ndev, self.windows == LAST, plan['J'], js, jh, sj0, self._g0[1])
+        else:
+            kd, pd = self._cadence_dev(plan['cad'], pin)
+            ops.stream_jobs_strided(self._g0[0], self._ndev, kd, pd, plan['J'], js, jh, sj0, self._g0[1])
         plan['mapped'] = True
+
+    def _cadence_dev(self, cad: dict, pin: dict):
+        """Device int32 [S] copies of the strides and phases, uploaded through the pinned staging `pin` when they changed."""
+        if self._cad_dev is None:
+            self._cad_dev = tuple(torch.empty(self.S, dtype=torch.int32, device=self.device) for _ in range(2))
+        host = self._cad_host
+        if host is None or not (np.array_equal(host[0], cad['k']) and np.array_equal(host[1], cad['phase'])):
+            pin['k'].numpy()[:] = cad['k']
+            pin['ph'].numpy()[:] = cad['phase']
+            self._cad_dev[0].copy_(pin['k'], non_blocking=True)
+            self._cad_dev[1].copy_(pin['ph'], non_blocking=True)
+            self._cad_host = (cad['k'].copy(), cad['phase'].copy())
+        return self._cad_dev
 
     def _pinned(self, turn: int) -> dict:
         """Pinned staging buffers of result turn `turn`, once the device has consumed their previous contents."""
         if self._staging[turn] is None:
             mk = lambda dt: torch.empty(self.S, dtype=dt).pin_memory()
-            self._staging[turn] = dict(n=mk(torch.int32), g0=mk(torch.int64), m0=mk(torch.int64), ev=torch.cuda.Event(), used=False)
+            self._staging[turn] = dict(n=mk(torch.int32), g0=mk(torch.int64), m0=mk(torch.int64), k=mk(torch.int32),
+                                       ph=mk(torch.int32), ev=torch.cuda.Event(), used=False)
         pin = self._staging[turn]
         if pin['used']:
             pin['ev'].synchronize()
@@ -342,6 +432,7 @@ class BatchedSignalProcessor:
         are BPV_NO_BOX (x0 = NO_BOX).  A step in which no stream takes a frame enqueues nothing (samples = None)."""
         S, T = frames.shape[:2]
         self._check_step(S, T, boxes)
+        cad = self._cadence()
         n = self._frame_counts(frame_counts, T)
         if n is not None and not n.any():
             return self._empty_step(None)
@@ -370,17 +461,19 @@ class BatchedSignalProcessor:
             samples = self._samples[self._turn][:, :T]
             if T != self.Tmax:
                 samples = torch.empty((S, T, self.R), dtype=torch.float64, device=self.device)
-            design_ahead = bool(self.overlap & OVERLAP_DESIGN) and any(m in (_cabi.FILTER_BUTTER, _cabi.FILTER_FIR) for m in self.methods)
-            plan = None if self._lockstep(n, T) else self._plan(n, T)
-            if design_ahead and plan is None:
-                self._design_ahead(timestamps, T)
+            plan = self._plan(n, T, cad)
+            design_ahead = (bool(self.overlap & OVERLAP_DESIGN)
+                            and any(m in (_cabi.FILTER_BUTTER, _cabi.FILTER_FIR) for m in self.methods)
+                            and (plan is None or plan['J'] > 0))      # a step without jobs has nothing to design
+            if design_ahead and (plan is None or plan['lock']):
+                self._design_ahead(timestamps, T, plan)
             elif design_ahead:
                 self._design_ahead_jobs(timestamps, plan)
             ops.roi_sample(frames.view(S * T, *frames.shape[2:]), boxes.view(S * T, self.R, 4), self.color_channel,
                            roi_pixels_hint=self.roi_pixels_hint, out_value=samples.view(S * T, self.R))
             return self.step_signals(samples, timestamps, _count_roi=True, _designed=design_ahead, frame_counts=n, _plan=plan)
 
-    def _design_ahead(self, timestamps: torch.Tensor, T: int) -> None:
+    def _design_ahead(self, timestamps: torch.Tensor, T: int, plan) -> None:
         """Push the step's timestamps and start the filter design of its window jobs on the side stream: make_filter
         depends on nothing else (signal_processor.py:158-173), so it runs beside F1 instead of between F1 and F2."""
         _, ev = self._streams()
@@ -388,9 +481,8 @@ class BatchedSignalProcessor:
         main = torch.cuda.current_stream(self.device)
         ops.ring_push(self.ring_t, self.ring_y, self._cnt, timestamps.contiguous(), None)
         ev['ts'].record(main)
-        jobs = T if self.windows == EVERY_FRAME else 1
-        head0 = self._cnt if self.windows == EVERY_FRAME else self._cnt + T - 1
-        p = self._params(head0, 1, jobs)
+        head0, head_step, jobs = self._lock_jobs(T, plan)
+        p = self._params(head0, head_step, jobs)
         side.wait_event(ev['ts'])
         with torch.cuda.stream(side):
             ops.window_design(self.ring_t, p, self._ws, self._cache())
@@ -468,16 +560,18 @@ class BatchedSignalProcessor:
         self._check_step(S, T)
         if R != self.R or tuple(timestamps.shape) != (S, T):
             raise ValueError(f'step_signals: samples must be [S, T, {self.R}] and timestamps [S, T]')
+        cad = self._cadence()
         n = self._frame_counts(frame_counts, T)
         if n is not None and not n.any():
             return self._empty_step(samples)
-        if _plan is None and not self._lockstep(n, T):
-            _plan = self._plan(n, T)
+        if _plan is None:
+            _plan = self._plan(n, T, cad)
         with torch.cuda.device(self.device):
             return self._step_signals(samples, timestamps, S, T, _count_roi, _designed, _plan)
 
-    def _empty_step(self, samples) -> StepResult:
-        """The result of a step in which no stream takes a frame: zero jobs, nothing enqueued, no state changed."""
+    def _empty_step(self, samples, jobs_per_stream=None, launches: int = 0) -> StepResult:
+        """A result of zero jobs.  A step in which no stream takes a frame enqueues nothing and changes no state; a strided
+        step without jobs has pushed its frames (`launches`)."""
         dev, f64, f32, i32 = self.device, torch.float64, torch.float32, torch.int32
         R, P, W = self.R, self.P, self.W
         e = lambda *shape, dt=f64: torch.empty(shape, dtype=dt, device=dev)
@@ -490,9 +584,10 @@ class BatchedSignalProcessor:
             means = dict(mean_bpm=e(0, R), mean_bpm_int=e(0, R))
             if P:
                 means.update(mean_ptt=e(0, P), mean_ptt_int=e(0, P))
-        self.launches_per_step = 0
-        return StepResult(None, samples, e(0, R), e(0, R, dt=i32), e(0, R), e(0, P), e(0, P, dt=i32), e(0, P), e(0, R, dt=i32),
-                          arrays, means, _job_offsets=np.zeros(self.S + 1, dtype=np.int64), _job_stream=e(0, dt=i32))
+        self.launches_per_step = launches
+        return StepResult(jobs_per_stream, samples, e(0, R), e(0, R, dt=i32), e(0, R), e(0, P), e(0, P, dt=i32), e(0, P),
+                          e(0, R, dt=i32), arrays, means, _job_offsets=np.zeros(self.S + 1, dtype=np.int64),
+                          _job_stream=e(0, dt=i32))
 
     def _outputs(self, turn: int, J: int):
         """F3 / F4 output dicts of a step: views of the first J rows of result turn `turn`'s Jmax-row buffers."""
@@ -507,14 +602,16 @@ class BatchedSignalProcessor:
         turn = self._turn
         self._turn = (turn + 1) % self._nbuf
         has_filter = any(m in (_cabi.FILTER_BUTTER, _cabi.FILTER_FIR) for m in self.methods)
-        if plan is None:
+        lock = plan is None or plan['lock']
+        roi_launches = 1 + self._extra_launches if _count_roi else 0
+        if lock:
+            head0, head_step, jobs = self._lock_jobs(T, plan)
             ops.ring_push(self.ring_t, self.ring_y, self._cnt, None if _designed else timestamps.contiguous(), samples.contiguous())
-            g0 = self._cnt
             self._cnt += T
             self._g0_ok = False
-            jobs = T if self.windows == EVERY_FRAME else 1
-            head0 = g0 if self.windows == EVERY_FRAME else g0 + T - 1
-            p = self._params(head0, 1, jobs)
+            if jobs == 0:                       # a strided step between cadence points: F1 + push
+                return self._empty_step(samples, 0, roi_launches + 1)
+            p = self._params(head0, head_step, jobs)
             pj, J = p, S * jobs
         else:
             # job-map path: stream s pushes n_s frames and owns jobs job_offsets[s]:job_offsets[s+1]; F3 / F4 see the J jobs
@@ -524,6 +621,9 @@ class BatchedSignalProcessor:
             ops.ring_push_ragged(self.ring_t, self.ring_y, self._g0[0], self._ndev, None if _designed else timestamps.contiguous(),
                                  samples.contiguous())
             jobs, J = None, plan['J']
+            if J == 0:                          # a strided step between cadence points: F1 + map + push
+                self._advance(plan, turn, main)
+                return self._empty_step(samples, None, roi_launches + 2)
             p = self._params(0, 1, 1)
             pj = ops.jobs_params(p, J)
             js, jh, sj0 = self._jobmap[turn]
@@ -531,11 +631,11 @@ class BatchedSignalProcessor:
         px, py, st = proc[0, :J], proc[1, :J], self._status[turn][:J]
         if _designed:
             main.wait_event(self._ev['design'])
-        elif has_filter and plan is None:
+        elif has_filter and lock:
             ops.window_design(self.ring_t, p, self._ws, self._cache())
         elif has_filter:
             ops.window_design_jobs(self.ring_t, p, self._ws, js, jh, J, self._cache())
-        if plan is None:
+        if lock:
             ops.window_filter(self.ring_t, self.ring_y, p, self._ws, px, py, st, cache=self._dcache if has_filter else None)
         else:
             ops.window_filter_jobs(self.ring_t, self.ring_y, p, self._ws, js, jh, J, px, py, st,
@@ -583,8 +683,8 @@ class BatchedSignalProcessor:
             interp = any(m in (_cabi.INTERP_LINEAR, _cabi.INTERP_CUBIC) for m in self.methods)
             if (env[:1] == '1') if env is not None else interp:
                 n_spec = 6              # dft_image + seal + dft_split + dft_tc_tma2 + dft_peak kernels + spectrum_dense_kernel for the flagged windows
-        n_push = (2 if _designed else 1) + (0 if plan is None else 1)          # (+ the job map)
-        self.launches_per_step = (1 + self._extra_launches if _count_roi else 0) + n_push + n_pre + n_spec + (1 if self.P and not (fused and self.W <= 320) else 0)
+        n_push = (2 if _designed else 1) + (0 if lock else 1)          # (+ the job map)
+        self.launches_per_step = roi_launches + n_push + n_pre + n_spec + (1 if self.P and not (fused and self.W <= 320) else 0)
         if not self.store_arrays and self.discard_scratch:
             self.launches_per_step += 1 if J == self._Jmax else 2
         arrays = {}
@@ -592,7 +692,7 @@ class BatchedSignalProcessor:
             arrays = dict(proc_x=px, proc_y=py, freqs=sp['freqs'], mags=sp['mags'], num_bins=sp['num_bins'],
                           lags=xc['lags'], corr=xc['corr'], num_lags=xc['num_lags'])
         means = {}
-        if self.peak_max_samples and plan is None:
+        if self.peak_max_samples and lock:
             mb, mbi = ops.running_mean(self._bpm_ring, self._mcnt, sp['peak_freq'].view(S, jobs, self.R), 60.0)
             means = dict(mean_bpm=mb.view(J, self.R), mean_bpm_int=mbi.view(J, self.R))
             if self.P:
@@ -612,15 +712,20 @@ class BatchedSignalProcessor:
                 means.update(mean_ptt=mp, mean_ptt_int=mpi)
             self._mcnt = self._level(mcnt + plan['jobs'])
             self.launches_per_step += 2 if self.P else 1
-        if plan is None:
+        if lock:
             return StepResult(jobs, samples, sp['peak_freq'], sp['peak_idx'], sp['peak_mag'], xc['lag_sec'], xc['lag_idx'],
                               xc['lag_corr'], st, arrays, means)
+        self._advance(plan, turn, main)
+        return StepResult(None, samples, sp['peak_freq'], sp['peak_idx'], sp['peak_mag'], xc['lag_sec'], xc['lag_idx'],
+                          xc['lag_corr'], st, arrays, means, _job_offsets=plan['off'], _job_stream=js[:J])
+
+    def _advance(self, plan: dict, turn: int, main) -> None:
+        """End of a job-map step on the host: the staging of `turn` is in flight until the device passes this point, and
+        the counts advance by the frames taken."""
         self._staging[turn]['ev'].record(main)
         self._staging[turn]['used'] = True
         self._cnt = self._level(self.counts + plan['n'])
         self._g0.reverse()                      # bpv_stream_jobs left the advanced counts in the other buffer
-        return StepResult(None, samples, sp['peak_freq'], sp['peak_idx'], sp['peak_mag'], xc['lag_sec'], xc['lag_idx'],
-                          xc['lag_corr'], st, arrays, means, _job_offsets=plan['off'], _job_stream=js[:J])
 
     # ------------------------------------------------------------------------------------------
     # SURVEY.md §8(f) row 3: snapshot / resume of the per-stream state (the reference's deepcopy(store), :313, is the

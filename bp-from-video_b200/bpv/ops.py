@@ -137,6 +137,20 @@ def stream_jobs(g0: torch.Tensor, n: torch.Tensor, last_only: bool, num_jobs: in
          ptr(stream_job0), ptr(g0_next))
 
 
+def stream_jobs_strided(g0: torch.Tensor, n: torch.Tensor, stride: torch.Tensor | None, phase: torch.Tensor | None, num_jobs: int,
+                        job_stream: torch.Tensor, job_head: torch.Tensor, stream_job0: torch.Tensor, g0_next: torch.Tensor) -> None:
+    """Job map of a step with a window cadence (include/bpv.h bpv_stream_jobs_strided): stream s evaluates its window after
+    each sample m with (m + phase[s]) % stride[s] == 0.  stride / phase int32 [S] on the device (None = 1 / 0); the other
+    arguments as in stream_jobs."""
+    S = g0.numel()
+    _require(n.numel() == S and stream_job0.numel() == S + 1 and g0_next.numel() == S, 'stream_jobs_strided: sizes do not match')
+    _require(all(t is None or (t.dtype == torch.int32 and t.numel() == S) for t in (stride, phase)),
+             'stream_jobs_strided: stride / phase must be int32 [S]')
+    _require(job_stream.numel() >= num_jobs and job_head.numel() >= num_jobs, 'stream_jobs_strided: job map buffers too small')
+    _run(g0.device, 'bpv_stream_jobs_strided', S, ptr(g0), ptr(n), ptr(stride), ptr(phase), int(num_jobs), ptr(job_stream),
+         ptr(job_head), ptr(stream_job0), ptr(g0_next))
+
+
 def running_mean_jobs(ring, g0: torch.Tensor, stream_job0: torch.Tensor, values, scale: float):
     """running_mean over the job map of a ragged step (include/bpv.h bpv_running_mean_jobs): values [J,C]; returns (mean,
     mean_int) f64 [J,C].  g0 int64 [S] = the streams' history counts (not advanced)."""

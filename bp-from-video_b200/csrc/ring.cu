@@ -53,6 +53,9 @@ __global__ void ring_push_ragged_kernel(double* __restrict__ ring_t, double* __r
 // so one launch needs no inter-CTA scratch; a warp-shuffle block scan places the chunk's streams.  The map entries are then
 // written job-parallel (thread per job, coalesced stores; the job's stream by a binary search over the chunk's offsets in
 // shared memory): a stream's up to T entries written by one thread would make every store of a warp touch 32 lines.
+// STRIDED (bpv_stream_jobs_strided): stream s evaluates its window after its m-th sample exactly when (m + phase) % stride
+// == 0, so of a step's n frames from count c it takes q = (c + n + phase) / stride - (c + phase) / stride jobs, job i with its
+// newest sample at ((c + phase) / stride + 1 + i) * stride - phase - 1.  The !STRIDED instantiation is bpv_stream_jobs's.
 constexpr int STREAM_JOBS_THREADS = 1024;
 __device__ __forceinline__ long long block_sum_ll(long long v, long long* red) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -64,12 +67,29 @@ __device__ __forceinline__ long long block_sum_ll(long long v, long long* red) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
 }
+// A stream's cadence: a stride below 1 reads as 1, a phase as its remainder modulo the stride (in [0, stride)); NULL arrays
+// read as stride 1 / phase 0.  Whatever the entries hold, a stream then takes between 0 and n of its step's jobs.
+__device__ __forceinline__ void stream_cadence(const int32_t* __restrict__ stride, const int32_t* __restrict__ phase, int s,
+                                               long long& k, long long& ph) {
+  k = stride ? max(stride[s], 1) : 1;
+  ph = phase ? ((long long)phase[s] % k + k) % k : 0;
+}
+__device__ __forceinline__ int strided_jobs(const int64_t* __restrict__ g0, const int32_t* __restrict__ stride,
+                                            const int32_t* __restrict__ phase, int s, int n) {
+  long long k, ph;
+  stream_cadence(stride, phase, s, k, ph);
+  const long long c = g0[s] + ph;                            // 64-bit: counts grow without bound on long-running streams
+  return (int)((c + n) / k - c / k);
+}
+template <bool STRIDED>
 __global__ void __launch_bounds__(STREAM_JOBS_THREADS) stream_jobs_kernel(int S, const int64_t* __restrict__ g0,
                                                                           const int32_t* __restrict__ n, int last_only,
                                                                           long long num_jobs, int32_t* __restrict__ job_stream,
                                                                           int64_t* __restrict__ job_head,
                                                                           int32_t* __restrict__ stream_job0,
-                                                                          int64_t* __restrict__ g0_next) {
+                                                                          int64_t* __restrict__ g0_next,
+                                                                          const int32_t* __restrict__ stride,
+                                                                          const int32_t* __restrict__ phase) {
   __shared__ long long red[32];
   __shared__ int first[STREAM_JOBS_THREADS];                  // first job of each of the chunk's streams, chunk-relative
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
@@ -77,7 +97,7 @@ __global__ void __launch_bounds__(STREAM_JOBS_THREADS) stream_jobs_kernel(int S,
   long long all = 0, before = 0;
   for (int s = tid; s < S; s += STREAM_JOBS_THREADS) {
     const int k = max(n[s], 0);
-    const int jk = last_only ? (k > 0) : k;
+    const int jk = STRIDED ? strided_jobs(g0, stride, phase, s, k) : last_only ? (k > 0) : k;
     all += jk;
     if (s < s0) before += jk;
   }
@@ -85,7 +105,7 @@ __global__ void __launch_bounds__(STREAM_JOBS_THREADS) stream_jobs_kernel(int S,
   before = block_sum_ll(before, red);
   const int s = s0 + tid;
   const int k = s < S ? max(n[s], 0) : 0;
-  const int jk = last_only ? (k > 0) : k;
+  const int jk = STRIDED ? (s < S ? strided_jobs(g0, stride, phase, s, k) : 0) : last_only ? (k > 0) : k;
   long long inc = jk;                                          // inclusive scan of the chunk's job counts
   for (int o = 1; o < 32; o <<= 1) {
     const long long v = __shfl_up_sync(0xffffffffu, inc, o);
@@ -124,7 +144,13 @@ __global__ void __launch_bounds__(STREAM_JOBS_THREADS) stream_jobs_kernel(int S,
     const int ss = s0 + lo;
     const long long base = g0[ss];
     job_stream[before + q] = ss;
-    job_head[before + q] = last_only ? base + max(n[ss], 0) - 1 : base + (q - first[lo]);
+    if (STRIDED) {
+      long long k, ph;
+      stream_cadence(stride, phase, ss, k, ph);
+      job_head[before + q] = ((base + ph) / k + 1 + (q - first[lo])) * k - ph - 1;
+    } else {
+      job_head[before + q] = last_only ? base + max(n[ss], 0) - 1 : base + (q - first[lo]);
+    }
   }
 }
 }  // namespace bpv
@@ -140,17 +166,36 @@ extern "C" int bpv_ring_push_ragged(double* ring_t, double* ring_y, int32_t S, i
   return check_launch("bpv_ring_push_ragged");
 }
 
+namespace bpv {
+static int stream_jobs(const char* who, int32_t S, const int64_t* g0, const int32_t* n, int32_t last_only, const int32_t* stride,
+                       const int32_t* phase, int64_t num_jobs, int32_t* job_stream, int64_t* job_head, int32_t* stream_job0,
+                       int64_t* g0_next, void* stream) {
+  BPV_REQUIRE(g0 && n && stream_job0 && g0_next && (num_jobs == 0 || (job_stream && job_head)), BPV_E_INVALID,
+              "%s: NULL pointer", who);
+  BPV_REQUIRE(S > 0 && S <= 65536 && num_jobs >= 0 && num_jobs <= INT32_MAX, BPV_E_INVALID,
+              "%s: bad sizes (1 <= S <= 65536, 0 <= num_jobs < 2^31)", who);
+  const unsigned grid = (unsigned)((S + STREAM_JOBS_THREADS - 1) / STREAM_JOBS_THREADS);
+  if (stride || phase)
+    stream_jobs_kernel<true><<<grid, STREAM_JOBS_THREADS, 0, (cudaStream_t)stream>>>(S, g0, n, 0, num_jobs, job_stream, job_head,
+                                                                                     stream_job0, g0_next, stride, phase);
+  else
+    stream_jobs_kernel<false><<<grid, STREAM_JOBS_THREADS, 0, (cudaStream_t)stream>>>(S, g0, n, last_only != 0, num_jobs, job_stream,
+                                                                                      job_head, stream_job0, g0_next, nullptr, nullptr);
+  return check_launch(who);
+}
+}  // namespace bpv
+
 extern "C" int bpv_stream_jobs(int32_t S, const int64_t* g0, const int32_t* n, int32_t last_only, int64_t num_jobs,
                                int32_t* job_stream, int64_t* job_head, int32_t* stream_job0, int64_t* g0_next, void* stream) {
-  using namespace bpv;
-  BPV_REQUIRE(g0 && n && stream_job0 && g0_next && (num_jobs == 0 || (job_stream && job_head)), BPV_E_INVALID,
-              "bpv_stream_jobs: NULL pointer");
-  BPV_REQUIRE(S > 0 && S <= 65536 && num_jobs >= 0 && num_jobs <= INT32_MAX, BPV_E_INVALID,
-              "bpv_stream_jobs: bad sizes (1 <= S <= 65536, 0 <= num_jobs < 2^31)");
-  const unsigned grid = (unsigned)((S + STREAM_JOBS_THREADS - 1) / STREAM_JOBS_THREADS);
-  stream_jobs_kernel<<<grid, STREAM_JOBS_THREADS, 0, (cudaStream_t)stream>>>(S, g0, n, last_only != 0, num_jobs, job_stream, job_head,
-                                                                             stream_job0, g0_next);
-  return check_launch("bpv_stream_jobs");
+  return bpv::stream_jobs("bpv_stream_jobs", S, g0, n, last_only, nullptr, nullptr, num_jobs, job_stream, job_head, stream_job0,
+                          g0_next, stream);
+}
+
+extern "C" int bpv_stream_jobs_strided(int32_t S, const int64_t* g0, const int32_t* n, const int32_t* stride, const int32_t* phase,
+                                       int64_t num_jobs, int32_t* job_stream, int64_t* job_head, int32_t* stream_job0,
+                                       int64_t* g0_next, void* stream) {
+  return bpv::stream_jobs("bpv_stream_jobs_strided", S, g0, n, 0, stride, phase, num_jobs, job_stream, job_head, stream_job0,
+                          g0_next, stream);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -175,6 +175,19 @@ int bpv_ring_push_ragged(double* ring_t, double* ring_y, int32_t S, int32_t R, i
  *   status of a mismatch; nothing is written out of bounds.  Counts are expected in 0..T (a negative count reads as 0). */
 int bpv_stream_jobs(int32_t S, const int64_t* g0, const int32_t* n, int32_t last_only, int64_t num_jobs,
                     int32_t* job_stream, int64_t* job_head, int32_t* stream_job0, int64_t* g0_next, void* stream);
+/* bpv_stream_jobs_strided: the job map of a step with a window cadence (windows evaluated every stride[s]-th sample of
+ *   stream s).  Stream s evaluates its window after its m-th sample (m = 1, 2, ...; global index m - 1) exactly when
+ *   (m + phase[s]) % stride[s] == 0; the phase is tied to the stream's own count, so it carries across steps.  Of a step in
+ *   which it holds c = g0[s] samples and takes n[s] frames it contributes q = floor((c + n + phase) / stride) -
+ *   floor((c + phase) / stride) jobs, job i (0 <= i < q) with its newest sample at (floor((c + phase) / stride) + 1 + i) *
+ *   stride - phase - 1.  stride = phase = 1 / 0 everywhere is bpv_stream_jobs with last_only = 0.  stride, phase: int32 [S]
+ *   in device memory; NULL reads as 1 / 0 for every stream.  A stride below 1 reads as 1 and a phase as its remainder
+ *   modulo the stride, in [0, stride), so whatever the entries hold a stream takes between 0 and n[s] jobs.  The
+ *   arithmetic is 64-bit.  Outputs, num_jobs, the mismatch status and the bounds are those of bpv_stream_jobs; one launch
+ *   for up to 65 536 streams. */
+int bpv_stream_jobs_strided(int32_t S, const int64_t* g0, const int32_t* n, const int32_t* stride, const int32_t* phase,
+                            int64_t num_jobs, int32_t* job_stream, int64_t* job_head, int32_t* stream_job0, int64_t* g0_next,
+                            void* stream);
 
 /* Running means of the per-frame results — replaces sg_bpm / sg_ptt (deque(maxlen=peak_max_samples)) and
  * their get_means() (signal_processor.py:49, 83-84, 310, 312; signal_data.py:60-63; read by drawer.py:134-135).
