@@ -72,6 +72,8 @@ _SIGS = {
                                            C.c_double, C.c_double, _P]),
     'bpv_window_xcorr_band': (C.c_int, [_P, _P, C.POINTER(WindowParams), _P, _P, _P, _P, _P, _P, C.c_double, C.c_double, _P]),
     'bpv_window_welch_xcorr': (C.c_int, [_P, _P, C.POINTER(WindowParams), C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    'bpv_window_snr': (C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_double, C.c_double,
+                                 _P, _P, C.c_int32, C.c_double, _P, _P, _P, _P]),
     'bpv_butter_sos_design': (C.c_int, [_P, C.c_int32, C.POINTER(WindowParams), _P, _P]),
     'bpv_firls_design': (C.c_int, [_P, C.c_int32, C.POINTER(WindowParams), _P, _P]),
 }

@@ -61,6 +61,26 @@ and one phi runs the lockstep kernels with head_step = k; any other strided step
 its frames and returns a zero-row result.  k = 1 and phi = 0 everywhere is the 'every_frame' step, unchanged; a stride needs
 windows='every_frame' ('last' has its own cadence).  Bad settings raise ValueError at the step, before anything is enqueued.
 `cadence_jobs` is the host planning of both paths.
+
+Signal quality (`snr`, `snr_half_width`, `min_snr_db`; default off).  Every window job returns a heart rate, whether its ROI
+held a pulsing forehead, a face that turned away or a dark frame, and peak_mag is no quality measure (its unit depends on
+the transform, and for DFT / Welch it scales with the signal).  snr=True adds StepResult.snr_db f64 [J, R], the spectral SNR of
+de Haan & Jeanne (IEEE TBME 2013), dimensionless and scale-free, computed by one kernel (include/bpv.h bpv_window_snr) from the
+spectrum F3 stores: on the stored float32 values widened to float64, the bin power P_k is m_k^2 for DFT_RFFT (amplitude
+spectrum) and m_k for PGRAM_WELCH / PGRAM_LS; B = the bins k < num_bins with a finite m_k and lo <= f_k <= hi; a bin is in the
+template when |f_k - f0| <= snr_half_width or |f_k - 2 f0| <= snr_half_width (f0 = f_{peak_idx}, in Hz; default 0.125 Hz =
+7.5 bpm: the peak bin and its two neighbours on the 0.1 Hz DFT grid of 10 s at 30 fps, where 0.1 Hz would put a neighbour in
+or out on float32 rounding, and on the 0.117 Hz Welch grid); snr_db = 10 log10(S_sig / S_noise) with IEEE semantics (0/x ->
+-inf, x/0 -> +inf, 0/0 -> NaN), NaN when there is no peak or |B| < 2.  The band is freq_band when set, else (min_freq,
+max_freq); an unbanded DC peak (0 bpm) therefore gets -inf.  B is decided on the stored float32 frequencies, so it can differ
+from the band-limited peak search (float64) in a bin within float32 rounding of lo or hi.  min_snr_db (dB, -inf allowed; a plain
+attribute, reassignable between steps; needs snr=True) gates what the running means push: a heart rate is accepted when snr_db
+>= min_snr_db (NaN is rejected), a pair's PTT when both of its ROIs are, and a rejected value enters the history as NaN (which
+np.nanmean skips).  peak_freq, lag_sec, the indices and the packed records stay ungated; the gate adds no state.  The kernel runs
+on the main stream after F3 (and after the xcorr event) on every path: one more launch per step.  Memory: F3 then stores its
+spectrum into the result buffers even with store_arrays=False (res.arrays stays empty): 2 x 4 B x Jmax x R x max_bins per
+result buffer, 34 MB for c2 (16 384 jobs, R = 2, 129 Welch bins), 134 MB for 4096 jobs of a 2048-bin Lomb-Scargle grid.
+snr=False takes exactly the path and launches of an engine without the feature.
 """
 from __future__ import annotations
 
@@ -107,6 +127,7 @@ class StepResult:
     means: dict = field(default_factory=dict)    # mean_bpm, mean_bpm_int [J, R], mean_ptt, mean_ptt_int [J, P] when tracked
     _job_offsets: np.ndarray | None = field(default=None, repr=False)   # host int64 [S+1] of a ragged step
     _job_stream: torch.Tensor | None = field(default=None, repr=False)  # device int32 [J] of a ragged step
+    snr_db: torch.Tensor | None = None    # f64 [J, R]      spectral SNR of the heart-rate peak (engine snr=True)
 
     @property
     def job_offsets(self) -> np.ndarray:
@@ -152,7 +173,8 @@ class BatchedSignalProcessor:
                  device: str | torch.device = 'cuda', roi_pixels_hint: int = 0, peak_max_samples: int = 0,
                  result_buffers: int = 2, overlap: int | None = None, design_cache: bool | None = None,
                  freq_band: tuple[float, float] | None = None, lag_band: tuple[float, float] | None = None,
-                 window_stride=1, window_phase=0):
+                 window_stride=1, window_phase=0, snr: bool = False, snr_half_width: float = ops.SNR_HALF_WIDTH,
+                 min_snr_db: float | None = None):
         _cabi.lib()  # fail loudly if the CUDA library is missing: there is no CPU fallback
         if not torch.cuda.is_available():
             raise _cabi.BpvError('BatchedSignalProcessor needs a CUDA device (no CPU fallback)')
@@ -175,6 +197,11 @@ class BatchedSignalProcessor:
         # peak search ranges (module docstring): None = every bin / lag, as process()
         self.freq_band = ops.peak_band(freq_band, 'freq_band')
         self.lag_band = ops.peak_band(lag_band, 'lag_band')
+        # signal quality (module docstring): fixed at construction, since F3 then stores its spectrum into the result buffers
+        self.snr = bool(snr)
+        self.snr_half_width = ops.snr_half_width(snr_half_width)
+        self._min_snr_db = None
+        self.min_snr_db = min_snr_db
         self.roi_pixels_hint = int(roi_pixels_hint)
         self.device = torch.device(device)
         if self.device.type != 'cuda':
@@ -264,6 +291,19 @@ class BatchedSignalProcessor:
                 self._side_hi = torch.cuda.Stream(device=self.device, priority=prio)
                 self._ev = {k: torch.cuda.Event() for k in ('ts', 'design', 'pre', 'xc')}
         return self._side, self._ev
+
+    @property
+    def min_snr_db(self) -> float | None:
+        """SNR gate of the running means in dB (module docstring, signal quality); None = no gate.  Reassignable between
+        steps; needs snr=True."""
+        return self._min_snr_db
+
+    @min_snr_db.setter
+    def min_snr_db(self, value) -> None:
+        value = ops.snr_threshold(value)
+        if value is not None and not self.snr:
+            raise ValueError('min_snr_db needs an engine built with snr=True')
+        self._min_snr_db = value
 
     # per-stream counts (module docstring: ragged steps)
     @property
@@ -433,6 +473,8 @@ class BatchedSignalProcessor:
         S, T = frames.shape[:2]
         self._check_step(S, T, boxes)
         cad = self._cadence()
+        if self.snr:
+            self.snr_half_width = ops.snr_half_width(self.snr_half_width)
         n = self._frame_counts(frame_counts, T)
         if n is not None and not n.any():
             return self._empty_step(None)
@@ -561,6 +603,8 @@ class BatchedSignalProcessor:
         if R != self.R or tuple(timestamps.shape) != (S, T):
             raise ValueError(f'step_signals: samples must be [S, T, {self.R}] and timestamps [S, T]')
         cad = self._cadence()
+        if self.snr:
+            self.snr_half_width = ops.snr_half_width(self.snr_half_width)
         n = self._frame_counts(frame_counts, T)
         if n is not None and not n.any():
             return self._empty_step(samples)
@@ -587,14 +631,21 @@ class BatchedSignalProcessor:
         self.launches_per_step = launches
         return StepResult(jobs_per_stream, samples, e(0, R), e(0, R, dt=i32), e(0, R), e(0, P), e(0, P, dt=i32), e(0, P),
                           e(0, R, dt=i32), arrays, means, _job_offsets=np.zeros(self.S + 1, dtype=np.int64),
-                          _job_stream=e(0, dt=i32))
+                          _job_stream=e(0, dt=i32), snr_db=e(0, R) if self.snr else None)
 
     def _outputs(self, turn: int, J: int):
-        """F3 / F4 output dicts of a step: views of the first J rows of result turn `turn`'s Jmax-row buffers."""
+        """F3 / F4 (and SNR, with snr=True) output dicts of a step: views of the first J rows of result turn `turn`'s
+        Jmax-row buffers.  With snr=True F3 stores its spectrum even when the arrays are not stored."""
         if self._out[turn] is None:
             pm = ops.jobs_params(self._params(0, 1, 1), self._Jmax)
-            self._out[turn] = (ops._spectrum_out(pm, self.store_arrays, None, self.device),
-                               ops._xcorr_out(pm, self.store_arrays, None, self.device))
+            e = lambda C_: torch.empty((self._Jmax, C_), dtype=torch.float64, device=self.device)
+            q = {}
+            if self.snr:
+                q['snr_db'] = e(self.R)
+                if self.peak_max_samples:       # the gate only acts on the running means
+                    q.update(gated_freq=e(self.R), gated_lag=e(self.P))
+            self._out[turn] = (ops._spectrum_out(pm, self.store_arrays or self.snr, None, self.device),
+                               ops._xcorr_out(pm, self.store_arrays, None, self.device), q)
         return [{k: None if v is None else v[:J] for k, v in d.items()} for d in self._out[turn]]
 
     def _step_signals(self, samples, timestamps, S, T, _count_roi, _designed, plan=None) -> StepResult:
@@ -640,14 +691,16 @@ class BatchedSignalProcessor:
         else:
             ops.window_filter_jobs(self.ring_t, self.ring_y, p, self._ws, js, jh, J, px, py, st,
                                    cache=self._dcache if has_filter else None)
-        spo, xco = self._outputs(turn, J)
+        spo, xco, qo = self._outputs(turn, J)
         p = pj
         # (windows over 320 samples: the entry point itself runs the two stand-alone launches, on this stream)
         fb, lb = ops.peak_band(self.freq_band, 'freq_band'), ops.peak_band(self.lag_band, 'lag_band')
         fused = (bool(self.overlap & OVERLAP_FUSED) and self.P > 0 and self.transform == _cabi.PGRAM_WELCH
                  and fb is None and lb is None)       # the fused grid has no band: two kernels instead
+        store_spec = self.store_arrays or self.snr
         if fused:
-            sp, xc = ops.window_welch_xcorr(px, py, p, store=self.store_arrays, out_spectrum=spo, out_xcorr=xco)
+            sp, xc = ops.window_welch_xcorr(px, py, p, store=store_spec, out_spectrum=spo, out_xcorr=xco,
+                                            store_xcorr=self.store_arrays)
         elif (self.overlap & OVERLAP_XCORR) and self.P:
             # launch order matters for co-residency: the spectrum kernels' CTAs are small (Welch: 24 KB of shared memory),
             # the xcorr CTAs large (51 KB); with xcorr first its 4 CTAs fill an SM's shared memory and the spectrum only
@@ -658,16 +711,23 @@ class BatchedSignalProcessor:
             side.wait_event(ev['pre'])
             xc_first = os.environ.get('BPV_XC_FIRST', '') == '1'
             if not xc_first:
-                sp = ops.window_spectrum(px, py, p, store=self.store_arrays, workspace=self._ws_spec, out=spo, band=fb)
+                sp = ops.window_spectrum(px, py, p, store=store_spec, workspace=self._ws_spec, out=spo, band=fb)
             with torch.cuda.stream(side):
                 xc = ops.window_xcorr(px, py, p, store=self.store_arrays, out=xco, band=lb)
                 ev['xc'].record(side)
             if xc_first:
-                sp = ops.window_spectrum(px, py, p, store=self.store_arrays, workspace=self._ws_spec, out=spo, band=fb)
+                sp = ops.window_spectrum(px, py, p, store=store_spec, workspace=self._ws_spec, out=spo, band=fb)
             main.wait_event(ev['xc'])
         else:
-            sp = ops.window_spectrum(px, py, p, store=self.store_arrays, workspace=self._ws_spec, out=spo, band=fb)
+            sp = ops.window_spectrum(px, py, p, store=store_spec, workspace=self._ws_spec, out=spo, band=fb)
             xc = ops.window_xcorr(px, py, p, store=self.store_arrays, out=xco, band=lb)
+        gate = self.snr and self._min_snr_db is not None and self.peak_max_samples > 0
+        if self.snr:
+            # after F3 and, on the two-stream schedule, after the xcorr event: the gate reads lag_sec
+            band = fb if fb is not None else (self.kw['min_freq'], self.kw['max_freq'])
+            qo = ops.window_snr(sp['freqs'], sp['mags'], sp['num_bins'], sp['peak_idx'], self.transform, band, self.snr_half_width,
+                                min_snr_db=self._min_snr_db if gate else None, peak_freq=sp['peak_freq'] if gate else None,
+                                lag_sec=xc['lag_sec'] if gate else None, out=qo)
         if not self.store_arrays and self.discard_scratch:
             # the processed windows are dead now: drop their dirty L2 lines instead of letting the next step's ROI sampling
             # push them out to DRAM (F1 64.5 -> 69.7 us with 80 MB of dirty scratch in L2, profiles/r2p_f1_dirty.txt)
@@ -687,16 +747,21 @@ class BatchedSignalProcessor:
         self.launches_per_step = roi_launches + n_push + n_pre + n_spec + (1 if self.P and not (fused and self.W <= 320) else 0)
         if not self.store_arrays and self.discard_scratch:
             self.launches_per_step += 1 if J == self._Jmax else 2
+        self.launches_per_step += 1 if self.snr else 0
         arrays = {}
         if self.store_arrays:
             arrays = dict(proc_x=px, proc_y=py, freqs=sp['freqs'], mags=sp['mags'], num_bins=sp['num_bins'],
                           lags=xc['lags'], corr=xc['corr'], num_lags=xc['num_lags'])
+        # the running means push the gated values: a rejected heart rate / PTT enters the history as NaN
+        bpm_in = qo['gated_freq'] if gate else sp['peak_freq']
+        ptt_in = qo['gated_lag'] if gate else xc['lag_sec']
+        snr_db = qo['snr_db'] if self.snr else None
         means = {}
         if self.peak_max_samples and lock:
-            mb, mbi = ops.running_mean(self._bpm_ring, self._mcnt, sp['peak_freq'].view(S, jobs, self.R), 60.0)
+            mb, mbi = ops.running_mean(self._bpm_ring, self._mcnt, bpm_in.view(S, jobs, self.R), 60.0)
             means = dict(mean_bpm=mb.view(J, self.R), mean_bpm_int=mbi.view(J, self.R))
             if self.P:
-                mp, mpi = ops.running_mean(self._ptt_ring, self._mcnt, xc['lag_sec'].view(S, jobs, self.P), 1000.0)
+                mp, mpi = ops.running_mean(self._ptt_ring, self._mcnt, ptt_in.view(S, jobs, self.P), 1000.0)
                 means.update(mean_ptt=mp.view(J, self.P), mean_ptt_int=mpi.view(J, self.P))
             self._mcnt += jobs
             self.launches_per_step += 2 if self.P else 1
@@ -705,19 +770,19 @@ class BatchedSignalProcessor:
             pin = self._pinned(turn)
             pin['m0'].numpy()[:] = mcnt
             self._mg0.copy_(pin['m0'], non_blocking=True)
-            mb, mbi = ops.running_mean_jobs(self._bpm_ring, self._mg0, sj0, sp['peak_freq'], 60.0)
+            mb, mbi = ops.running_mean_jobs(self._bpm_ring, self._mg0, sj0, bpm_in, 60.0)
             means = dict(mean_bpm=mb, mean_bpm_int=mbi)
             if self.P:
-                mp, mpi = ops.running_mean_jobs(self._ptt_ring, self._mg0, sj0, xc['lag_sec'], 1000.0)
+                mp, mpi = ops.running_mean_jobs(self._ptt_ring, self._mg0, sj0, ptt_in, 1000.0)
                 means.update(mean_ptt=mp, mean_ptt_int=mpi)
             self._mcnt = self._level(mcnt + plan['jobs'])
             self.launches_per_step += 2 if self.P else 1
         if lock:
             return StepResult(jobs, samples, sp['peak_freq'], sp['peak_idx'], sp['peak_mag'], xc['lag_sec'], xc['lag_idx'],
-                              xc['lag_corr'], st, arrays, means)
+                              xc['lag_corr'], st, arrays, means, snr_db=snr_db)
         self._advance(plan, turn, main)
         return StepResult(None, samples, sp['peak_freq'], sp['peak_idx'], sp['peak_mag'], xc['lag_sec'], xc['lag_idx'],
-                          xc['lag_corr'], st, arrays, means, _job_offsets=plan['off'], _job_stream=js[:J])
+                          xc['lag_corr'], st, arrays, means, _job_offsets=plan['off'], _job_stream=js[:J], snr_db=snr_db)
 
     def _advance(self, plan: dict, turn: int, main) -> None:
         """End of a job-map step on the host: the staging of `turn` is in flight until the device passes this point, and

@@ -6,6 +6,7 @@ computes on the host.
 from __future__ import annotations
 
 import ctypes as C
+import math
 
 import torch
 
@@ -310,13 +311,16 @@ def _xcorr_out(p: WindowParams, store: bool, out, dev) -> dict:
     return o
 
 
-def window_welch_xcorr(proc_x, proc_y, p: WindowParams, store: bool = True, out_spectrum=None, out_xcorr=None):
+def window_welch_xcorr(proc_x, proc_y, p: WindowParams, store: bool = True, out_spectrum=None, out_xcorr=None,
+                       store_xcorr: bool | None = None):
     """F3 (PGRAM_WELCH) + F4 of the same window jobs in ONE grid of interleaved Welch / xcorr CTAs (include/bpv.h
-    bpv_window_welch_xcorr).  Returns the dicts of window_spectrum and window_xcorr; same values bit for bit."""
+    bpv_window_welch_xcorr).  Returns the dicts of window_spectrum and window_xcorr; same values bit for bit.
+    store: keep the spectrum; store_xcorr: keep the correlations (None = as `store`)."""
     if p.transform != _cabi.PGRAM_WELCH or p.R < 2:
         raise ValueError('window_welch_xcorr: PGRAM_WELCH and at least two ROIs')
     dev = proc_y.device
-    sp, xc = _spectrum_out(p, store, out_spectrum, dev), _xcorr_out(p, store, out_xcorr, dev)
+    store_xcorr = store if store_xcorr is None else store_xcorr
+    sp, xc = _spectrum_out(p, store, out_spectrum, dev), _xcorr_out(p, store_xcorr, out_xcorr, dev)
     _run(dev, 'bpv_window_welch_xcorr', ptr(proc_x), ptr(proc_y), C.byref(p), max_bins(p), ptr(sp['freqs']), ptr(sp['mags']),
          ptr(sp['num_bins']), ptr(sp['peak_idx']), ptr(sp['peak_freq']), ptr(sp['peak_mag']), ptr(xc['lags']), ptr(xc['corr']),
          ptr(xc['num_lags']), ptr(xc['lag_idx']), ptr(xc['lag_sec']), ptr(xc['lag_corr']))
@@ -377,6 +381,67 @@ def window_xcorr(proc_x, proc_y, p: WindowParams, store: bool = True, out=None, 
             _run(proc_y.device, 'bpv_window_xcorr', *args)
         else:
             _run(proc_y.device, 'bpv_window_xcorr_band', *args, *band)
+    return o
+
+
+SNR_HALF_WIDTH = 0.125      # Hz (7.5 bpm): the peak bin and its two neighbours on the 0.1 / 0.117 Hz DFT / Welch grids
+
+
+def snr_half_width(value) -> float:
+    """The template half-width of window_snr in Hz: a finite number >= 0."""
+    try:
+        v = float(value)
+    except (TypeError, ValueError):
+        raise ValueError(f'snr_half_width must be a number, not {value!r}') from None
+    if not (math.isfinite(v) and v >= 0.0):
+        raise ValueError(f'snr_half_width must be finite and >= 0, not {value!r}')
+    return v
+
+
+def snr_threshold(value):
+    """None, or the SNR gate threshold in dB as a float (-inf allowed, NaN rejected)."""
+    if value is None:
+        return None
+    try:
+        v = float(value)
+    except (TypeError, ValueError):
+        raise ValueError(f'min_snr_db must be None or a number, not {value!r}') from None
+    if v != v:
+        raise ValueError('min_snr_db must not be NaN')
+    return v
+
+
+def window_snr(freqs, mags, num_bins, peak_idx, transform: int, band, half_width: float = SNR_HALF_WIDTH, *,
+               min_snr_db=None, peak_freq=None, lag_sec=None, out=None) -> dict:
+    """Spectral SNR of the heart-rate peak of every window (include/bpv.h bpv_window_snr) from the spectrum F3 stored:
+    freqs, mags f32 [J,R,max_bins], num_bins, peak_idx i32 [J,R]; band = (lo, hi) in Hz.  Returns dict(snr_db f64 [J,R]),
+    plus, when min_snr_db is set, gated_freq f64 [J,R] (with peak_freq) and gated_lag f64 [J,P] (with lag_sec): the values
+    where snr_db >= min_snr_db (both ROIs of a pair for a lag), NaN elsewhere.  out: preallocated tensors by those names."""
+    lo, hi = peak_band(band, 'band')
+    hw, thr = snr_half_width(half_width), snr_threshold(min_snr_db)
+    J, R, mb = mags.shape
+    P = R * (R - 1) // 2
+    _require(freqs.shape == mags.shape and freqs.dtype == mags.dtype == torch.float32 and freqs.is_contiguous() and mags.is_contiguous(),
+             'window_snr: freqs / mags must be contiguous float32 [J, R, max_bins]')
+    _require(all(t.shape == (J, R) and t.dtype == torch.int32 and t.is_contiguous() for t in (num_bins, peak_idx)),
+             'window_snr: num_bins / peak_idx must be contiguous int32 [J, R]')
+    for t, shape, name in ((peak_freq, (J, R), 'peak_freq'), (lag_sec, (J, P), 'lag_sec')):
+        _require(t is None or (t.shape == shape and t.dtype == torch.float64 and t.is_contiguous()),
+                 f'window_snr: {name} must be contiguous float64 {list(shape)}')
+    dev = mags.device
+    o = dict(out or {})
+    if 'snr_db' not in o:
+        o['snr_db'] = torch.empty((J, R), dtype=torch.float64, device=dev)
+    gf = gl = None
+    if thr is not None and peak_freq is not None:
+        gf = o.get('gated_freq')
+        o['gated_freq'] = gf = torch.empty((J, R), dtype=torch.float64, device=dev) if gf is None else gf
+    if thr is not None and lag_sec is not None:
+        gl = o.get('gated_lag')
+        o['gated_lag'] = gl = torch.empty((J, P), dtype=torch.float64, device=dev) if gl is None else gl
+    if J:
+        _run(dev, 'bpv_window_snr', ptr(freqs), ptr(mags), ptr(num_bins), ptr(peak_idx), J, R, mb, int(transform), lo, hi, hw,
+             ptr(peak_freq), ptr(lag_sec), P, -math.inf if thr is None else thr, ptr(o['snr_db']), ptr(gf), ptr(gl) if P else None)
     return o
 
 

@@ -339,6 +339,31 @@ int bpv_window_welch_xcorr(const double* proc_x, const double* proc_y, const bpv
                            double* peak_mag, float* corr_lag, float* corr_val, int32_t* num_lags, int32_t* lag_idx,
                            double* lag_sec, double* lag_corr, void* stream);
 
+/* Per-window signal quality: spectral SNR of the heart-rate peak (de Haan & Jeanne, IEEE TBME 2013) over the spectrum
+ *     F3 stored, and the SNR gate of the values the running means push.  No reference counterpart: process() reports a
+ *     peak for every window, whether the ROI held a pulse or not.
+ * Inputs: spec_f, spec_mag float32 [J, R, max_bins], num_bins, peak_idx int32 [J, R] as bpv_window_spectrum(_band) wrote
+ * them.  For signal (j, r), in float64 arithmetic on the stored float32 values f_k, m_k widened to float64:
+ *   - bin power P_k = m_k^2 for BPV_DFT_RFFT (the stored spectrum is the amplitude 2|X|/n), m_k for PGRAM_WELCH / PGRAM_LS;
+ *   - B = the bins k < num_bins with a finite m_k and lo <= f_k <= hi;
+ *   - f0 = f_{peak_idx}; a bin is in the template when |f_k - f0| <= half_width or |f_k - 2 f0| <= half_width (Hz);
+ *   - S_sig = sum of P_k over B within the template, S_noise = over B outside it;
+ *   - snr_db = 10 log10(S_sig / S_noise) with IEEE semantics (0/x -> -inf, x/0 -> +inf, 0/0 -> NaN); NaN when
+ *     peak_idx < 0 or |B| < 2.  A DC peak of the unbanded search puts no template bin in a band above 0 Hz: -inf.
+ * B is decided on the stored float32 frequencies, so it can differ from the band of bpv_window_spectrum_band (which decides
+ * on float64 frequencies) in a bin that lies within float32 rounding of lo or hi.  The sums are float64 in a fixed lane
+ * order and shuffle tree: reproducible from run to run.
+ * Gate (optional outputs, NULL to skip): a heart rate is accepted when snr_db >= min_snr_db (NaN is rejected); the PTT of
+ * pair (a, b), itertools.combinations order, when both a and b are.  gated_freq [J, R] = peak_freq where accepted, else
+ * NaN; gated_lag [J, P] = lag_sec likewise.  snr_db float64 [J, R] is always written.  P must be R(R-1)/2.
+ * BPV_E_INVALID before anything is enqueued: a NaN bound, a negative or non-finite half_width, a NaN min_snr_db (-inf is
+ * allowed), J < 0, R < 1, max_bins < 1, a bad P or transform, a NULL input / snr_db, gated_freq without peak_freq,
+ * gated_lag without lag_sec.  J = 0 enqueues nothing.  lo > hi leaves B empty (NaN). */
+int bpv_window_snr(const float* spec_f, const float* spec_mag, const int32_t* num_bins, const int32_t* peak_idx,
+                   int64_t J, int32_t R, int32_t max_bins, int32_t transform, double lo, double hi, double half_width,
+                   const double* peak_freq, const double* lag_sec, int32_t P, double min_snr_db,
+                   double* snr_db, double* gated_freq, double* gated_lag, void* stream);
+
 /* Filter design alone (debug / parity of make_filter, signal_processor.py:158-173).
  * fs float64 [n]; sos_out float64 [n, order, 6]; taps_out float64 [n, fir_taps]. */
 int bpv_butter_sos_design(const double* fs, int32_t n, const bpv_window_params* p, double* sos_out, void* stream);
