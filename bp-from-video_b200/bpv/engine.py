@@ -108,6 +108,53 @@ def cadence_jobs(counts, n, stride, phase):
     return jobs, int(np.sum(jobs)), (b + 1) * stride - phase - 1
 
 
+@dataclass(slots=True)
+class StepPlan:
+    """What the stages of one step need, decided before anything is enqueued.  Lockstep: `jobs` per stream at heads head0 +
+    i * head_step.  Job map: jobs, offsets `off` and frames `n` per stream.  p / pj / max_bins: set when J > 0."""
+    T: int
+    lock: bool
+    J: int
+    jobs: int | np.ndarray
+    head0: int = 0
+    head_step: int = 1
+    n: np.ndarray | None = None
+    off: np.ndarray | None = None
+    cad: tuple[np.ndarray, np.ndarray] | None = None     # strides and phases; None = a job after every frame
+    freq_band: tuple[float, float] | None = None
+    lag_band: tuple[float, float] | None = None
+    has_filter: bool = False
+    p: _cabi.WindowParams | None = None
+    pj: _cabi.WindowParams | None = None
+    max_bins: int = 0
+    launches: int = 0                                    # kernels the step's stages enqueued so far
+
+
+def plan_jobs(S: int, counts, mean_counts, n, T: int, cad=None, *, last: bool = False, force_jobmap: bool = False):
+    """The window jobs of a step of T frames from host values: sample and running-mean history counts (one int while
+    level, else int64 [S]), frames taken n (int64 [S]; None = T each), cad = (strides, phases) int64 [S] or None.  None
+    when no stream takes a frame; lockstep when every stream takes T frames from level counts with one stride and one
+    phase (unless force_jobmap); else a job map."""
+    if n is not None and not n.any():
+        return None
+    uniform = cad is None or bool((cad[0] == cad[0][0]).all() and (cad[1] == cad[1][0]).all())
+    if ((n is None or bool((n == T).all())) and isinstance(counts, int) and isinstance(mean_counts, int) and uniform
+            and not force_jobmap):
+        if cad is not None:
+            k = int(cad[0][0])
+            jobs, _, head0 = cadence_jobs(counts, T, k, int(cad[1][0]))
+            return StepPlan(T, True, S * jobs, jobs, head0=head0, head_step=k, cad=cad)
+        return StepPlan(T, True, S, 1, head0=counts + T - 1) if last else StepPlan(T, True, S * T, T, head0=counts)
+    n = np.full(S, T, dtype=np.int64) if n is None else n
+    if cad is not None:
+        jobs = cadence_jobs(counts, n, *cad)[0]
+    else:
+        jobs = (n > 0).astype(np.int64) if last else n
+    off = np.zeros(S + 1, dtype=np.int64)
+    np.cumsum(jobs, out=off[1:])
+    return StepPlan(T, False, int(off[-1]), jobs, n=n, off=off, cad=cad)
+
+
 @dataclass
 class StepResult:
     """Device tensors for the J window jobs of one step.  A lockstep step has J = S * jobs_per_stream (job =
@@ -240,14 +287,11 @@ class BatchedSignalProcessor:
         self._proc = [torch.empty((2, Jmax, self.R, self.W), dtype=f64, device=dev) for _ in range(nproc)]   # [x | y]
         self._status = [torch.empty((Jmax, self.R), dtype=torch.int32, device=dev) for _ in range(self._nbuf)]
         self._out = [None] * self._nbuf          # per result buffer: F3 / F4 outputs of Jmax jobs, sliced to each step's J
-        p = self._params(0, 1, self.Tmax if windows == EVERY_FRAME else 1)
-        self._mb = ops.max_bins(p)
-        need = max(_cabi.lib().bpv_window_workspace_bytes(p), 16)
+        need = max(_cabi.lib().bpv_window_workspace_bytes(self._params(0, 1, Jmax // self.S)), 16)
         self._ws = torch.empty(need, dtype=torch.uint8, device=dev)                 # per-job filter designs
-        need = max(_cabi.lib().bpv_spectrum_workspace_bytes(p, self._mb), 16)
-        self._ws_spec = torch.zeros(need, dtype=torch.uint8, device=dev)    # zeroed: holds the DFT twiddle images' header
-        self.launches_per_step = self._extra_launches = 0
-        self._has_filter = any(m in (_cabi.FILTER_BUTTER, _cabi.FILTER_FIR) for m in self.methods)
+        # F3's workspace (zeroed: holds the DFT twiddle images' header), sized by _outputs for the (transform, bins) in _spec_key
+        self._ws_spec, self._spec_key = torch.zeros(16, dtype=torch.uint8, device=dev), None
+        self.launches_per_step = 0
         # design cache (include/bpv.h bpv_window_design): make_filter is a pure function of fs, so sampling rates that were
         # designed before — constant-fps streams: every window of every stream on that clock — are looked up, not redesigned
         if design_cache is None:
@@ -312,6 +356,11 @@ class BatchedSignalProcessor:
         return np.full(self.S, self._cnt, dtype=np.int64) if isinstance(self._cnt, int) else self._cnt.copy()
 
     @property
+    def mean_counts(self) -> np.ndarray:
+        """Host int64 [S]: values pushed so far per stream into the running-mean histories (peak_max_samples)."""
+        return np.full(self.S, self._mcnt, dtype=np.int64) if isinstance(self._mcnt, int) else self._mcnt.copy()
+
+    @property
     def count(self) -> int:
         """The samples pushed per stream while every stream holds the same count; raises ValueError otherwise (see
         `counts`).  Assigning it sets every stream's count."""
@@ -345,18 +394,9 @@ class BatchedSignalProcessor:
             raise ValueError(f'{name} must be integers, got {a.dtype}')
         return a.astype(np.int64)
 
-    def _frame_counts(self, frame_counts, T: int):
-        """frame_counts (host sequence / numpy array / CPU int tensor of S values in 0..T) as int64 [S], or None."""
-        if frame_counts is None:
-            return None
-        a = self._host_ints(frame_counts, 'frame_counts')
-        if a.size and (a.min() < 0 or a.max() > T):
-            raise ValueError(f'frame_counts must lie in [0, {T}]')
-        return a
-
     def _cadence(self):
         """window_stride / window_phase checked for the coming step: None for the default (a job after every frame), else
-        dict(k=, phase= host int64 [S], uniform= one k and one phase for every stream)."""
+        (strides, phases) as host int64 [S]."""
         k, ph = self.window_stride, self.window_phase
         if type(k) is int and type(ph) is int and k == 1 and ph == 0:
             return None
@@ -369,74 +409,67 @@ class BatchedSignalProcessor:
             return None
         if self.windows == LAST:
             raise ValueError("window_stride != 1 needs windows='every_frame' ('last' has its own cadence)")
-        return dict(k=k, phase=ph, uniform=bool((k == k[0]).all() and (ph == ph[0]).all()))
+        return k, ph
 
-    def _lockstep(self, n, T: int, cad) -> bool:
-        """The lockstep path serves a step in which every stream takes T frames from the same counts with the same cadence."""
-        return ((n is None or bool((n == T).all())) and isinstance(self._cnt, int) and isinstance(self._mcnt, int)
-                and (cad is None or cad['uniform']) and not self.force_jobmap)
+    def _plan(self, S: int, T: int, timestamps, frame_counts, boxes=None) -> StepPlan | None:
+        """The plan of a step of S x T frames, after every check that can raise ValueError; None when no stream takes a
+        frame."""
+        if S != self.S or not 1 <= T <= self.Tmax:
+            raise ValueError(f'step: expected {self.S} streams and 1..{self.Tmax} frames per stream, got {S} x {T}')
+        if tuple(timestamps.shape) != (S, T):
+            raise ValueError(f'step: timestamps must be [{S}, {T}], got {tuple(timestamps.shape)}')
+        if boxes is not None and tuple(boxes.shape) != (S, T, self.R, 4):
+            raise ValueError(f'step: boxes must be int32 [{S}, {T}, {self.R}, 4], got {tuple(boxes.shape)}')
+        cad = self._cadence()
+        if self.snr:
+            self.snr_half_width = ops.snr_half_width(self.snr_half_width)
+        fb, lb = ops.peak_band(self.freq_band, 'freq_band'), ops.peak_band(self.lag_band, 'lag_band')
+        n = None if frame_counts is None else self._host_ints(frame_counts, 'frame_counts')
+        if n is not None and (n.min() < 0 or n.max() > T):
+            raise ValueError(f'frame_counts must lie in [0, {T}]')
+        plan = plan_jobs(self.S, self._cnt, self._mcnt, n, T, cad, last=self.windows == LAST, force_jobmap=self.force_jobmap)
+        if plan is None:
+            self.launches_per_step = 0          # a step without frames enqueues nothing
+            return None
+        plan.freq_band, plan.lag_band = fb, lb
+        plan.has_filter = any(m in (_cabi.FILTER_BUTTER, _cabi.FILTER_FIR) for m in self.methods)
+        if plan.J:
+            # job-map path: F2 reads the rings through the job map; F3 / F4 see the J jobs as J streams of one job (include/bpv.h)
+            plan.p = self._params(plan.head0, plan.head_step, plan.jobs) if plan.lock else self._params(0, 1, 1)
+            plan.pj = plan.p if plan.lock else ops.jobs_params(plan.p, plan.J)
+            plan.max_bins = ops.max_bins(plan.p)
+        return plan
 
-    def _plan(self, n, T: int, cad) -> dict | None:
-        """Host side of a step: None for a lockstep step at the default cadence; for a strided lockstep step its head0,
-        head_step, jobs per stream and J; for a job-map step the per-stream frame counts, job counts, offsets and J."""
-        if self._lockstep(n, T, cad):
-            if cad is None:
-                return None
-            k, ph = int(cad['k'][0]), int(cad['phase'][0])
-            jobs, _, head0 = cadence_jobs(self._cnt, T, k, ph)
-            return dict(lock=True, head0=head0, head_step=k, jobs=jobs, J=self.S * jobs)
-        n = np.full(self.S, T, dtype=np.int64) if n is None else n
-        if cad is not None:
-            jobs = cadence_jobs(self.counts, n, cad['k'], cad['phase'])[0]
-        else:
-            jobs = n if self.windows == EVERY_FRAME else (n > 0).astype(np.int64)
-        off = np.zeros(self.S + 1, dtype=np.int64)
-        np.cumsum(jobs, out=off[1:])
-        return dict(lock=False, n=n, jobs=jobs, off=off, J=int(off[-1]), T=T, mapped=False, cad=cad)
-
-    def _lock_jobs(self, T: int, plan):
-        """(head0, head_step, jobs per stream) of a lockstep step from the current count."""
-        if plan is not None:
-            return plan['head0'], plan['head_step'], plan['jobs']
-        if self.windows == EVERY_FRAME:
-            return self._cnt, 1, T
-        return self._cnt + T - 1, 1, 1
-
-    def _map_jobs(self, plan: dict, turn: int) -> None:
+    def _map_jobs(self, plan: StepPlan, turn: int) -> None:
         """Upload the step's frame counts (and the sample counts when the device copy is stale) and build the job map of
-        the plan on the device (bpv_stream_jobs), into the buffers of result turn `turn`."""
+        the plan on the device (bpv_stream_jobs / bpv_stream_jobs_strided), into the buffers of result turn `turn`."""
         dev = self.device
         if self._jobmap[turn] is None:
             self._jobmap[turn] = (torch.empty(self._Jmax, dtype=torch.int32, device=dev),
                                   torch.empty(self._Jmax, dtype=torch.int64, device=dev),
                                   torch.empty(self.S + 1, dtype=torch.int32, device=dev))
         pin = self._pinned(turn)
-        pin['n'].numpy()[:] = plan['n']
+        pin['n'].numpy()[:] = plan.n
         self._ndev.copy_(pin['n'], non_blocking=True)
         if not self._g0_ok:
             pin['g0'].numpy()[:] = self.counts
             self._g0[0].copy_(pin['g0'], non_blocking=True)
             self._g0_ok = True
         js, jh, sj0 = self._jobmap[turn]
-        if plan['cad'] is None:
-            ops.stream_jobs(self._g0[0], self._ndev, self.windows == LAST, plan['J'], js, jh, sj0, self._g0[1])
+        if plan.cad is None:
+            ops.stream_jobs(self._g0[0], self._ndev, self.windows == LAST, plan.J, js, jh, sj0, self._g0[1])
         else:
-            kd, pd = self._cadence_dev(plan['cad'], pin)
-            ops.stream_jobs_strided(self._g0[0], self._ndev, kd, pd, plan['J'], js, jh, sj0, self._g0[1])
-        plan['mapped'] = True
-
-    def _cadence_dev(self, cad: dict, pin: dict):
-        """Device int32 [S] copies of the strides and phases, uploaded through the pinned staging `pin` when they changed."""
-        if self._cad_dev is None:
-            self._cad_dev = tuple(torch.empty(self.S, dtype=torch.int32, device=self.device) for _ in range(2))
-        host = self._cad_host
-        if host is None or not (np.array_equal(host[0], cad['k']) and np.array_equal(host[1], cad['phase'])):
-            pin['k'].numpy()[:] = cad['k']
-            pin['ph'].numpy()[:] = cad['phase']
-            self._cad_dev[0].copy_(pin['k'], non_blocking=True)
-            self._cad_dev[1].copy_(pin['ph'], non_blocking=True)
-            self._cad_host = (cad['k'].copy(), cad['phase'].copy())
-        return self._cad_dev
+            # device int32 copies of the strides and phases, uploaded through the pinned staging when they changed
+            k, ph = plan.cad
+            if self._cad_dev is None:
+                self._cad_dev = tuple(torch.empty(self.S, dtype=torch.int32, device=dev) for _ in range(2))
+            if self._cad_host is None or not (np.array_equal(self._cad_host[0], k) and np.array_equal(self._cad_host[1], ph)):
+                pin['k'].numpy()[:], pin['ph'].numpy()[:] = k, ph
+                self._cad_dev[0].copy_(pin['k'], non_blocking=True)
+                self._cad_dev[1].copy_(pin['ph'], non_blocking=True)
+                self._cad_host = (k.copy(), ph.copy())
+            ops.stream_jobs_strided(self._g0[0], self._ndev, *self._cad_dev, plan.J, js, jh, sj0, self._g0[1])
+        plan.launches += 1
 
     def _pinned(self, turn: int) -> dict:
         """Pinned staging buffers of result turn `turn`, once the device has consumed their previous contents."""
@@ -449,12 +482,6 @@ class BatchedSignalProcessor:
             pin['ev'].synchronize()
             pin['used'] = False
         return pin
-
-    def _check_step(self, S, T, boxes=None):
-        if S != self.S or not 1 <= T <= self.Tmax:
-            raise ValueError(f'step: expected {self.S} streams and 1..{self.Tmax} frames per stream, got {S} x {T}')
-        if boxes is not None and tuple(boxes.shape) != (S, T, self.R, 4):
-            raise ValueError(f'step: boxes must be int32 [{S}, {T}, {self.R}, 4], got {tuple(boxes.shape)}')
 
     def step(self, frames: torch.Tensor, boxes: torch.Tensor, timestamps: torch.Tensor, view=None, nv12_size=None,
              resize_to=None, masks: torch.Tensor | None = None, mask_category=0, frame_counts=None) -> StepResult:
@@ -471,79 +498,39 @@ class BatchedSignalProcessor:
         frames.  F1 still samples all S x T rows; the rows a stream does not take cost next to nothing when their boxes
         are BPV_NO_BOX (x0 = NO_BOX).  A step in which no stream takes a frame enqueues nothing (samples = None)."""
         S, T = frames.shape[:2]
-        self._check_step(S, T, boxes)
-        cad = self._cadence()
-        if self.snr:
-            self.snr_half_width = ops.snr_half_width(self.snr_half_width)
-        n = self._frame_counts(frame_counts, T)
-        if n is not None and not n.any():
+        plan = self._plan(S, T, timestamps, frame_counts, boxes)
+        if plan is None:
             return self._empty_step(None)
-        self._extra_launches = 0
-        with torch.cuda.device(self.device):
+        designed, dev = False, self.device
+        with torch.cuda.device(dev):
             if view is not None:
                 boxes = ops.view_boxes(boxes.contiguous(), *view)
-                self._extra_launches = 1
+                plan.launches += 1
+            fr, bx = frames.view(S * T, *frames.shape[2:]), boxes.reshape(S * T, self.R, 4).contiguous()
             if resize_to is not None:
                 # boxes live in the frame cv2.resize(frame, (dst_w, dst_h)) would produce (video_reader.py:95-96); pixels
                 # are generated on the fly with OpenCV's integer bilinear arithmetic, the resized frame is never materialised
-                dst_h, dst_w = resize_to
-                val, _ = ops.roi_sample_resized(frames.view(S * T, *frames.shape[2:]), dst_h, dst_w,
-                                                boxes.reshape(S * T, self.R, 4).contiguous(), self.color_channel)
-                return self.step_signals(val.view(S, T, self.R), timestamps, _count_roi=True, frame_counts=n)
-            if nv12_size is not None:
-                H, W = nv12_size
-                val, _ = ops.roi_sample_nv12(frames.view(S * T, *frames.shape[2:]), H, W,
-                                             boxes.reshape(S * T, self.R, 4).contiguous(), self.color_channel)
-                return self.step_signals(val.view(S, T, self.R), timestamps, _count_roi=True, frame_counts=n)
-            if masks is not None:
-                val, _ = ops.roi_sample_masked(frames.view(S * T, *frames.shape[2:]), masks.view(S * T, *masks.shape[2:]),
-                                               mask_category, boxes.reshape(S * T, self.R, 4).contiguous(),
-                                               self.color_channel)
-                return self.step_signals(val.view(S, T, self.R), timestamps, _count_roi=True, frame_counts=n)
-            samples = self._samples[self._turn][:, :T]
-            if T != self.Tmax:
-                samples = torch.empty((S, T, self.R), dtype=torch.float64, device=self.device)
-            plan = self._plan(n, T, cad)
-            design_ahead = (bool(self.overlap & OVERLAP_DESIGN)
-                            and any(m in (_cabi.FILTER_BUTTER, _cabi.FILTER_FIR) for m in self.methods)
-                            and (plan is None or plan['J'] > 0))      # a step without jobs has nothing to design
-            if design_ahead and (plan is None or plan['lock']):
-                self._design_ahead(timestamps, T, plan)
-            elif design_ahead:
-                self._design_ahead_jobs(timestamps, plan)
-            ops.roi_sample(frames.view(S * T, *frames.shape[2:]), boxes.view(S * T, self.R, 4), self.color_channel,
-                           roi_pixels_hint=self.roi_pixels_hint, out_value=samples.view(S * T, self.R))
-            return self.step_signals(samples, timestamps, _count_roi=True, _designed=design_ahead, frame_counts=n, _plan=plan)
-
-    def _design_ahead(self, timestamps: torch.Tensor, T: int, plan) -> None:
-        """Push the step's timestamps and start the filter design of its window jobs on the side stream: make_filter
-        depends on nothing else (signal_processor.py:158-173), so it runs beside F1 instead of between F1 and F2."""
-        _, ev = self._streams()
-        side = self._side_hi
-        main = torch.cuda.current_stream(self.device)
-        ops.ring_push(self.ring_t, self.ring_y, self._cnt, timestamps.contiguous(), None)
-        ev['ts'].record(main)
-        head0, head_step, jobs = self._lock_jobs(T, plan)
-        p = self._params(head0, head_step, jobs)
-        side.wait_event(ev['ts'])
-        with torch.cuda.stream(side):
-            ops.window_design(self.ring_t, p, self._ws, self._cache())
-            ev['design'].record(side)
-
-    def _design_ahead_jobs(self, timestamps: torch.Tensor, plan: dict) -> None:
-        """_design_ahead for a job-map step: ragged timestamp push, job map, then the design of the mapped jobs on the
-        side stream."""
-        _, ev = self._streams()
-        side = self._side_hi
-        main = torch.cuda.current_stream(self.device)
-        self._map_jobs(plan, self._turn)
-        ops.ring_push_ragged(self.ring_t, self.ring_y, self._g0[0], self._ndev, timestamps.contiguous(), None)
-        ev['ts'].record(main)
-        js, jh, _ = self._jobmap[self._turn]
-        side.wait_event(ev['ts'])
-        with torch.cuda.stream(side):
-            ops.window_design_jobs(self.ring_t, self._params(0, 1, 1), self._ws, js, jh, plan['J'], self._cache())
-            ev['design'].record(side)
+                samples, _ = ops.roi_sample_resized(fr, *resize_to, bx, self.color_channel)
+            elif nv12_size is not None:
+                samples, _ = ops.roi_sample_nv12(fr, *nv12_size, bx, self.color_channel)
+            elif masks is not None:
+                samples, _ = ops.roi_sample_masked(fr, masks.view(S * T, *masks.shape[2:]), mask_category, bx, self.color_channel)
+            else:
+                samples = self._samples[self._turn] if T == self.Tmax else torch.empty((S, T, self.R), dtype=torch.float64, device=dev)
+                designed = bool(self.overlap & OVERLAP_DESIGN) and plan.has_filter and plan.J > 0
+                if designed:
+                    # make_filter needs only the timestamps (signal_processor.py:158-173): push them and design the step's
+                    # jobs on the side stream, beside F1 instead of between F1 and F2
+                    _, ev = self._streams()
+                    self._push(plan, self._turn, timestamps, None)
+                    ev['ts'].record(torch.cuda.current_stream(self.device))
+                    self._side_hi.wait_event(ev['ts'])
+                    with torch.cuda.stream(self._side_hi):
+                        self._design(plan, self._turn)
+                        ev['design'].record(self._side_hi)
+                ops.roi_sample(fr, bx, self.color_channel, roi_pixels_hint=self.roi_pixels_hint, out_value=samples.view(S * T, self.R))
+            plan.launches += 1
+            return self._run(plan, samples.view(S, T, self.R), timestamps, designed)
 
     def _cache(self):
         """The design cache, emptied whenever the filter parameters it was filled under have changed (the drop-in
@@ -594,50 +581,48 @@ class BatchedSignalProcessor:
                        roi_pixels_hint=self.roi_pixels_hint, out_value=out.view(S * T, self.R))
         return out
 
-    def step_signals(self, samples: torch.Tensor, timestamps: torch.Tensor, _count_roi: bool = False,
-                     _designed: bool = False, frame_counts=None, _plan: dict | None = None) -> StepResult:
+    def step_signals(self, samples: torch.Tensor, timestamps: torch.Tensor, frame_counts=None) -> StepResult:
         """Signals-only entry: samples float64 [S, T, R] (already ROI-sampled), timestamps float64 [S, T].
         frame_counts: as in `step`; stream s takes rows [:n_s] of its samples and timestamps, the others are not read."""
         S, T, R = samples.shape
-        self._check_step(S, T)
-        if R != self.R or tuple(timestamps.shape) != (S, T):
+        if R != self.R:
             raise ValueError(f'step_signals: samples must be [S, T, {self.R}] and timestamps [S, T]')
-        cad = self._cadence()
-        if self.snr:
-            self.snr_half_width = ops.snr_half_width(self.snr_half_width)
-        n = self._frame_counts(frame_counts, T)
-        if n is not None and not n.any():
+        plan = self._plan(S, T, timestamps, frame_counts)
+        if plan is None:
             return self._empty_step(samples)
-        if _plan is None:
-            _plan = self._plan(n, T, cad)
         with torch.cuda.device(self.device):
-            return self._step_signals(samples, timestamps, S, T, _count_roi, _designed, _plan)
+            return self._run(plan, samples, timestamps)
 
-    def _empty_step(self, samples, jobs_per_stream=None, launches: int = 0) -> StepResult:
-        """A result of zero jobs.  A step in which no stream takes a frame enqueues nothing and changes no state; a strided
-        step without jobs has pushed its frames (`launches`)."""
+    def _empty_step(self, samples, plan: StepPlan | None = None) -> StepResult:
+        """A result of zero jobs: of a step without frames (no plan), or of a strided step that pushed frames without a job."""
         dev, f64, f32, i32 = self.device, torch.float64, torch.float32, torch.int32
         R, P, W = self.R, self.P, self.W
         e = lambda *shape, dt=f64: torch.empty(shape, dtype=dt, device=dev)
         arrays, means = {}, {}
         if self.store_arrays:
-            arrays = dict(proc_x=e(0, R, W), proc_y=e(0, R, W), freqs=e(0, R, self._mb, dt=f32), mags=e(0, R, self._mb, dt=f32),
+            mb = ops.max_bins(self._params(0, 1, 1))
+            arrays = dict(proc_x=e(0, R, W), proc_y=e(0, R, W), freqs=e(0, R, mb, dt=f32), mags=e(0, R, mb, dt=f32),
                           num_bins=e(0, R, dt=i32), lags=e(0, P, 2 * W - 1, dt=f32), corr=e(0, P, 2 * W - 1, dt=f32),
                           num_lags=e(0, P, dt=i32))
         if self.peak_max_samples:
             means = dict(mean_bpm=e(0, R), mean_bpm_int=e(0, R))
             if P:
                 means.update(mean_ptt=e(0, P), mean_ptt_int=e(0, P))
-        self.launches_per_step = launches
-        return StepResult(jobs_per_stream, samples, e(0, R), e(0, R, dt=i32), e(0, R), e(0, P), e(0, P, dt=i32), e(0, P),
-                          e(0, R, dt=i32), arrays, means, _job_offsets=np.zeros(self.S + 1, dtype=np.int64),
-                          _job_stream=e(0, dt=i32), snr_db=e(0, R) if self.snr else None)
+        return StepResult(0 if plan is not None and plan.lock else None, samples, e(0, R), e(0, R, dt=i32), e(0, R), e(0, P),
+                          e(0, P, dt=i32), e(0, P), e(0, R, dt=i32), arrays, means,
+                          _job_offsets=np.zeros(self.S + 1, dtype=np.int64), _job_stream=e(0, dt=i32),
+                          snr_db=e(0, R) if self.snr else None)
 
-    def _outputs(self, turn: int, J: int):
-        """F3 / F4 (and SNR, with snr=True) output dicts of a step: views of the first J rows of result turn `turn`'s
-        Jmax-row buffers.  With snr=True F3 stores its spectrum even when the arrays are not stored."""
+    def _outputs(self, turn: int, plan: StepPlan):
+        """F3 / F4 (and SNR) outputs of a step: the first J rows of result turn `turn`'s Jmax-row buffers (with snr=True F3
+        stores its spectrum).  A new transform or bin count gets new buffers, and the spectrum workspace grows to fit."""
+        if (self.transform, plan.max_bins) != self._spec_key:
+            self._spec_key, self._out = (self.transform, plan.max_bins), [None] * self._nbuf
+            need = _cabi.lib().bpv_spectrum_workspace_bytes(ops.jobs_params(plan.p, self._Jmax), plan.max_bins)
+            if need > self._ws_spec.numel():
+                self._ws_spec = torch.zeros(need, dtype=torch.uint8, device=self.device)
         if self._out[turn] is None:
-            pm = ops.jobs_params(self._params(0, 1, 1), self._Jmax)
+            pm = ops.jobs_params(plan.p, self._Jmax)
             e = lambda C_: torch.empty((self._Jmax, C_), dtype=torch.float64, device=self.device)
             q = {}
             if self.snr:
@@ -646,61 +631,95 @@ class BatchedSignalProcessor:
                     q.update(gated_freq=e(self.R), gated_lag=e(self.P))
             self._out[turn] = (ops._spectrum_out(pm, self.store_arrays or self.snr, None, self.device),
                                ops._xcorr_out(pm, self.store_arrays, None, self.device), q)
-        return [{k: None if v is None else v[:J] for k, v in d.items()} for d in self._out[turn]]
+        return [{k: None if v is None else v[:plan.J] for k, v in d.items()} for d in self._out[turn]]
 
-    def _step_signals(self, samples, timestamps, S, T, _count_roi, _designed, plan=None) -> StepResult:
+    # ------------------------------------------------------------------------------------------
+    # The stages of a step, each called once in this order: each makes the lockstep / job-map choice for its own calls and
+    # adds the kernels it enqueues to plan.launches.
+    def _run(self, plan: StepPlan, samples, timestamps, designed: bool = False) -> StepResult:
+        """The window pipeline of a planned step (designed: step() pushed the timestamps and started the designs)."""
         main = torch.cuda.current_stream(self.device)
         turn = self._turn
         self._turn = (turn + 1) % self._nbuf
-        has_filter = any(m in (_cabi.FILTER_BUTTER, _cabi.FILTER_FIR) for m in self.methods)
-        lock = plan is None or plan['lock']
-        roi_launches = 1 + self._extra_launches if _count_roi else 0
-        if lock:
-            head0, head_step, jobs = self._lock_jobs(T, plan)
-            ops.ring_push(self.ring_t, self.ring_y, self._cnt, None if _designed else timestamps.contiguous(), samples.contiguous())
-            self._cnt += T
-            self._g0_ok = False
-            if jobs == 0:                       # a strided step between cadence points: F1 + push
-                return self._empty_step(samples, 0, roi_launches + 1)
-            p = self._params(head0, head_step, jobs)
-            pj, J = p, S * jobs
-        else:
-            # job-map path: stream s pushes n_s frames and owns jobs job_offsets[s]:job_offsets[s+1]; F3 / F4 see the J jobs
-            # as J streams of one job (include/bpv.h)
-            if not plan['mapped']:
-                self._map_jobs(plan, turn)
-            ops.ring_push_ragged(self.ring_t, self.ring_y, self._g0[0], self._ndev, None if _designed else timestamps.contiguous(),
-                                 samples.contiguous())
-            jobs, J = None, plan['J']
-            if J == 0:                          # a strided step between cadence points: F1 + map + push
-                self._advance(plan, turn, main)
-                return self._empty_step(samples, None, roi_launches + 2)
-            p = self._params(0, 1, 1)
-            pj = ops.jobs_params(p, J)
-            js, jh, sj0 = self._jobmap[turn]
+        self._push(plan, turn, None if designed else timestamps, samples)
+        J = plan.J
+        if J == 0:                              # a strided step between cadence points: F1 + (map +) push
+            return self._finish(plan, turn, self._empty_step(samples, plan))
         proc = self._proc[turn % len(self._proc)]
         px, py, st = proc[0, :J], proc[1, :J], self._status[turn][:J]
-        if _designed:
+        if designed:
             main.wait_event(self._ev['design'])
-        elif has_filter and lock:
-            ops.window_design(self.ring_t, p, self._ws, self._cache())
-        elif has_filter:
-            ops.window_design_jobs(self.ring_t, p, self._ws, js, jh, J, self._cache())
-        if lock:
-            ops.window_filter(self.ring_t, self.ring_y, p, self._ws, px, py, st, cache=self._dcache if has_filter else None)
+        elif plan.has_filter:
+            self._design(plan, turn)
+        self._filter(plan, turn, px, py, st)
+        spo, xco, qo = self._outputs(turn, plan)
+        sp, xc = self._spectrum_xcorr(plan, main, px, py, spo, xco)
+        snr_db, bpm_in, ptt_in = self._snr(plan, sp, xc, qo)
+        if not self.store_arrays and self.discard_scratch:
+            # the processed windows are dead now: drop their dirty L2 lines instead of letting the next step's ROI sampling
+            # push them out to DRAM (F1 64.5 -> 69.7 us with 80 MB of dirty scratch in L2, profiles/r2p_f1_dirty.txt)
+            dead = (proc,) if J == self._Jmax else (px, py)
+            ops.scratch_discard(*dead)
+            plan.launches += len(dead)
+        means = self._means(plan, turn, bpm_in, ptt_in)
+        arrays = {}
+        if self.store_arrays:
+            arrays = dict(proc_x=px, proc_y=py, freqs=sp['freqs'], mags=sp['mags'], num_bins=sp['num_bins'],
+                          lags=xc['lags'], corr=xc['corr'], num_lags=xc['num_lags'])
+        res = StepResult(plan.jobs if plan.lock else None, samples, sp['peak_freq'], sp['peak_idx'], sp['peak_mag'],
+                         xc['lag_sec'], xc['lag_idx'], xc['lag_corr'], st, arrays, means, snr_db=snr_db)
+        if not plan.lock:
+            res._job_offsets, res._job_stream = plan.off, self._jobmap[turn][0][:J]
+        return self._finish(plan, turn, res)
+
+    def _push(self, plan: StepPlan, turn: int, ts, values) -> None:
+        """Append the step's timestamps and / or samples to the rings; the job-map path builds its job map first."""
+        if not plan.lock and ts is not None:   # the first push of a step carries its timestamps
+            self._map_jobs(plan, turn)
+        ts, values = None if ts is None else ts.contiguous(), None if values is None else values.contiguous()
+        if plan.lock:
+            ops.ring_push(self.ring_t, self.ring_y, self._cnt, ts, values)
         else:
-            ops.window_filter_jobs(self.ring_t, self.ring_y, p, self._ws, js, jh, J, px, py, st,
-                                   cache=self._dcache if has_filter else None)
-        spo, xco, qo = self._outputs(turn, J)
-        p = pj
-        # (windows over 320 samples: the entry point itself runs the two stand-alone launches, on this stream)
-        fb, lb = ops.peak_band(self.freq_band, 'freq_band'), ops.peak_band(self.lag_band, 'lag_band')
+            ops.ring_push_ragged(self.ring_t, self.ring_y, self._g0[0], self._ndev, ts, values)
+        plan.launches += 1
+
+    def _design(self, plan: StepPlan, turn: int) -> None:
+        """make_filter of the step's jobs on the current stream: a kernel per filter method (+ the design cache's probe)."""
+        if plan.lock:
+            ops.window_design(self.ring_t, plan.p, self._ws, self._cache())
+        else:
+            ops.window_design_jobs(self.ring_t, plan.p, self._ws, *self._jobmap[turn][:2], plan.J, self._cache())
+        plan.launches += len({m for m in self.methods if m in (_cabi.FILTER_BUTTER, _cabi.FILTER_FIR)}) + (self._dcache is not None)
+
+    def _filter(self, plan: StepPlan, turn: int, px, py, st) -> None:
+        """F2 of the step's window jobs given their designs."""
+        cache = self._dcache if plan.has_filter else None
+        if plan.lock:
+            ops.window_filter(self.ring_t, self.ring_y, plan.p, self._ws, px, py, st, cache=cache)
+        else:
+            ops.window_filter_jobs(self.ring_t, self.ring_y, plan.p, self._ws, *self._jobmap[turn][:2], plan.J, px, py, st, cache=cache)
+        plan.launches += 1
+
+    def _spectrum(self, plan: StepPlan, px, py, out) -> dict:
+        """F3 + heart-rate peak.  bpv_window_spectrum runs two kernels for Lomb-Scargle (coarse grid + peak) and six for
+        DFT_RFFT on the tensor cores (twiddle images + seal + split + MMA + peak + the float64 kernel for flagged windows),
+        which it takes for windows of 16..2048 samples with BPV_DFT_TC=1, or by default when the methods resample."""
+        sp = ops.window_spectrum(px, py, plan.pj, store=self.store_arrays or self.snr, workspace=self._ws_spec, out=out,
+                                 band=plan.freq_band)
+        tc = self.transform == _cabi.DFT_RFFT and 16 <= self.W <= 2048 and (
+            os.environ['BPV_DFT_TC'][:1] == '1' if 'BPV_DFT_TC' in os.environ
+            else any(m in (_cabi.INTERP_LINEAR, _cabi.INTERP_CUBIC) for m in self.methods))
+        plan.launches += 2 if self.transform == _cabi.PGRAM_LS else 6 if tc else 1
+        return sp
+
+    def _spectrum_xcorr(self, plan: StepPlan, main, px, py, spo, xco):
+        """F3 and F4 on the overlap schedule: one fused grid (bit 4), the two kernels on two streams (bit 2) or serial."""
         fused = (bool(self.overlap & OVERLAP_FUSED) and self.P > 0 and self.transform == _cabi.PGRAM_WELCH
-                 and fb is None and lb is None)       # the fused grid has no band: two kernels instead
-        store_spec = self.store_arrays or self.snr
+                 and plan.freq_band is None and plan.lag_band is None)       # the fused grid has no band: two kernels instead
         if fused:
-            sp, xc = ops.window_welch_xcorr(px, py, p, store=store_spec, out_spectrum=spo, out_xcorr=xco,
-                                            store_xcorr=self.store_arrays)
+            sp, xc = ops.window_welch_xcorr(px, py, plan.pj, store=self.store_arrays or self.snr, out_spectrum=spo,
+                                            out_xcorr=xco, store_xcorr=self.store_arrays)
+            plan.launches += 1 if self.W <= 320 else 2        # above 320 samples: the two stand-alone kernels, on this stream
         elif (self.overlap & OVERLAP_XCORR) and self.P:
             # launch order matters for co-residency: the spectrum kernels' CTAs are small (Welch: 24 KB of shared memory),
             # the xcorr CTAs large (51 KB); with xcorr first its 4 CTAs fill an SM's shared memory and the spectrum only
@@ -711,86 +730,69 @@ class BatchedSignalProcessor:
             side.wait_event(ev['pre'])
             xc_first = os.environ.get('BPV_XC_FIRST', '') == '1'
             if not xc_first:
-                sp = ops.window_spectrum(px, py, p, store=store_spec, workspace=self._ws_spec, out=spo, band=fb)
+                sp = self._spectrum(plan, px, py, spo)
             with torch.cuda.stream(side):
-                xc = ops.window_xcorr(px, py, p, store=self.store_arrays, out=xco, band=lb)
+                xc = ops.window_xcorr(px, py, plan.pj, store=self.store_arrays, out=xco, band=plan.lag_band)
                 ev['xc'].record(side)
+            plan.launches += 1
             if xc_first:
-                sp = ops.window_spectrum(px, py, p, store=store_spec, workspace=self._ws_spec, out=spo, band=fb)
+                sp = self._spectrum(plan, px, py, spo)
             main.wait_event(ev['xc'])
         else:
-            sp = ops.window_spectrum(px, py, p, store=store_spec, workspace=self._ws_spec, out=spo, band=fb)
-            xc = ops.window_xcorr(px, py, p, store=self.store_arrays, out=xco, band=lb)
-        gate = self.snr and self._min_snr_db is not None and self.peak_max_samples > 0
-        if self.snr:
-            # after F3 and, on the two-stream schedule, after the xcorr event: the gate reads lag_sec
-            band = fb if fb is not None else (self.kw['min_freq'], self.kw['max_freq'])
-            qo = ops.window_snr(sp['freqs'], sp['mags'], sp['num_bins'], sp['peak_idx'], self.transform, band, self.snr_half_width,
-                                min_snr_db=self._min_snr_db if gate else None, peak_freq=sp['peak_freq'] if gate else None,
-                                lag_sec=xc['lag_sec'] if gate else None, out=qo)
-        if not self.store_arrays and self.discard_scratch:
-            # the processed windows are dead now: drop their dirty L2 lines instead of letting the next step's ROI sampling
-            # push them out to DRAM (F1 64.5 -> 69.7 us with 80 MB of dirty scratch in L2, profiles/r2p_f1_dirty.txt)
-            if J == self._Jmax:
-                ops.scratch_discard(proc)
-            else:
-                ops.scratch_discard(px, py)
-        n_design = sum(1 for m in set(self.methods) if m in (_cabi.FILTER_BUTTER, _cabi.FILTER_FIR))
-        n_pre = 1 + n_design + (1 if n_design and self._dcache is not None else 0)     # filter + designs (+ cache probe)
-        n_spec = 2 if self.transform == _cabi.PGRAM_LS else 1
-        if self.transform == _cabi.DFT_RFFT and 16 <= self.W <= 2048:
-            env = os.environ.get('BPV_DFT_TC')
-            interp = any(m in (_cabi.INTERP_LINEAR, _cabi.INTERP_CUBIC) for m in self.methods)
-            if (env[:1] == '1') if env is not None else interp:
-                n_spec = 6              # dft_image + seal + dft_split + dft_tc_tma2 + dft_peak kernels + spectrum_dense_kernel for the flagged windows
-        n_push = (2 if _designed else 1) + (0 if lock else 1)          # (+ the job map)
-        self.launches_per_step = roi_launches + n_push + n_pre + n_spec + (1 if self.P and not (fused and self.W <= 320) else 0)
-        if not self.store_arrays and self.discard_scratch:
-            self.launches_per_step += 1 if J == self._Jmax else 2
-        self.launches_per_step += 1 if self.snr else 0
-        arrays = {}
-        if self.store_arrays:
-            arrays = dict(proc_x=px, proc_y=py, freqs=sp['freqs'], mags=sp['mags'], num_bins=sp['num_bins'],
-                          lags=xc['lags'], corr=xc['corr'], num_lags=xc['num_lags'])
-        # the running means push the gated values: a rejected heart rate / PTT enters the history as NaN
-        bpm_in = qo['gated_freq'] if gate else sp['peak_freq']
-        ptt_in = qo['gated_lag'] if gate else xc['lag_sec']
-        snr_db = qo['snr_db'] if self.snr else None
+            sp = self._spectrum(plan, px, py, spo)
+            xc = ops.window_xcorr(px, py, plan.pj, store=self.store_arrays, out=xco, band=plan.lag_band)
+            plan.launches += self.P > 0                 # F4 enqueues nothing without a pair
+        return sp, xc
+
+    def _snr(self, plan: StepPlan, sp: dict, xc: dict, qo: dict):
+        """(snr_db or None, heart rates, PTTs): the values the running means push are gated by min_snr_db (rejected -> NaN)."""
+        if not self.snr:
+            return None, sp['peak_freq'], xc['lag_sec']
+        gate = self._min_snr_db is not None and self.peak_max_samples > 0
+        # after F3 and, on the two-stream schedule, after the xcorr event: the gate reads lag_sec
+        band = plan.freq_band if plan.freq_band is not None else (self.kw['min_freq'], self.kw['max_freq'])
+        g = dict(min_snr_db=self._min_snr_db, peak_freq=sp['peak_freq'], lag_sec=xc['lag_sec']) if gate else {}
+        qo = ops.window_snr(sp['freqs'], sp['mags'], sp['num_bins'], sp['peak_idx'], self.transform, band, self.snr_half_width,
+                            out=qo, **g)
+        plan.launches += 1
+        return (qo['snr_db'], qo['gated_freq'], qo['gated_lag']) if gate else (qo['snr_db'], sp['peak_freq'], xc['lag_sec'])
+
+    def _means(self, plan: StepPlan, turn: int, bpm_in, ptt_in) -> dict:
+        """Running means of the heart rates and PTTs (peak_max_samples): one push per window job into each stream's history."""
+        if not self.peak_max_samples:
+            return {}
+        cols = [('bpm', self._bpm_ring, bpm_in, 60.0)] + ([('ptt', self._ptt_ring, ptt_in, 1000.0)] if self.P else [])
         means = {}
-        if self.peak_max_samples and lock:
-            mb, mbi = ops.running_mean(self._bpm_ring, self._mcnt, bpm_in.view(S, jobs, self.R), 60.0)
-            means = dict(mean_bpm=mb.view(J, self.R), mean_bpm_int=mbi.view(J, self.R))
-            if self.P:
-                mp, mpi = ops.running_mean(self._ptt_ring, self._mcnt, ptt_in.view(S, jobs, self.P), 1000.0)
-                means.update(mean_ptt=mp.view(J, self.P), mean_ptt_int=mpi.view(J, self.P))
-            self._mcnt += jobs
-            self.launches_per_step += 2 if self.P else 1
-        elif self.peak_max_samples:
-            mcnt = np.full(self.S, self._mcnt, dtype=np.int64) if isinstance(self._mcnt, int) else self._mcnt
+        if plan.lock:
+            for name, ring, v, scale in cols:
+                m, mi = ops.running_mean(ring, self._mcnt, v.view(self.S, plan.jobs, -1), scale)
+                means[f'mean_{name}'], means[f'mean_{name}_int'] = m.view(plan.J, -1), mi.view(plan.J, -1)
+                plan.launches += 1
+            self._mcnt += plan.jobs
+        else:
+            mcnt = self.mean_counts
             pin = self._pinned(turn)
             pin['m0'].numpy()[:] = mcnt
             self._mg0.copy_(pin['m0'], non_blocking=True)
-            mb, mbi = ops.running_mean_jobs(self._bpm_ring, self._mg0, sj0, bpm_in, 60.0)
-            means = dict(mean_bpm=mb, mean_bpm_int=mbi)
-            if self.P:
-                mp, mpi = ops.running_mean_jobs(self._ptt_ring, self._mg0, sj0, ptt_in, 1000.0)
-                means.update(mean_ptt=mp, mean_ptt_int=mpi)
-            self._mcnt = self._level(mcnt + plan['jobs'])
-            self.launches_per_step += 2 if self.P else 1
-        if lock:
-            return StepResult(jobs, samples, sp['peak_freq'], sp['peak_idx'], sp['peak_mag'], xc['lag_sec'], xc['lag_idx'],
-                              xc['lag_corr'], st, arrays, means, snr_db=snr_db)
-        self._advance(plan, turn, main)
-        return StepResult(None, samples, sp['peak_freq'], sp['peak_idx'], sp['peak_mag'], xc['lag_sec'], xc['lag_idx'],
-                          xc['lag_corr'], st, arrays, means, _job_offsets=plan['off'], _job_stream=js[:J], snr_db=snr_db)
+            sj0 = self._jobmap[turn][2]
+            for name, ring, v, scale in cols:
+                means[f'mean_{name}'], means[f'mean_{name}_int'] = ops.running_mean_jobs(ring, self._mg0, sj0, v, scale)
+                plan.launches += 1
+            self._mcnt = self._level(mcnt + plan.jobs)
+        return means
 
-    def _advance(self, plan: dict, turn: int, main) -> None:
-        """End of a job-map step on the host: the staging of `turn` is in flight until the device passes this point, and
-        the counts advance by the frames taken."""
-        self._staging[turn]['ev'].record(main)
-        self._staging[turn]['used'] = True
-        self._cnt = self._level(self.counts + plan['n'])
-        self._g0.reverse()                      # bpv_stream_jobs left the advanced counts in the other buffer
+    def _finish(self, plan: StepPlan, turn: int, res: StepResult) -> StepResult:
+        """End of a step on the host: the counts advance; a job-map step's staging is in flight until the device gets here."""
+        if plan.lock:
+            self._cnt += plan.T
+            self._g0_ok = False
+        else:
+            self._staging[turn]['ev'].record(torch.cuda.current_stream(self.device))
+            self._staging[turn]['used'] = True
+            self._cnt = self._level(self.counts + plan.n)
+            self._g0.reverse()                  # bpv_stream_jobs left the advanced counts in the other buffer
+        self.launches_per_step = plan.launches
+        return res
 
     # ------------------------------------------------------------------------------------------
     # SURVEY.md §8(f) row 3: snapshot / resume of the per-stream state (the reference's deepcopy(store), :313, is the
@@ -805,10 +807,9 @@ class BatchedSignalProcessor:
         copied to the host."""
         torch.cuda.synchronize(self.device)
         cpu = lambda t: None if t is None else t.detach().to('cpu', copy=True)
-        mcnt = np.full(self.S, self._mcnt, dtype=np.int64) if isinstance(self._mcnt, int) else self._mcnt.copy()
         return dict(version=STATE_VERSION, signature=self._signature(), counts=self.counts,
                     ring_t=cpu(self.ring_t), ring_y=cpu(self.ring_y),
-                    mean_counts=mcnt, bpm_ring=cpu(self._bpm_ring), ptt_ring=cpu(self._ptt_ring),
+                    mean_counts=self.mean_counts, bpm_ring=cpu(self._bpm_ring), ptt_ring=cpu(self._ptt_ring),
                     roi_count=int(self._roi_count), roi_hist=cpu(self._roi_hist))
 
     def load_state_dict(self, state: dict) -> None:
@@ -863,10 +864,7 @@ class BatchedSignalProcessor:
         for t in (self.ring_t, self.ring_y, self._bpm_ring, self._ptt_ring, self._roi_hist):
             if t is not None:
                 t.index_fill_(0, rows, nan)
-        counts = self.counts
-        counts[idx] = 0
-        self._cnt = self._level(counts)
-        mcnt = np.full(self.S, self._mcnt, dtype=np.int64) if isinstance(self._mcnt, int) else self._mcnt.copy()
-        mcnt[idx] = 0
-        self._mcnt = self._level(mcnt)
+        counts, mcnt = self.counts, self.mean_counts
+        counts[idx] = mcnt[idx] = 0
+        self._cnt, self._mcnt = self._level(counts), self._level(mcnt)
         self._g0_ok = False

@@ -5,8 +5,12 @@
 #include "common.cuh"
 
 namespace bpv {
+// RAGGED (bpv_ring_push_ragged): stream s appends its first n[s] rows at global indices g0s[s] ...; the other rows of its T are
+// not read.  The ragged parameters follow the lockstep ones, so the lockstep instantiation keeps its parameter layout.
+template <bool RAGGED>
 __global__ void ring_push_kernel(double* __restrict__ ring_t, double* __restrict__ ring_y, int S, int R, int cap,
-                                 long long g0, int T, const double* __restrict__ ts, const double* __restrict__ values) {
+                                 long long g0, int T, const double* __restrict__ ts, const double* __restrict__ values,
+                                 const int64_t* __restrict__ g0s, const int32_t* __restrict__ n) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;  // over S*T*(R+1)
   const long long total = (long long)S * T * (R + 1);
   if (i >= total) return;
@@ -14,7 +18,8 @@ __global__ void ring_push_kernel(double* __restrict__ ring_t, double* __restrict
   const long long st = i / (R + 1);
   const int t = (int)(st % T);
   const long long s = st / T;
-  const int slot = (int)((g0 + t) % cap);
+  if (RAGGED && t >= n[s]) return;
+  const int slot = (int)(((RAGGED ? g0s[s] : g0) + t) % cap);
   if (c == R) { if (ts) ring_t[s * cap + slot] = ts[s * T + t]; }
   else if (values) ring_y[(s * R + c) * cap + slot] = values[(s * T + t) * R + c];
 }
@@ -26,28 +31,12 @@ extern "C" int bpv_ring_push(double* ring_t, double* ring_y, int32_t S, int32_t 
   BPV_REQUIRE(ring_t && ring_y && (ts || values), BPV_E_INVALID, "bpv_ring_push: NULL pointer");
   BPV_REQUIRE(S > 0 && R > 0 && cap > 0 && T > 0 && T <= cap && g0 >= 0, BPV_E_INVALID, "bpv_ring_push: bad sizes");
   const long long total = (long long)S * T * (R + 1);
-  ring_push_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ring_t, ring_y, S, R, cap, g0, T, ts, values);
+  ring_push_kernel<false><<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ring_t, ring_y, S, R, cap, g0, T, ts, values,
+                                                                                            nullptr, nullptr);
   return check_launch("bpv_ring_push");
 }
 
-// Ragged push: stream s appends its first n[s] rows at global indices g0[s] ...; the other rows of its T are not read.
 namespace bpv {
-__global__ void ring_push_ragged_kernel(double* __restrict__ ring_t, double* __restrict__ ring_y, int S, int R, int cap,
-                                        const int64_t* __restrict__ g0, const int32_t* __restrict__ n, int T,
-                                        const double* __restrict__ ts, const double* __restrict__ values) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;  // over S*T*(R+1)
-  const long long total = (long long)S * T * (R + 1);
-  if (i >= total) return;
-  const int c = (int)(i % (R + 1));
-  const long long st = i / (R + 1);
-  const int t = (int)(st % T);
-  const long long s = st / T;
-  if (t >= n[s]) return;
-  const int slot = (int)((g0[s] + t) % cap);
-  if (c == R) { if (ts) ring_t[s * cap + slot] = ts[s * T + t]; }
-  else if (values) ring_y[(s * R + c) * cap + slot] = values[(s * T + t) * R + c];
-}
-
 // Job map of a ragged step: CTA b owns streams [1024 b, 1024 b + 1024), one per thread.  Every CTA sums the job counts of
 // ALL streams (coalesced, L2-resident after the first CTA: 256 KB at S = 65 536) to get its chunk's first job and the total,
 // so one launch needs no inter-CTA scratch; a warp-shuffle block scan places the chunk's streams.  The map entries are then
@@ -161,8 +150,8 @@ extern "C" int bpv_ring_push_ragged(double* ring_t, double* ring_y, int32_t S, i
   BPV_REQUIRE(ring_t && ring_y && g0 && n && (ts || values), BPV_E_INVALID, "bpv_ring_push_ragged: NULL pointer");
   BPV_REQUIRE(S > 0 && R > 0 && cap > 0 && T > 0 && T <= cap, BPV_E_INVALID, "bpv_ring_push_ragged: bad sizes");
   const long long total = (long long)S * T * (R + 1);
-  ring_push_ragged_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ring_t, ring_y, S, R, cap, g0, n, T,
-                                                                                          ts, values);
+  ring_push_kernel<true><<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ring_t, ring_y, S, R, cap, 0, T, ts, values,
+                                                                                           g0, n);
   return check_launch("bpv_ring_push_ragged");
 }
 
@@ -224,6 +213,26 @@ __device__ inline double np_sum_small(const double* a, int n) {   // numpy pairw
 
 constexpr int MAX_MEAN_HIST = 128;
 
+// Push v into the history rg [H] at slot `newest` and write the nanmean over the history, oldest slot first (deque order;
+// NaN -> 0 as np.nanmean does), and its rounded value to element e of mean / mean_int.
+__device__ __forceinline__ void push_nanmean(double* __restrict__ rg, int H, int newest, double v, long long e,
+                                             double* __restrict__ mean, double* __restrict__ mean_int) {
+  double tmp[MAX_MEAN_HIST];
+  rg[newest] = v;
+  int cnt = 0;
+  for (int h = 0; h < H; ++h) {
+    int slot = newest + 1 + h; if (slot >= H) slot -= H;
+    const double x = rg[slot];
+    const bool ok = isfinite(x);
+    tmp[h] = ok ? x : 0.0;
+    cnt += ok;
+  }
+  double m = nan_f64();
+  if (cnt) m = np_sum_small(tmp, H) / (double)cnt;
+  if (mean) mean[e] = m;
+  if (mean_int) mean_int[e] = cnt ? rint(m) : nan_f64();
+}
+
 __global__ void running_mean_kernel(double* __restrict__ ring, int S, int C, int H, long long g0, int T,
                                     const double* __restrict__ values, double scale,
                                     double* __restrict__ mean, double* __restrict__ mean_int) {
@@ -231,24 +240,10 @@ __global__ void running_mean_kernel(double* __restrict__ ring, int S, int C, int
   if (idx >= S * C) return;
   const int s = idx / C, c = idx % C;
   double* rg = ring + (long long)idx * H;
-  double tmp[MAX_MEAN_HIST];
   for (int t = 0; t < T; ++t) {
     const long long e = ((long long)s * T + t) * C + c;
-    rg[(int)((g0 + t) % H)] = values[e] * scale;             // f * 60 / t * 1000 (signal_processor.py:310, 312)
-    // chronological order: oldest slot first (deque order), NaN -> 0 as np.nanmean does
-    const int newest = (int)((g0 + t) % H);
-    int cnt = 0;
-    for (int h = 0; h < H; ++h) {
-      int slot = newest + 1 + h; if (slot >= H) slot -= H;
-      const double v = rg[slot];
-      const bool ok = isfinite(v);
-      tmp[h] = ok ? v : 0.0;
-      cnt += ok;
-    }
-    double m = nan_f64();
-    if (cnt) m = np_sum_small(tmp, H) / (double)cnt;
-    if (mean) mean[e] = m;
-    if (mean_int) mean_int[e] = cnt ? rint(m) : nan_f64();
+    const double v = values[e] * scale;                        // f * 60 / t * 1000 (signal_processor.py:310, 312)
+    push_nanmean(rg, H, (int)((g0 + t) % H), v, e, mean, mean_int);
   }
 }
 }  // namespace bpv
@@ -273,25 +268,11 @@ __global__ void running_mean_jobs_kernel(double* __restrict__ ring, int S, int C
   if (idx >= S * C) return;
   const int s = idx / C, c = idx % C;
   double* rg = ring + (long long)idx * H;
-  double tmp[MAX_MEAN_HIST];
   const long long gs = g0[s];
   const int j0 = stream_job0[s], j1 = stream_job0[s + 1];
   for (int j = j0; j < j1; ++j) {
     const long long e = (long long)j * C + c;
-    const int newest = (int)((gs + (j - j0)) % H);
-    rg[newest] = values[e] * scale;
-    int cnt = 0;
-    for (int h = 0; h < H; ++h) {
-      int slot = newest + 1 + h; if (slot >= H) slot -= H;
-      const double v = rg[slot];
-      const bool ok = isfinite(v);
-      tmp[h] = ok ? v : 0.0;
-      cnt += ok;
-    }
-    double m = nan_f64();
-    if (cnt) m = np_sum_small(tmp, H) / (double)cnt;
-    if (mean) mean[e] = m;
-    if (mean_int) mean_int[e] = cnt ? rint(m) : nan_f64();
+    push_nanmean(rg, H, (int)((gs + (j - j0)) % H), values[e] * scale, e, mean, mean_int);
   }
 }
 }  // namespace bpv

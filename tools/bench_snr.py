@@ -99,7 +99,7 @@ def run_shape(name, wl, rounds, iters, reps):
     out['snr_kernel_us'] = round(timed(lambda: ops.window_snr(f, m, nb, r.peak_idx, eng.transform, band), reps), 2)
     out['snr_gated_kernel_us'] = round(timed(lambda: ops.window_snr(f, m, nb, r.peak_idx, eng.transform, band, min_snr_db=3.0,
                                                                     peak_freq=r.peak_freq, lag_sec=r.lag_sec), reps), 2)
-    out['spectrum_bytes_read_by_snr'] = int(2 * 4 * J * eng.R * eng._mb)
+    out['spectrum_bytes_read_by_snr'] = int(2 * 4 * f.numel())
     proc = eng._proc[0]
     px, py = proc[0, :J], proc[1, :J]
     p = ops.jobs_params(eng._params(0, 1, 1), J)
