@@ -48,7 +48,6 @@ _SIGS = {
     'bpv_view_boxes': (C.c_int, [_P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
     'bpv_pack_records': (C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_int32, C.c_int32, _P, _P]),
     'bpv_pack_records32': (C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_int32, C.c_int32, _P, _P]),
-    'bpv_scratch_discard': (C.c_int, [_P, C.c_int64, _P]),
     'bpv_dft256_tc': (C.c_int, [_P, C.c_int32, _P, _P]),
     'bpv_ring_push': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int32, _P, _P, _P]),
     'bpv_ring_push_ragged': (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P, C.c_int32, _P, _P, _P]),

@@ -18,7 +18,7 @@ NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
 FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
          '-Xcompiler', '-fPIC', '--use_fast_math', '-Xptxas', '-v']
 # --use_fast_math only affects fp32 intrinsics choices; every fp64 path is IEEE.
-# BPV_NVCC_EXTRA (e.g. "-DBPV_ROI_TUNING" for tools/roi_variants.sh) is appended for development builds.
+# BPV_NVCC_EXTRA (extra nvcc flags, e.g. "-Xptxas -warn-spills") is appended for development builds.
 FLAGS += os.environ.get('BPV_NVCC_EXTRA', '').split()
 
 

@@ -298,9 +298,6 @@ class BatchedSignalProcessor:
             design_cache = os.environ.get('BPV_DESIGN_CACHE', '1') != '0'
         self._dcache = ops.new_design_cache(dev) if design_cache else None
         self._dcache_sig = None
-        # measured (profiles/r2q_discard_depth_ab.txt): at 8192 jobs per step the discard saves 2.2 us of F1 and costs 4 us itself; at
-        # 16 384 jobs the scratch (157 MB) no longer fits L2 and has been written back before F1 starts -> off by default
-        self.discard_scratch = os.environ.get('BPV_DISCARD', '0') == '1'
         self._side = None
         self._side_hi = None
         self._ev = None
@@ -327,12 +324,9 @@ class BatchedSignalProcessor:
         if self._side is None:
             with torch.cuda.device(self.device):
                 self._side = torch.cuda.Stream(device=self.device)
-                # BPV_DESIGN_PRIO=1 puts the design probe (512 CTAs, F2 waits for it) on a high-priority stream: its CTAs are then
-                # placed as soon as F1's retire instead of behind the 32 768 F1 CTAs already queued.  Measured (profiles/r4b): the
-                # probe finishes 90 us earlier, the step gains 2 us (0.7011 -> 0.6990 ms) and F1 loses 2.4 us to the probe's CTAs
-                # (0.722 -> 0.708 of the HBM peak by the events around it) -> off by default
-                prio = -1 if os.environ.get('BPV_DESIGN_PRIO', '0') == '1' else 0
-                self._side_hi = torch.cuda.Stream(device=self.device, priority=prio)
+                # the design-ahead stream, at default priority: a high-priority one was measured to cost F1 more than it
+                # gains the step (profiles/r4b)
+                self._side_hi = torch.cuda.Stream(device=self.device)
                 self._ev = {k: torch.cuda.Event() for k in ('ts', 'design', 'pre', 'xc')}
         return self._side, self._ev
 
@@ -655,12 +649,6 @@ class BatchedSignalProcessor:
         spo, xco, qo = self._outputs(turn, plan)
         sp, xc = self._spectrum_xcorr(plan, main, px, py, spo, xco)
         snr_db, bpm_in, ptt_in = self._snr(plan, sp, xc, qo)
-        if not self.store_arrays and self.discard_scratch:
-            # the processed windows are dead now: drop their dirty L2 lines instead of letting the next step's ROI sampling
-            # push them out to DRAM (F1 64.5 -> 69.7 us with 80 MB of dirty scratch in L2, profiles/r2p_f1_dirty.txt)
-            dead = (proc,) if J == self._Jmax else (px, py)
-            ops.scratch_discard(*dead)
-            plan.launches += len(dead)
         means = self._means(plan, turn, bpm_in, ptt_in)
         arrays = {}
         if self.store_arrays:
@@ -724,19 +712,15 @@ class BatchedSignalProcessor:
             # launch order matters for co-residency: the spectrum kernels' CTAs are small (Welch: 24 KB of shared memory),
             # the xcorr CTAs large (51 KB); with xcorr first its 4 CTAs fill an SM's shared memory and the spectrum only
             # gets in as they retire (168 us for the pair against 103 + 75 serial); spectrum first leaves room for two xcorr
-            # CTAs beside five Welch CTAs.  BPV_XC_FIRST=1 restores the other order (measurement switch).
+            # CTAs beside five Welch CTAs.
             side, ev = self._streams()
             ev['pre'].record(main)
             side.wait_event(ev['pre'])
-            xc_first = os.environ.get('BPV_XC_FIRST', '') == '1'
-            if not xc_first:
-                sp = self._spectrum(plan, px, py, spo)
+            sp = self._spectrum(plan, px, py, spo)
             with torch.cuda.stream(side):
                 xc = ops.window_xcorr(px, py, plan.pj, store=self.store_arrays, out=xco, band=plan.lag_band)
                 ev['xc'].record(side)
             plan.launches += 1
-            if xc_first:
-                sp = self._spectrum(plan, px, py, spo)
             main.wait_event(ev['xc'])
         else:
             sp = self._spectrum(plan, px, py, spo)

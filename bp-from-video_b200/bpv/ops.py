@@ -490,14 +490,6 @@ def pack_records32(peak_freq, lag_sec, peak_idx, lag_idx, out=None):
     return out
 
 
-def scratch_discard(*tensors) -> None:
-    """Drop the L2 lines of dead scratch tensors without writing them back to DRAM (include/bpv.h bpv_scratch_discard).
-    Their contents are undefined afterwards."""
-    for t in tensors:
-        _require(t.is_cuda and t.is_contiguous(), 'scratch_discard: contiguous CUDA tensors only')
-        _run(t.device, 'bpv_scratch_discard', ptr(t), t.numel() * t.element_size())
-
-
 def unpack_records32(rec: torch.Tensor, R: int, P: int):
     """(bpm f32 [J,R], ptt_ms f32 [J,P], peak_idx i32 [J,R], lag_idx i32 [J,P]) views of a packed int32 record tensor."""
     f = rec.view(torch.float32)

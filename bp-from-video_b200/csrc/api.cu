@@ -53,31 +53,6 @@ extern "C" int bpv_get_l2_fetch_granularity(void) {
 }
 
 
-// ---- L2 discard of dead scratch (engine: proc_x / proc_y after F3 and F4 have consumed them) ----
-// The processed windows are scratch between F2 and F3 / F4 (~80 MB per 8192-job step, rewritten every step).  Left dirty in
-// L2 they are written back to DRAM while the next step's ROI sampling streams its frames through the cache: measured 64.5 us
-// -> 69.7 us for the 8192-frame F1 launch with 80 MB of dirty lines in L2 (profiles/r2p_f1_dirty.txt).  discard.global.L2
-// drops the lines without the write-back; their contents are undefined afterwards, which is exactly what scratch is.
-namespace bpv {
-__global__ void __launch_bounds__(256) l2_discard_kernel(uint8_t* base, long long lines) {
-  const long long i = (long long)blockIdx.x * 256 + threadIdx.x;
-  if (i < lines) asm volatile("discard.global.L2 [%0], 128;" :: "l"(base + i * 128) : "memory");
-}
-}  // namespace bpv
-
-extern "C" int bpv_scratch_discard(void* ptr, int64_t bytes, void* stream) {
-  using namespace bpv;
-  BPV_REQUIRE(ptr || bytes == 0, BPV_E_INVALID, "bpv_scratch_discard: NULL ptr");
-  BPV_REQUIRE(bytes >= 0, BPV_E_INVALID, "bpv_scratch_discard: negative size");
-  // only the 128-byte lines that lie entirely inside [ptr, ptr + bytes)
-  const uintptr_t lo = ((uintptr_t)ptr + 127) & ~(uintptr_t)127, hi = ((uintptr_t)ptr + (uintptr_t)bytes) & ~(uintptr_t)127;
-  if (hi <= lo) return 0;
-  const long long lines = (long long)((hi - lo) >> 7);
-  l2_discard_kernel<<<(unsigned)((lines + 255) / 256), 256, 0, (cudaStream_t)stream>>>((uint8_t*)lo, lines);
-  return check_launch("bpv_scratch_discard");
-}
-
-
 // ---- FMA throughput probe (bench.py: measured FP64 / FP32 peaks for the roofline of the filter / spectrum families) ----
 namespace bpv {
 template <typename T>

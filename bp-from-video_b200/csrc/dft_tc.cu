@@ -20,7 +20,6 @@
 // visible to the tensor core with fence.proxy.async; one thread issues the MMAs; tcgen05.commit -> mbarrier tells the
 // CTA when the chunk buffers may be overwritten and when the accumulator is complete; tcgen05.ld (32 lanes x 32 columns
 // per warp) brings each row's spectrum back to the thread that owns that segment.
-#include <stdlib.h>
 #include "common.cuh"
 
 namespace bpv {
@@ -882,7 +881,7 @@ long long dft_tc_split_bytes(int W, long long nsig) { return dtc_split_bytes(W, 
 long long dft_tc_image_bytes(int W) { return dtc_image_bytes(W); }
 
 // image_ws: caller-owned, persistent device memory of dft_tc_image_bytes(W) bytes (zero-initialised once) for the TMA-fed
-// kernel, or NULL for the kernel that generates its operands itself.  BPV_DFT_TMA=0 forces the latter (measurement switch).
+// kernel, or NULL for the kernel that generates its operands itself.
 int launch_dft_tc(const double* proc_x, const double* proc_y, int W, long long nsig, int max_bins, float* spec_f, float* mags,
                   int32_t* num_bins, int32_t* peak_idx, double* peak_freq, double* peak_mag, void* image_ws, void* split_ws,
                   bool banded, PeakBand band, cudaStream_t st) {
@@ -890,13 +889,12 @@ int launch_dft_tc(const double* proc_x, const double* proc_y, int W, long long n
   if (int rc = ensure_dyn_smem(banded ? (const void*)dft_peak_kernel<true> : (const void*)dft_peak_kernel<false>, smem_p)) return rc;
   const int F = W / 2 + 1;
   dim3 grid((unsigned)((nsig + TC_M - 1) / TC_M), (unsigned)((F + 127) / 128));
-  const char* env = getenv("BPV_DFT_TMA");
-  if (image_ws && !(env && env[0] == '0')) {
+  if (image_ws) {
     if (int rc = ensure_dyn_smem((const void*)dft_tc_tma_kernel, DTM_SMEM)) return rc;
     const int NB = (W + DTC_KB - 1) / DTC_KB;
     // bins per CTA: one CTA per SM (209 KB of shared memory), so the launch costs waves x (MMA time ~ 2 BC columns + the
     // per-block operand conversion, ~64 columns' worth).  2048 signals x 601 bins: 16 x 5 CTAs of 128 bins leave 68 SMs idle,
-    // 16 x 9 CTAs of 72 bins fill 144 of the 148 (BPV_DFT_BC overrides: measurement switch).
+    // 16 x 9 CTAs of 72 bins fill 144 of the 148.
     static int sms = 0;
     if (sms == 0) {
       int dev = 0;
@@ -911,16 +909,13 @@ int launch_dft_tc(const double* proc_x, const double* proc_y, int W, long long n
         const long long cost = ((ctas + sms - 1) / sms) * (2 * bc + 64);
         if (best < 0 || cost < best || (cost == best && bc > BC)) { best = cost; BC = bc; }
       }
-      const char* ebc = getenv("BPV_DFT_BC");
-      if (ebc && atoi(ebc) >= 16 && atoi(ebc) <= 128 && atoi(ebc) % 8 == 0) BC = atoi(ebc);
     }
     grid.y = (unsigned)((F + BC - 1) / BC);
     dft_image_kernel<<<dim3((unsigned)NB, grid.y), 256, 0, st>>>(W, BC, (unsigned char*)image_ws);
     if (int rc = check_launch("dft_image_kernel")) return rc;
     dft_image_seal_kernel<<<1, 1, 0, st>>>(W, BC, (unsigned char*)image_ws);
     if (int rc = check_launch("dft_image_seal_kernel")) return rc;
-    const char* esp = getenv("BPV_DFT_SPLIT");               // BPV_DFT_SPLIT=0: convert the samples inside the kernel (measurement switch)
-    if (split_ws && !(esp && esp[0] == '0')) {
+    if (split_ws) {
       if (int rc = ensure_dyn_smem((const void*)dft_tc_tma2_kernel, DT2_SMEM)) return rc;
       const long long mt = (nsig + TC_M - 1) / TC_M, rows = mt * TC_M;
       unsigned char* a_img = (unsigned char*)split_ws;

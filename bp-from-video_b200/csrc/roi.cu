@@ -7,7 +7,6 @@
 // bytes whose channel phase depends on its offset from the row's first pixel; the three channel
 // sums come from 12 dp4a against constant 0/1 byte selectors and are rotated by the phase.
 // Head/tail vectors are byte-masked.  Integer partials are reduced with warp shuffles (uint64).
-#include <stdlib.h>
 #include "common.cuh"
 
 namespace bpv {
@@ -32,22 +31,19 @@ __device__ __forceinline__ void py_slice(int a, int b, int L, int& s, int& e) {
   s = (int)aa; e = (int)bb;
 }
 
-template <int MODE>
-__device__ __forceinline__ uint4 ld_v4(const void* p) {
-  uint4 v;
-  if (MODE == 0) asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-  else if (MODE == 1) asm volatile("ld.global.nc.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-  else if (MODE == 2) asm volatile("ld.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-  else if (MODE == 3) asm volatile("ld.global.cg.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-  else if (MODE == 4) asm volatile("ld.global.cs.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-  else asm volatile("ld.global.nc.L1::no_allocate.L2::64B.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-  return v;
-}
-
 __device__ __forceinline__ uint4 ld_stream_v4(const void* p) {
   uint4 v;
   asm volatile("ld.global.nc.L1::no_allocate.L2::64B.v4.u32 {%0,%1,%2,%3}, [%4];"
                : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
+  return v;
+}
+
+// HOST: frames in pinned host memory, read with plain ld.global (see launch_rows); else ld_stream_v4
+template <bool HOST>
+__device__ __forceinline__ uint4 ld_row_v4(const void* p) {
+  if (!HOST) return ld_stream_v4(p);
+  uint4 v;
+  asm volatile("ld.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
   return v;
 }
 
@@ -176,8 +172,9 @@ __device__ __forceinline__ uint32_t sel_word(int q, int j) {  // selector q, wor
   return k == 0 ? 0x01000001u : (k == 1 ? 0x00010000u : 0x00000100u);
 }
 
-template <int GROUP, int UNROLL, bool WANT_SUMS, int LDMODE, int MINB>
-__global__ void __launch_bounds__(256, MINB) roi_rows_kernel(const RoiArgs a) {
+template <int GROUP, bool WANT_SUMS, bool HOST>
+__global__ void __launch_bounds__(256, 4) roi_rows_kernel(const RoiArgs a) {
+  constexpr int UNROLL = 4;
   constexpr int GROUPS_PER_BLOCK = 256 / GROUP;
   constexpr int WARPS_PER_GROUP = GROUP / 32;
   const int grp = threadIdx.x / GROUP, gt = threadIdx.x % GROUP;
@@ -226,7 +223,7 @@ __global__ void __launch_bounds__(256, MINB) roi_rows_kernel(const RoiArgs a) {
         uint4 d[UNROLL];
 #pragma unroll
         for (int u = 0; u < UNROLL; ++u)
-          if (r + u * rps < nrows) d[u] = ld_v4<LDMODE>(p + u * step);
+          if (r + u * rps < nrows) d[u] = ld_row_v4<HOST>(p + u * step);
 #pragma unroll
         for (int u = 0; u < UNROLL; ++u) {
           if (r + u * rps < nrows) {
@@ -282,10 +279,8 @@ __global__ void __launch_bounds__(256, MINB) roi_rows_kernel(const RoiArgs a) {
 // Shared-memory staged fast path: one ROI per CTA.  The register path above can keep at most
 // UNROLL x 16 B per thread in flight (64 KB per SM at 4 CTAs); staging decouples the bytes in flight
 // from the register file, so a CTA has its whole ROI tile (or a K-row-step batch of it) outstanding.
-//   STAGE 1: every thread issues up to K 16-byte cp.async (LDGSTS, L2::64B fill) into its OWN slots
-//            and reads the same slots back -> no CTA barrier at all, only cp.async.wait_all.
-//   STAGE 2: warp 0 issues one cp.async.bulk (TMA 1-D) per ROI row (16-byte aligned span) against
-//            an mbarrier; the CTA then reduces the tile from shared memory.
+// Every thread issues up to K 16-byte cp.async (LDGSTS, L2::64B fill) into its OWN slots and reads
+// the same slots back -> no CTA barrier at all, only cp.async.wait_all.
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -308,10 +303,9 @@ __device__ __forceinline__ uint4 lds128(uint32_t addr) {
   return v;
 }
 
-template <int THREADS, int K, bool WANT_SUMS, int STAGE>
-__global__ void __launch_bounds__(THREADS) roi_staged_kernel(const RoiArgs a, const int stage_bytes) {
+template <int THREADS, int K, bool WANT_SUMS>
+__global__ void __launch_bounds__(THREADS) roi_staged_kernel(const RoiArgs a) {
   extern __shared__ __align__(128) uint8_t stage[];
-  __shared__ __align__(8) unsigned long long bar;
   constexpr int WARPS = THREADS / 32;
   const int gt = threadIdx.x;
   const long long roi = blockIdx.x;
@@ -338,100 +332,40 @@ __global__ void __launch_bounds__(THREADS) roi_staged_kernel(const RoiArgs a, co
     int rps, r0, v0;
     if (vpr >= THREADS) { rps = 1; r0 = 0; v0 = gt; }
     else { rps = THREADS / vpr; r0 = gt / vpr; v0 = gt - r0 * vpr; if (r0 >= rps) v0 = vpr; }
-    const uint32_t sbase = smem_u32(stage);
-    if (STAGE == 1) {
-      const long long step = (long long)rps * a.row_stride;
-      const uint32_t slot0 = sbase + 16u * (uint32_t)gt;
-      const unsigned long long pol = l2_evict_first_policy();
-      for (int v = v0; v < vpr; v += THREADS) {
-        const int rel = 16 * v - off;
-        const int lo = rel < 0 ? -rel : 0;
-        const int e = row_bytes - rel;
-        const int hi = e < 16 ? e : 16;
-        const int ph = (rel + 15) % 3;
-        uint32_t cT[4], cG[4], cB[4];
+    const long long step = (long long)rps * a.row_stride;
+    const uint32_t slot0 = smem_u32(stage) + 16u * (uint32_t)gt;
+    const unsigned long long pol = l2_evict_first_policy();
+    for (int v = v0; v < vpr; v += THREADS) {
+      const int rel = 16 * v - off;
+      const int lo = rel < 0 ? -rel : 0;
+      const int e = row_bytes - rel;
+      const int hi = e < 16 ? e : 16;
+      const int ph = (rel + 15) % 3;
+      uint32_t cT[4], cG[4], cB[4];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const uint32_t m = byte_mask(lo - 4 * j, hi - 4 * j);
-          cT[j] = m & 0x01010101u;
-          cG[j] = m & sel_word((ph + 2) % 3, j);
-          cB[j] = m & sel_word(ph, j);
-        }
-        const uint8_t* p = reinterpret_cast<const uint8_t*>(base - off) + (long long)r0 * a.row_stride + 16 * v;
-        for (int r = r0; r < nrows; r += rps * K) {
-#pragma unroll
-          for (int u = 0; u < K; ++u)
-            if (r + u * rps < nrows) cp_async16_64B(slot0 + (uint32_t)(u * THREADS * 16), p + u * step, pol);
-          cp_async_wait_all();
-#pragma unroll
-          for (int u = 0; u < K; ++u) {
-            if (r + u * rps < nrows) {
-              const uint4 d = lds128(slot0 + (uint32_t)(u * THREADS * 16));
-              sT = __dp4a(d.x, cT[0], __dp4a(d.y, cT[1], __dp4a(d.z, cT[2], __dp4a(d.w, cT[3], sT))));
-              sG = __dp4a(d.x, cG[0], __dp4a(d.y, cG[1], __dp4a(d.z, cG[2], __dp4a(d.w, cG[3], sG))));
-              if (WANT_SUMS)
-                sB = __dp4a(d.x, cB[0], __dp4a(d.y, cB[1], __dp4a(d.z, cB[2], __dp4a(d.w, cB[3], sB))));
-            }
-          }
-          p += K * step;
-        }
+      for (int j = 0; j < 4; ++j) {
+        const uint32_t m = byte_mask(lo - 4 * j, hi - 4 * j);
+        cT[j] = m & 0x01010101u;
+        cG[j] = m & sel_word((ph + 2) % 3, j);
+        cB[j] = m & sel_word(ph, j);
       }
-    } else {
-      const uint32_t bar_a = smem_u32(&bar);
-      if (gt == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(bar_a) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-      }
-      __syncthreads();
-      const uint32_t rowb = 16u * (uint32_t)vpr;
-      int chunk = stage_bytes / (int)rowb;
-      if (chunk < 1) chunk = 1;  // host sizes the stage for at least one full-width row
-      uint32_t phase = 0;
-      const uint8_t* g0 = reinterpret_cast<const uint8_t*>(base - off);
-      for (int c0 = 0; c0 < nrows; c0 += chunk) {
-        const int rows = nrows - c0 < chunk ? nrows - c0 : chunk;
-        if (gt < 32) {
-          if (gt == 0)
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(bar_a), "r"(rowb * (uint32_t)rows) : "memory");
-          __syncwarp();
-          for (int r = gt; r < rows; r += 32)
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         :: "r"(sbase + (uint32_t)r * rowb), "l"(g0 + (long long)(c0 + r) * a.row_stride), "r"(rowb), "r"(bar_a) : "memory");
-        }
-        {
-          uint32_t done = 0;
-          while (!done)
-            asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
-                         : "=r"(done) : "r"(bar_a), "r"(phase) : "memory");
-          phase ^= 1;
-        }
-        for (int v = v0; v < vpr; v += THREADS) {
-          const int rel = 16 * v - off;
-          const int lo = rel < 0 ? -rel : 0;
-          const int e = row_bytes - rel;
-          const int hi = e < 16 ? e : 16;
-          const int ph = (rel + 15) % 3;
-          uint32_t cT[4], cG[4], cB[4];
+      const uint8_t* p = reinterpret_cast<const uint8_t*>(base - off) + (long long)r0 * a.row_stride + 16 * v;
+      for (int r = r0; r < nrows; r += rps * K) {
 #pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const uint32_t m = byte_mask(lo - 4 * j, hi - 4 * j);
-            cT[j] = m & 0x01010101u;
-            cG[j] = m & sel_word((ph + 2) % 3, j);
-            cB[j] = m & sel_word(ph, j);
-          }
-          uint32_t sp = sbase + (uint32_t)r0 * rowb + 16u * (uint32_t)v;
-          const uint32_t sstep = (uint32_t)rps * rowb;
-#pragma unroll 4
-          for (int r = r0; r < rows; r += rps) {
-            const uint4 d = lds128(sp);
-            sp += sstep;
+        for (int u = 0; u < K; ++u)
+          if (r + u * rps < nrows) cp_async16_64B(slot0 + (uint32_t)(u * THREADS * 16), p + u * step, pol);
+        cp_async_wait_all();
+#pragma unroll
+        for (int u = 0; u < K; ++u) {
+          if (r + u * rps < nrows) {
+            const uint4 d = lds128(slot0 + (uint32_t)(u * THREADS * 16));
             sT = __dp4a(d.x, cT[0], __dp4a(d.y, cT[1], __dp4a(d.z, cT[2], __dp4a(d.w, cT[3], sT))));
             sG = __dp4a(d.x, cG[0], __dp4a(d.y, cG[1], __dp4a(d.z, cG[2], __dp4a(d.w, cG[3], sG))));
             if (WANT_SUMS)
               sB = __dp4a(d.x, cB[0], __dp4a(d.y, cB[1], __dp4a(d.z, cB[2], __dp4a(d.w, cB[3], sB))));
           }
         }
-        if (c0 + chunk < nrows) __syncthreads();  // tile consumed before the next chunk overwrites it
+        p += K * step;
       }
     }
   }
@@ -469,303 +403,38 @@ __global__ void __launch_bounds__(THREADS) roi_staged_kernel(const RoiArgs a, co
   }
 }
 
-#ifdef BPV_ROI_TUNING
-// ---------------------------------------------------------------------------------------------
-// Persistent, double-buffered variant of the staged path (tuning builds only: -DBPV_ROI_TUNING, BPV_ROI_PIPELINED=1).
-// MEASURED AND REJECTED on the config-2 boxes: 77.8 us per 8192 frames against 64.5 us for the one-ROI-per-CTA kernel
-// (profiles/r2d_roi_ab.txt) — 128 registers and 49 KB per CTA leave 4 CTAs per SM where the simple kernel runs 9.  The one-ROI-per-CTA kernel above has its loads in flight for
-// only part of a CTA's life (launch, the dependent box load, address set-up, the reduction and the exit carry none), and
-// a 16 384-CTA grid on 148 x 9 slots ends in a partial wave.  Here a CTA lives for the whole launch and claims ROIs from a
-// global counter (perfect balance, no tail); it owns TWO stages of K slots per thread, and issues the cp.async of its
-// next ROI before it waits for the current one, so every CTA always has one whole ROI tile in flight and usually two.
-// ROIs that do not fit one stage (wider than THREADS vectors, or more than K row steps) are processed in place, round by
-// round, as the kernel above does.  work[0] = next ROI, work[1] = CTAs done; the last CTA out resets both.
-// ---------------------------------------------------------------------------------------------
-struct PTile {
-  long long roi;
-  uintptr_t p0;                 // address of this thread's first vector
-  long long step;               // bytes between its row steps
-  int nrows, row_bytes, ncols, nslots;
-  bool has_box, simple;
-  uint32_t cT[4], cG[4], cB[4];
-};
-
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
 template <int THREADS, int K>
-__device__ __forceinline__ void ptile_setup(PTile& t, const RoiArgs& a, long long roi, int gt) {
-  t.roi = roi;
-  int xs = 0, xe = 0, ys = 0, ye = 0;
-  const int4 b = __ldg(reinterpret_cast<const int4*>(a.boxes) + roi);
-  t.has_box = b.x != BPV_NO_BOX;
-  uintptr_t base = 0;
-  if (t.has_box) {
-    py_slice(b.x, b.z, a.W, xs, xe);
-    py_slice(b.y, b.w, a.H, ys, ye);
-    const long long f = roi / a.R;
-    const uint8_t* fp = a.frame_ptrs ? a.frame_ptrs[f] : a.frames + f * a.frame_stride;
-    base = reinterpret_cast<uintptr_t>(fp) + (uintptr_t)((long long)ys * a.row_stride + (long long)xs * 3);
-  }
-  t.nrows = ye - ys; t.ncols = xe - xs; t.row_bytes = (xe - xs) * 3;
-  t.nslots = 0; t.simple = true; t.p0 = base; t.step = 0;
-  if (t.nrows > 0 && t.row_bytes > 0) {
-    const int off = (int)(base & 15);
-    const int vpr = (off + t.row_bytes + 15) >> 4;
-    if (vpr > THREADS) { t.simple = false; return; }
-    const int rps = THREADS / vpr, r0 = gt / vpr, v0 = gt - r0 * vpr;
-    if (t.nrows > rps * K) { t.simple = false; return; }
-    if (r0 < rps && r0 < t.nrows) {
-      const int rel = 16 * v0 - off;
-      const int lo = rel < 0 ? -rel : 0;
-      const int e = t.row_bytes - rel;
-      const int hi = e < 16 ? e : 16;
-      const int ph = (rel + 15) % 3;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const uint32_t m = byte_mask(lo - 4 * j, hi - 4 * j);
-        t.cT[j] = m & 0x01010101u;
-        t.cG[j] = m & sel_word((ph + 2) % 3, j);
-        t.cB[j] = m & sel_word(ph, j);
-      }
-      t.p0 = base - off + (uintptr_t)((long long)r0 * a.row_stride + 16 * v0);
-      t.step = (long long)rps * a.row_stride;
-      t.nslots = (t.nrows - r0 + rps - 1) / rps;
-    }
-  }
-}
-
-// One turn of the pipeline: issue the tile after `t` into the other stage, wait for `t`, reduce and emit it.
-// CUR is a compile-time stage index so that both tiles stay in registers.
-template <int THREADS, int K, bool WANT_SUMS, int CUR>
-__device__ __forceinline__ bool roi_pipeline_turn(const RoiArgs& a, PTile& t, PTile& n, unsigned int* __restrict__ work,
-                                                  long long* s_claim, unsigned long long (*part)[THREADS / 32][3],
-                                                  uint32_t slot0, unsigned long long pol) {
-  constexpr int WARPS = THREADS / 32;
-  constexpr uint32_t STAGE_BYTES = THREADS * K * 16;
-  const int gt = threadIdx.x, wid = gt >> 5, lane = gt & 31;
-  const long long rn = s_claim[CUR ^ 1];
-  const bool have_next = rn < a.num_rois;
-  unsigned int claim = 0xffffffffu;
-  if (gt == 0 && have_next) claim = atomicAdd(work, 1u);          // the ROI after next; published before the barrier below
-  const uint32_t sb_next = slot0 + (uint32_t)(CUR ^ 1) * STAGE_BYTES, sb_cur = slot0 + (uint32_t)CUR * STAGE_BYTES;
-  if (have_next) {
-    ptile_setup<THREADS, K>(n, a, rn, gt);
-#pragma unroll
-    for (int u = 0; u < K; ++u)
-      if (u < n.nslots) cp_async16_64B(sb_next + (uint32_t)(u * THREADS * 16), reinterpret_cast<const void*>(n.p0 + u * n.step), pol);
-    cp_async_commit();
-    cp_async_wait_group<1>();
-  } else {
-    cp_async_wait_group<0>();
-  }
-  uint32_t sG = 0, sT = 0, sB = 0;
-  if (t.simple) {
-#pragma unroll
-    for (int u = 0; u < K; ++u) {
-      if (u < t.nslots) {
-        const uint4 d = lds128(sb_cur + (uint32_t)(u * THREADS * 16));
-        sT = __dp4a(d.x, t.cT[0], __dp4a(d.y, t.cT[1], __dp4a(d.z, t.cT[2], __dp4a(d.w, t.cT[3], sT))));
-        sG = __dp4a(d.x, t.cG[0], __dp4a(d.y, t.cG[1], __dp4a(d.z, t.cG[2], __dp4a(d.w, t.cG[3], sG))));
-        if (WANT_SUMS)
-          sB = __dp4a(d.x, t.cB[0], __dp4a(d.y, t.cB[1], __dp4a(d.z, t.cB[2], __dp4a(d.w, t.cB[3], sB))));
-      }
-    }
-  } else {
-    // a tile larger than one stage: round by round through this stage's slots (waits for everything in flight)
-    const uintptr_t base = t.p0;
-    const int off = (int)(base & 15);
-    const int vpr = (off + t.row_bytes + 15) >> 4;
-    int rps, r0, v0;
-    if (vpr >= THREADS) { rps = 1; r0 = 0; v0 = gt; }
-    else { rps = THREADS / vpr; r0 = gt / vpr; v0 = gt - r0 * vpr; if (r0 >= rps) v0 = vpr; }
-    const long long step = (long long)rps * a.row_stride;
-    for (int v = v0; v < vpr; v += THREADS) {
-      const int rel = 16 * v - off;
-      const int lo = rel < 0 ? -rel : 0;
-      const int e = t.row_bytes - rel;
-      const int hi = e < 16 ? e : 16;
-      const int ph = (rel + 15) % 3;
-      uint32_t cT[4], cG[4], cB[4];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const uint32_t m = byte_mask(lo - 4 * j, hi - 4 * j);
-        cT[j] = m & 0x01010101u;
-        cG[j] = m & sel_word((ph + 2) % 3, j);
-        cB[j] = m & sel_word(ph, j);
-      }
-      const uint8_t* p = reinterpret_cast<const uint8_t*>(base - off) + (long long)r0 * a.row_stride + 16 * v;
-      for (int r = r0; r < t.nrows; r += rps * K) {
-#pragma unroll
-        for (int u = 0; u < K; ++u)
-          if (r + u * rps < t.nrows) cp_async16_64B(sb_cur + (uint32_t)(u * THREADS * 16), p + u * step, pol);
-        cp_async_commit();
-        cp_async_wait_group<0>();
-#pragma unroll
-        for (int u = 0; u < K; ++u) {
-          if (r + u * rps < t.nrows) {
-            const uint4 d = lds128(sb_cur + (uint32_t)(u * THREADS * 16));
-            sT = __dp4a(d.x, cT[0], __dp4a(d.y, cT[1], __dp4a(d.z, cT[2], __dp4a(d.w, cT[3], sT))));
-            sG = __dp4a(d.x, cG[0], __dp4a(d.y, cG[1], __dp4a(d.z, cG[2], __dp4a(d.w, cG[3], sG))));
-            if (WANT_SUMS)
-              sB = __dp4a(d.x, cB[0], __dp4a(d.y, cB[1], __dp4a(d.z, cB[2], __dp4a(d.w, cB[3], sB))));
-          }
-        }
-        p += K * step;
-      }
-    }
-  }
-  const unsigned long long N = (unsigned long long)(t.nrows > 0 ? t.nrows : 0) * (unsigned long long)(t.ncols > 0 ? t.ncols : 0);
-  unsigned long long tG, tT, tB = 0;
-  if (N < 5600000ull) {
-    tG = warp_sum<uint32_t>(sG); tT = warp_sum<uint32_t>(sT);
-    if (WANT_SUMS) tB = warp_sum<uint32_t>(sB);
-  } else {
-    tG = warp_sum_u64(sG); tT = warp_sum_u64(sT);
-    if (WANT_SUMS) tB = warp_sum_u64(sB);
-  }
-  if (lane == 0) { part[CUR][wid][0] = tG; part[CUR][wid][1] = tT; part[CUR][wid][2] = tB; }
-  if (gt == 0) s_claim[CUR] = have_next ? (long long)claim : a.num_rois;   // everyone holds t.roi in registers by now
-  __syncthreads();
-  if (gt == 0) {
-    tG = tT = tB = 0;
-#pragma unroll
-    for (int w = 0; w < WARPS; ++w) { tG += part[CUR][w][0]; tT += part[CUR][w][1]; tB += part[CUR][w][2]; }
-    if (WANT_SUMS) {
-      ulonglong4 o; o.x = tB; o.y = tG; o.z = tT - tG - tB; o.w = N;
-      *reinterpret_cast<ulonglong4*>(a.out_sums + 4 * t.roi) = o;
-    }
-    double val;
-    if (!t.has_box || N == 0) val = nan_f64();
-    else if (a.mode == BPV_GREEN) val = (double)tG / (double)N;
-    else val = (double)(3 * (long long)tG - (long long)tT + 2 * (long long)N) / (double)(4 * N);
-    a.out_value[t.roi] = val;
-  }
-  return have_next;
-}
-
-template <int THREADS, int K, bool WANT_SUMS>
-__global__ void __launch_bounds__(THREADS, 4) roi_pipelined_kernel(const RoiArgs a, unsigned int* __restrict__ work) {
-  extern __shared__ __align__(128) uint8_t stage[];
-  __shared__ long long s_claim[2];
-  __shared__ unsigned long long part[2][THREADS / 32][3];
-  const int gt = threadIdx.x;
-  const unsigned long long pol = l2_evict_first_policy();
-  const uint32_t slot0 = smem_u32(stage) + 16u * (uint32_t)gt;
-  if (gt == 0) {
-    s_claim[0] = (long long)atomicAdd(work, 1u);
-    s_claim[1] = (long long)atomicAdd(work, 1u);
-  }
-  __syncthreads();
-  PTile T0, T1;
-  if (s_claim[0] < a.num_rois) {
-    ptile_setup<THREADS, K>(T0, a, s_claim[0], gt);
-#pragma unroll
-    for (int u = 0; u < K; ++u)
-      if (u < T0.nslots) cp_async16_64B(slot0 + (uint32_t)(u * THREADS * 16), reinterpret_cast<const void*>(T0.p0 + u * T0.step), pol);
-    cp_async_commit();
-    for (;;) {
-      if (!roi_pipeline_turn<THREADS, K, WANT_SUMS, 0>(a, T0, T1, work, s_claim, part, slot0, pol)) break;
-      if (!roi_pipeline_turn<THREADS, K, WANT_SUMS, 1>(a, T1, T0, work, s_claim, part, slot0, pol)) break;
-    }
-  }
-  if (gt == 0) {
-    __threadfence();
-    if (atomicAdd(work + 1, 1u) == gridDim.x - 1) { work[0] = 0u; work[1] = 0u; __threadfence(); }   // last CTA out: ready for the next launch
-  }
-}
-
-// work counters of the persistent kernel: a small ring so that launches in flight on different streams never share one
-constexpr int ROI_WORK_SLOTS = 64;
-__device__ unsigned int g_roi_work[ROI_WORK_SLOTS][2];
-
-template <int THREADS, int K>
-static int launch_pipelined(const RoiArgs& a, cudaStream_t st) {
-  static unsigned next_slot = 0;
-  static int sms = 0;
-  if (sms == 0) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (sms <= 0) sms = 148;
-  }
-  unsigned int* work = nullptr;
-  cudaError_t e = cudaGetSymbolAddress((void**)&work, g_roi_work);
-  if (e != cudaSuccess) { set_error("bpv_roi_sample_u8: cudaGetSymbolAddress: %s", cudaGetErrorString(e)); return (int)e; }
-  work += 2 * (next_slot++ % ROI_WORK_SLOTS);
-  const int smem = 2 * THREADS * K * 16;
-  auto k1 = roi_pipelined_kernel<THREADS, K, true>;
-  auto k0 = roi_pipelined_kernel<THREADS, K, false>;
-  (void)ensure_dyn_smem((const void*)k1, smem, true);
-  (void)ensure_dyn_smem((const void*)k0, smem, true);
-  long long grid = (long long)sms * 4;
-  if (grid > a.num_rois) grid = a.num_rois;
-  if (a.out_sums) k1<<<(unsigned)grid, THREADS, smem, st>>>(a, work);
-  else k0<<<(unsigned)grid, THREADS, smem, st>>>(a, work);
-  return 0;
-}
-
-#endif  // BPV_ROI_TUNING
-
-template <int THREADS, int K, int STAGE>
-static void launch_staged(const RoiArgs& a, int stage_bytes, cudaStream_t st) {
-  const int smem = STAGE == 1 ? THREADS * K * 16 : stage_bytes;
-  auto k1 = roi_staged_kernel<THREADS, K, true, STAGE>;
-  auto k0 = roi_staged_kernel<THREADS, K, false, STAGE>;
+static void launch_staged(const RoiArgs& a, cudaStream_t st) {
+  const int smem = THREADS * K * 16;
+  auto k1 = roi_staged_kernel<THREADS, K, true>;
+  auto k0 = roi_staged_kernel<THREADS, K, false>;
   // a failed opt-in is not fatal here: the launch below then fails and check_launch() reports it
   (void)ensure_dyn_smem((const void*)k1, 200 * 1024, true);
   (void)ensure_dyn_smem((const void*)k0, 200 * 1024, true);
-  if (a.out_sums) k1<<<(unsigned)a.num_rois, THREADS, smem, st>>>(a, stage_bytes);
-  else k0<<<(unsigned)a.num_rois, THREADS, smem, st>>>(a, stage_bytes);
+  if (a.out_sums) k1<<<(unsigned)a.num_rois, THREADS, smem, st>>>(a);
+  else k0<<<(unsigned)a.num_rois, THREADS, smem, st>>>(a);
 }
 
-template <int GROUP, int LDMODE>
+template <int GROUP, bool HOST>
 static void launch_rows(const RoiArgs& a, unsigned grid, cudaStream_t st) {
-  // LDMODE 5 = ld.global.nc.L1::no_allocate.L2::64B: the default L2 fill granule on B200 is the whole
+  // Device frames: ld.global.nc.L1::no_allocate.L2::64B: the default L2 fill granule on B200 is the whole
   // 128-byte line; asking for 64 B cuts the DRAM over-fetch around short unaligned ROI rows from 1.50x
   // to 1.17x of the algorithmic bytes (ncu dram__bytes_read, profiles/r1a_roi_l2_fill_probe.txt).
-  // LDMODE 2 = plain ld.global, for frames in pinned HOST memory: over PCIe the 128-byte requests move
+  // HOST: plain ld.global, for frames in pinned host memory: over PCIe the 128-byte requests move
   // 32.8 GB/s of ROI bytes (49 GB/s on the wire) against 19.9 GB/s with 64-byte requests
   // (profiles/r1e_roi_host_variants.txt).
   // Host frames are PCIe-bound (one 256-thread CTA per SM already keeps 2.4 MB of reads in flight): an unused dynamic
   // shared-memory request caps the kernel at one CTA per SM, so the window pipeline of the previous batch can run
   // beside it on another stream instead of queueing behind a machine-filling F1 grid.
   size_t smem = 0;
-  if (LDMODE == 2) {
+  if (HOST) {
     smem = 120 * 1024;
-    (void)ensure_dyn_smem((const void*)roi_rows_kernel<GROUP, 4, true, LDMODE, 4>, smem);
-    (void)ensure_dyn_smem((const void*)roi_rows_kernel<GROUP, 4, false, LDMODE, 4>, smem);
+    (void)ensure_dyn_smem((const void*)roi_rows_kernel<GROUP, true, HOST>, smem);
+    (void)ensure_dyn_smem((const void*)roi_rows_kernel<GROUP, false, HOST>, smem);
   }
-  if (a.out_sums) roi_rows_kernel<GROUP, 4, true, LDMODE, 4><<<grid, 256, smem, st>>>(a);
-  else roi_rows_kernel<GROUP, 4, false, LDMODE, 4><<<grid, 256, smem, st>>>(a);
+  if (a.out_sums) roi_rows_kernel<GROUP, true, HOST><<<grid, 256, smem, st>>>(a);
+  else roi_rows_kernel<GROUP, false, HOST><<<grid, 256, smem, st>>>(a);
 }
-
-// Tuning variants (register path load modes / unroll / occupancy, cp.async staging depth and CTA size, cp.async.bulk
-// rows) are compiled only with -DBPV_ROI_TUNING and selected with BPV_ROI_VARIANT (tools/roi_variants.sh produced
-// profiles/r1d_roi_variants.txt, r1e_roi_variants.txt, r1e_roi_host_variants.txt with them); the product library
-// contains only the paths it dispatches to.
-#ifdef BPV_ROI_TUNING
-static bool launch_variant(const RoiArgs& a, unsigned grid, cudaStream_t st) {
-  static const char* v = getenv("BPV_ROI_VARIANT");
-  if (!v) return false;
-  if (a.out_sums && v[0] < 'A') return false;
-  const unsigned grid128 = (unsigned)((a.num_rois + 1) / 2); (void)grid;
-#define V(ld, un, mb) if (v[0] == '0' + ld && v[1] == '0' + un && v[2] == '0' + mb) { roi_rows_kernel<128, un, false, ld, mb><<<grid128, 256, 0, st>>>(a); return true; }
-  V(0, 4, 3) V(0, 4, 4) V(0, 8, 3) V(0, 8, 4) V(0, 2, 4) V(0, 2, 6)
-  V(1, 4, 4) V(2, 4, 4) V(3, 4, 4) V(4, 4, 4) V(5, 4, 3) V(5, 8, 4) V(5, 2, 6) V(5, 2, 8) V(5, 4, 6)
-#define SA(tag, thr, k) if (v[0] == tag && atoi(v + 1) == k) { launch_staged<thr, k, 1>(a, 0, st); return true; }
-  SA('A', 128, 8) SA('A', 128, 10) SA('A', 128, 11) SA('A', 128, 12) SA('F', 96, 12) SA('F', 96, 14) SA('G', 64, 8) SA('H', 32, 12) SA('H', 32, 24) SA('A', 128, 16) SA('C', 256, 4) SA('C', 256, 6) SA('C', 256, 8) SA('G', 64, 12) SA('G', 64, 24)
-#undef SA
-  if (v[0] == 'B') { launch_staged<128, 1, 2>(a, atoi(v + 1) * 1024, st); return true; }
-  if (v[0] == 'D') { launch_staged<256, 1, 2>(a, atoi(v + 1) * 1024, st); return true; }
-  if (v[0] == 'E') { launch_staged<64, 1, 2>(a, atoi(v + 1) * 1024, st); return true; }
-#undef V
-  return false;
-}
-#else
-static inline bool launch_variant(const RoiArgs&, unsigned, cudaStream_t) { return false; }
-#endif
 
 // ---------------------------------------------------------------------------------------------
 // F1 on NV12 frames (SURVEY.md 8f row 2): decoders (NVDEC, V4L2) hand out NV12 — a full-resolution Y plane followed
@@ -782,11 +451,10 @@ __device__ __forceinline__ int sat_u8(int v) {
   return r;
 }
 
-// VEC: the frame base and the pitch are 16-byte aligned, so the 16 Y bytes and the 16 UV bytes (8 chroma pairs) of a
-// 16-pixel group are ONE 128-bit load each (the byte-load version issued 32 loads per group); ALL = false (GREEN without
-// sums): only the green channel is converted.  Thread layout as the BGR kernels: rows x 16-pixel vector columns, so a
-// thread's column — and with it the mask of its pixels that lie inside [xs, xe) — is loop invariant.
-template <bool WANT_SUMS, bool VEC, bool ALL>
+// Byte loads, for planes that are not 16-byte aligned (aligned ones go to roi_nv12_vec_kernel below); ALL = false (GREEN
+// without sums): only the green channel is converted.  Thread layout as the BGR kernels: rows x 16-pixel vector columns, so
+// a thread's column — and with it the mask of its pixels that lie inside [xs, xe) — is loop invariant.
+template <bool WANT_SUMS, bool ALL>
 __global__ void __launch_bounds__(128) roi_nv12_kernel(const uint8_t* __restrict__ frames, long long frame_stride, long long pitch,
                                                        int H, int W, int R, int mode, long long num_rois,
                                                        const int32_t* __restrict__ boxes,
@@ -823,28 +491,17 @@ __global__ void __launch_bounds__(128) roi_nv12_kernel(const uint8_t* __restrict
         const uint8_t* yrow = yp + (long long)(2 * cy) * pitch + xv;
         const uint8_t* uvrow = uvp + (long long)cy * pitch + xv;
         uint32_t yw[2][4], cw[4];
-        if (VEC) {
-          // whole aligned vectors: bytes beyond the row's last pixel lie inside the pitch (pitch % 16 == 0)
-          const uint4 c4 = ld_stream_v4(uvrow);
-          uint4 a4 = make_uint4(0, 0, 0, 0), b4 = make_uint4(0, 0, 0, 0);
-          if (row_on[0]) a4 = ld_stream_v4(yrow);
-          if (row_on[1]) b4 = ld_stream_v4(yrow + pitch);
-          yw[0][0] = a4.x; yw[0][1] = a4.y; yw[0][2] = a4.z; yw[0][3] = a4.w;
-          yw[1][0] = b4.x; yw[1][1] = b4.y; yw[1][2] = b4.z; yw[1][3] = b4.w;
-          cw[0] = c4.x; cw[1] = c4.y; cw[2] = c4.z; cw[3] = c4.w;
-        } else {
 #pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            yw[0][j] = yw[1][j] = cw[j] = 0;
+        for (int j = 0; j < 4; ++j) {
+          yw[0][j] = yw[1][j] = cw[j] = 0;
 #pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const int e = 4 * j + k;
-              if (inm >> e & 1) {
-                if (row_on[0]) yw[0][j] |= (uint32_t)yrow[e] << (8 * k);
-                if (row_on[1]) yw[1][j] |= (uint32_t)yrow[pitch + e] << (8 * k);
-              }
-              if (inm >> (e & ~1) & 3) cw[j] |= (uint32_t)uvrow[e] << (8 * k);   // a pair's U and V when either pixel is in range
+          for (int k = 0; k < 4; ++k) {
+            const int e = 4 * j + k;
+            if (inm >> e & 1) {
+              if (row_on[0]) yw[0][j] |= (uint32_t)yrow[e] << (8 * k);
+              if (row_on[1]) yw[1][j] |= (uint32_t)yrow[pitch + e] << (8 * k);
             }
+            if (inm >> (e & ~1) & 3) cw[j] |= (uint32_t)uvrow[e] << (8 * k);   // a pair's U and V when either pixel is in range
           }
         }
         // (a predicate-free copy of this body for interior vectors was measured: 217 us against 144 us per 8192 frames —
@@ -1331,20 +988,18 @@ extern "C" int bpv_roi_sample_nv12(const uint8_t* frames, int64_t frame_stride_b
   // 128-bit loads need aligned rows; the Y plane of frame f starts at f * frame_stride and the UV plane H * pitch later
   const bool vec = (((uintptr_t)frames | (uintptr_t)frame_stride_bytes | (uintptr_t)pitch_bytes) & 15) == 0;
   const bool all = mode != BPV_GREEN;
-#define BPV_NV12(S, V, A) roi_nv12_kernel<S, V, A><<<(unsigned)n, 128, 0, st>>>(frames, frame_stride_bytes, pitch_bytes, H, W, R, mode, n, boxes, \
-                                                                              (unsigned long long*)out_sums, out_value)
+#define BPV_NV12(S, A) roi_nv12_kernel<S, A><<<(unsigned)n, 128, 0, st>>>(frames, frame_stride_bytes, pitch_bytes, H, W, R, mode, n, boxes, \
+                                                                        (unsigned long long*)out_sums, out_value)
 #define BPV_NV12V(S, A) roi_nv12_vec_kernel<S, A><<<(unsigned)n, 128, 0, st>>>(frames, frame_stride_bytes, pitch_bytes, H, W, R, mode, n, boxes, \
                                                                              (unsigned long long*)out_sums, out_value)
-  // BPV_NV12_OLD=1: the per-pixel-predicate kernel on aligned planes too (measurement switch)
-  static const bool old_body = [] { const char* e = getenv("BPV_NV12_OLD"); return e && e[0] == '1'; }();
-  if (vec && !old_body) {
+  if (vec) {
     if (out_sums) BPV_NV12V(true, true);
     else if (all) BPV_NV12V(false, true);
     else BPV_NV12V(false, false);
   }
-  else if (out_sums) { if (vec) BPV_NV12(true, true, true); else BPV_NV12(true, false, true); }
-  else if (all) { if (vec) BPV_NV12(false, true, true); else BPV_NV12(false, false, true); }
-  else { if (vec) BPV_NV12(false, true, false); else BPV_NV12(false, false, false); }
+  else if (out_sums) BPV_NV12(true, true);
+  else if (all) BPV_NV12(false, true);
+  else BPV_NV12(false, false);
 #undef BPV_NV12
 #undef BPV_NV12V
   return check_launch("bpv_roi_sample_nv12");
@@ -1376,13 +1031,12 @@ extern "C" int bpv_roi_sample_resized_u8(const uint8_t* frames, int64_t frame_st
                                                                 (unsigned long long*)out_sums, out_value);                   \
   } while (0)
   // staged variant: aligned frames, bilinear case (the exact 2x decimation keeps the byte-load kernel), and a stage that holds
-  // the two source rows of one output row at the frame's full width.  BPV_RESIZE_OLD=1: measurement switch.
-  static const bool old_body = [] { const char* e = getenv("BPV_RESIZE_OLD"); return e && e[0] == '1'; }();
+  // the two source rows of one output row at the frame's full width
   const bool aligned = (((uintptr_t)frames | (uintptr_t)frame_stride_bytes | (uintptr_t)row_stride_bytes) & 15) == 0;
   const bool area2 = src_w == 2 * dst_w && src_h == 2 * dst_h;
   const int smem2 = 26 * 1024;                                        // 8 CTAs per SM
   const long long rowslot = ((3ll * src_w + 15) & ~15ll) + 32;
-  if (aligned && !area2 && !old_body && 2 * rowslot + (long long)dst_h * (long long)sizeof(RowTap4) <= smem2) {
+  if (aligned && !area2 && 2 * rowslot + (long long)dst_h * (long long)sizeof(RowTap4) <= smem2) {
 #define BPV_RSZ2(S, A)                                                                                                      \
   do {                                                                                                                      \
     if (int rc = ensure_dyn_smem((const void*)roi_resized_staged_kernel<S, A>, smem2)) return rc;                            \
@@ -1404,13 +1058,6 @@ extern "C" int bpv_roi_sample_resized_u8(const uint8_t* frames, int64_t frame_st
 #undef BPV_RSZ
   return check_launch("bpv_roi_sample_resized_u8");
 }
-
-#ifdef BPV_ROI_TUNING
-static bool roi_pipelined_enabled() {
-  const char* v = getenv("BPV_ROI_PIPELINED");
-  return v ? v[0] == '1' : false;
-}
-#endif
 
 extern "C" int bpv_roi_sample_u8(const uint8_t* frames, const uint8_t* const* frame_ptrs,
                                  int64_t frame_stride_bytes, int64_t row_stride_bytes,
@@ -1448,16 +1095,12 @@ extern "C" int bpv_roi_sample_u8(const uint8_t* frames, const uint8_t* const* fr
     // shared memory by cp.async (whole ROI in flight; measured 64.5 us vs 76.3 us for the register path on the
     // config-2 boxes, 6.2 TB/s on 320x160 boxes; profiles/r1e_roi_variants.txt).  Frames in pinned host memory
     // (zero-copy e2e path) are PCIe-bound and want full-line requests: register path with plain loads.
-    if (launch_variant(a, grid, st)) {}
-    else if (host_frames) {
-      if (g == 32) launch_rows<32, 2>(a, grid, st);
-      else launch_rows<128, 2>(a, (unsigned)((n + 1) / 2), st);
+    if (host_frames) {
+      if (g == 32) launch_rows<32, true>(a, grid, st);
+      else launch_rows<128, true>(a, (unsigned)((n + 1) / 2), st);
     }
-    else if (g == 32) launch_rows<32, 5>(a, grid, st);
-#ifdef BPV_ROI_TUNING
-    else if (roi_pipelined_enabled()) { if (int rc = launch_pipelined<128, 12>(a, st)) return rc; }
-#endif
-    else launch_staged<128, 12, 1>(a, 0, st);
+    else if (g == 32) launch_rows<32, false>(a, grid, st);
+    else launch_staged<128, 12>(a, st);
   } else {                           // generic path: alignment changes row by row
     if (g == 32) roi_sample_kernel<32, 4><<<grid, 256, 0, st>>>(a);
     else if (g == 128) roi_sample_kernel<128, 4><<<grid, 256, 0, st>>>(a);

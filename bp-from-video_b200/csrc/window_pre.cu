@@ -47,8 +47,7 @@ struct DesignRef {
 struct PreLayout {        // per-warp shared-memory plan, in bytes
   int yv, xv, posv, posb, buf0, buf1, coef, total;
   int buf_len;            // doubles in buf0
-  // FIR sub-plan inside buf0 (doubles): merged path  XT [0, fir_c) | c [fir_c, fir_c + Kmax) (only when the taps are staged in
-  // shared memory: always, but for pre_layout's taps_global)
+  // FIR sub-plan inside buf0 (doubles): merged path  XT [0, fir_c) | c [fir_c, fir_c + Kmax)
   //                                     two-pass path XT [0, fir_gt) | GT [fir_gt, fir_b)
   int fir_c, fir_gt, fir_b;
 };
@@ -65,7 +64,7 @@ __host__ __device__ inline int fir_ld_bwd(int n, int T) { return (round_up(T, 10
 __host__ __device__ inline int fir_merged_k(int T, int RT) { return round_up(2 * T - 1, RT); }
 __host__ __device__ inline int fir_merged_ld(int n, int T, int RT) { return (fir_merged_k(T, RT) / RT + (n + RT - 1) / RT) | 1; }
 
-__host__ __device__ inline PreLayout pre_layout(const bpv_window_params& p, bool taps_global = false) {
+__host__ __device__ inline PreLayout pre_layout(const bpv_window_params& p) {
   bool interp = false, cubic = false, butter = false, fir = false;
   for (int i = 0; i < p.num_methods; ++i) {
     const int m = p.methods[i];
@@ -90,7 +89,7 @@ __host__ __device__ inline PreLayout pre_layout(const bpv_window_params& p, bool
       const int x8 = 8 * fir_merged_ld(W, T, 8), x10 = 10 * fir_merged_ld(W, T, 10);
       L.fir_c = ((x8 > x10 ? x8 : x10) + 1) & ~1;                    // even: c[] 16-byte aligned inside buf0
       const int k8 = fir_merged_k(T, 8), k10 = fir_merged_k(T, 10);
-      const int m = L.fir_c + (taps_global ? 0 : (k8 > k10 ? k8 : k10));
+      const int m = L.fir_c + (k8 > k10 ? k8 : k10);
       if (m > need) need = m;
     }
     if (need > L.buf_len) L.buf_len = need;
@@ -644,10 +643,11 @@ __device__ void fir_filtfilt(Warp& w, const double* __restrict__ taps_g, int T) 
 // makes a 300-sample window ONE round of 30 lanes, RT = 8 a 250-sample window one round of 32.
 // LDC / KC: the operand buffer's leading dimension and the padded tap count as compile-time constants for the common
 // (taps, window) pairs (corr_tile.cuh); the leading dimension is the launch's (window length W), not the signal's.
-// CS = true (default): the merged taps — ready-made by the design kernel, c[k] = ac[|k - M|], zero padded — are copied into
-// the warp's shared-memory slice first; false (measurement switch BPV_FIR_TAPS_GLOBAL=1): the tiles read them from global
-// memory (warp-uniform loads), the plan is 2 KB smaller per warp; measured slower, see bpv_window_filter.
-template <int RT, int LDC = 0, int KC = 0, bool CS = true>
+// The merged taps — ready-made by the design kernel, c[k] = ac[|k - M|], zero padded — are copied into the warp's
+// shared-memory slice first.  (Tiles reading them from global memory, 2 KB less shared memory per warp, were measured
+// slower: 323 against 306 us per 32 768 signals, profiles/r4a — the ring gather streams through L1 and pushes the taps
+// out, so the tile loop opens its blocks with L2 round trips.)
+template <int RT, int LDC = 0, int KC = 0>
 __device__ void fir_merged(Warp& w, const double* __restrict__ c_g, int T) {
   const int M = T - 1;
   const int K = KC ? KC : fir_merged_k(T, RT);
@@ -656,12 +656,8 @@ __device__ void fir_merged(Warp& w, const double* __restrict__ c_g, int T) {
   const int tiles = (n + RT - 1) / RT;
   const int LD = LDC ? LDC : fir_merged_ld(w.W, T, RT);
   double* XT = w.buf0;              // X[j] = ext[j + xbase], de-interleaved by RT; output m sits at j = m + K
-  const double* c = c_g;            // c[k] = ac[|k - M|], k = 0 .. 2M; zero up to FIR_MERGED_LEN >= K
-  if (CS) {
-    double* cs = w.buf0 + w.fir_c;
-    for (int k = w.lane; k < K; k += 32) cs[k] = c_g[k];
-    c = cs;
-  }
+  double* c = w.buf0 + w.fir_c;     // c[k] = ac[|k - M|], k = 0 .. 2M; zero up to FIR_MERGED_LEN >= K
+  for (int k = w.lane; k < K; k += 32) c[k] = c_g[k];
   const int xbase = p + M - K;
   const double y_first = w.yv[0], y_last = w.yv[n - 1];
   // odd extension (scipy.signal._arraytools.odd_ext): head 2*y[0] - y[p-i], body y[i-p], tail 2*y[n-1] - y[2n-2+p-i];
@@ -694,7 +690,6 @@ __device__ void fir_merged(Warp& w, const double* __restrict__ c_g, int T) {
   __syncwarp();
 }
 
-template <bool CS>
 __device__ __forceinline__ void fir_apply(Warp& w, const double* __restrict__ tg, int T) {
   const int n = w.n;
   if (n >= T) {
@@ -703,12 +698,12 @@ __device__ __forceinline__ void fir_apply(Warp& w, const double* __restrict__ tg
     const int c10 = ((n + 9) / 10 + 31) / 32 * 10 * fir_merged_k(T, 10);
     const bool t127 = T == 127;                       // the reference's default filter (fir_taps = 127): K = 260 / 256
     if (c10 < c8) {
-      if (t127 && w.W == 300) fir_merged<10, 57, 260, CS>(w, tg + 256, T);       // fir_merged_ld(300, 127, 10)
-      else fir_merged<10, 0, 0, CS>(w, tg + 256, T);
+      if (t127 && w.W == 300) fir_merged<10, 57, 260>(w, tg + 256, T);       // fir_merged_ld(300, 127, 10)
+      else fir_merged<10, 0, 0>(w, tg + 256, T);
     } else {
-      if (t127 && w.W == 300) fir_merged<8, 71, 256, CS>(w, tg + 256, T);        // fir_merged_ld(300, 127, 8)
-      else if (t127 && w.W == 250) fir_merged<8, 65, 256, CS>(w, tg + 256, T);   // fir_merged_ld(250, 127, 8)
-      else fir_merged<8, 0, 0, CS>(w, tg + 256, T);
+      if (t127 && w.W == 300) fir_merged<8, 71, 256>(w, tg + 256, T);        // fir_merged_ld(300, 127, 8)
+      else if (t127 && w.W == 250) fir_merged<8, 65, 256>(w, tg + 256, T);   // fir_merged_ld(250, 127, 8)
+      else fir_merged<8, 0, 0>(w, tg + 256, T);
     }
   } else {
     fir_filtfilt(w, tg, T);
@@ -719,7 +714,6 @@ __device__ __forceinline__ void fir_apply(Warp& w, const double* __restrict__ tg
 // FEAT = which of the heavy stages this instantiation contains (register budget and code size follow the method list):
 // bit 0 INTERP_*, bit 1 FILTER_BUTTER, bit 2 FILTER_FIR.  diff / detrend are always present.
 constexpr int F_INTERP = 1, F_BUTTER = 2, F_FIR = 4;
-constexpr int F_TAPS_GLOBAL = 8;    // with F_FIR: merged taps read from global memory (fir_merged CS = false), needs pre_layout(p, true)
 
 // isfinite(fs) for fs = 1 / ((x_last - x_first) / (m - 1)), the guard of signal_processor.py:200 (Signal.get_fs,
 // signal_data.py:55-58), m >= 2.  For every spacing a clock can produce the quotient is far from the overflow / underflow
@@ -839,7 +833,7 @@ __device__ int apply_method(Warp& w, int method, const bpv_window_params& p, con
       if (FEAT & F_FIR) {
         const double* tg = dr.fir(job);
         if (!isfinite(tg[0])) return ST_BAD_BANDS;
-        fir_apply<(FEAT & F_TAPS_GLOBAL) == 0>(w, tg, p.fir_taps);
+        fir_apply(w, tg, p.fir_taps);
       }
       break;
     default: break;
@@ -1054,13 +1048,8 @@ static int window_filter(const double* ring_t, const double* ring_y, const bpv_w
   dr.taps_ws = ws ? (const double*)(ws + wp.fir) : nullptr;
   dr.ref = (ws && cache && (butter || fir)) ? (const int32_t*)(ws + wp.ref) : nullptr;
   dr.cache = (const unsigned char*)cache;
-  // BPV_FIR_TAPS_GLOBAL=1 (measurement switch): the FIR-only pipeline with the merged taps read from global memory by the
-  // tiles — 2 KB less shared memory per warp, an 80-register instantiation, 25 instead of 21 warps per SM.  Measured slower
-  // (profiles/r4a: 323 against 306 us per 32 768 signals): the ring gather streams through L1 and pushes the taps out, so
-  // the tile loop opens its blocks with L2 round trips.  Default: taps staged in shared memory per signal, 96 registers.
-  static const bool taps_global = [] { const char* e = getenv("BPV_FIR_TAPS_GLOBAL"); return e && e[0] == '1'; }();
   const bool fir_only = !interp && !butter && fir;
-  const PreLayout L = pre_layout(*p, fir_only && taps_global);
+  const PreLayout L = pre_layout(*p);
   cudaStream_t st = (cudaStream_t)stream;
 #define BPV_PRE(feat, minb, dual) return launch_preprocess<feat, minb, dual>(ring_t, ring_y, *p, L, dr, proc_x, proc_y, status, st, jm)
   // Two signals per warp pay off while enough warps stay resident to hide the stages that run for one signal after the
@@ -1069,7 +1058,6 @@ static int window_filter(const double* ring_t, const double* ring_y, const bpv_w
   // 3.57 ms against 2.86 ms per step), so large plans keep one signal per warp.  BPV_SOS_SINGLE = test switch.
   const bool single_sos = getenv("BPV_SOS_SINGLE") != nullptr || (227 * 1024) / (2 * L.total + 1024) < 8;
   if (!interp && !butter && !fir) BPV_PRE(0, 6, false);
-  if (fir_only && taps_global) BPV_PRE(F_FIR | F_TAPS_GLOBAL, 6, false);
   if (fir_only) BPV_PRE(F_FIR, 5, false);
   if (single_sos) {
     if (!interp && !fir) BPV_PRE(F_BUTTER, 4, false);

@@ -224,9 +224,7 @@ extern "C" int bpv_window_xcorr_band(const double* proc_x, const double* proc_y,
   const long long n = (long long)p->S * p->jobs_per_stream * P;
   BPV_REQUIRE(W > 0 && n > 0, BPV_E_INVALID, "bpv_window_xcorr: bad sizes");
   {  // warp-per-pair kernel whenever one pair fits the shared memory of a CTA
-    // BPV_XC_ONE=0 (measurement switch): coarse values through the cv[] array in shared memory, as before round 2's last change
-    static const bool force_cv = [] { const char* e = getenv("BPV_XC_ONE"); return e && e[0] == '0'; }();
-    const XwLayout Lw = xw_layout(W, force_cv);
+    const XwLayout Lw = xw_layout(W);
     int wpb = (200 * 1024) / Lw.total;
     if (wpb > 4) wpb = 4;
     if (wpb >= 1) {
@@ -245,7 +243,6 @@ extern "C" int bpv_window_xcorr_band(const double* proc_x, const double* proc_y,
   } while (0)
       if (Lw.LD == 63 && Lw.one_round) BPV_XW(63, true);      // windows of 291..300 samples (the 10 s window at 30 fps)
       else if (Lw.LD == 53 && Lw.one_round) BPV_XW(53, true); // 241..250 (the reference's default signal_max_samples)
-      else if (Lw.LD == 63) BPV_XW(63, false);
       else if (Lw.one_round) BPV_XW(0, true);
       else BPV_XW(0, false);
 #undef BPV_XW

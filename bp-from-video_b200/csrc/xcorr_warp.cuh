@@ -19,14 +19,14 @@ constexpr float XC_DELTA = 2.0e-4f;   // candidate band below the fp32 maximum (
 // ---------------------------------------------------------------------------------------------
 constexpr int XW_RT = 10;
 struct XwLayout { int b64, pos, cv, c, xt, total, K, LD, one_round; };
-__host__ __device__ inline XwLayout xw_layout(int W, bool force_cv = false) {
+__host__ __device__ inline XwLayout xw_layout(int W) {
   XwLayout L;
   L.K = (W + XW_RT - 1) / XW_RT * XW_RT;                 // taps, padded to the tile
   L.LD = (2 * (L.K / XW_RT) + 2) | 1;                    // columns of the de-interleaved periodic operand (odd: no bank conflicts)
   int o = W * 8;
   L.b64 = o; o += W * 8;
   L.pos = o; o += (W * 2 + 15) / 16 * 16;
-  L.one_round = !force_cv && L.K / XW_RT <= 32;                       // every lane owns at most one tile: coarse values stay in registers
+  L.one_round = L.K / XW_RT <= 32;                       // every lane owns at most one tile: coarse values stay in registers
   L.cv = o; o += L.one_round ? 0 : 2 * W * 4;
   L.c = o; o += L.K * 4;
   L.xt = o; o += XW_RT * L.LD * 4;

@@ -383,14 +383,6 @@ int bpv_pack_records32(const double* peak_freq, const double* lag_sec, const int
                        int64_t J, int32_t R, int32_t P, int32_t* out, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
- * Scratch hygiene (no reference counterpart: the reference's intermediate arrays die in the CPU cache).  Drops the
- * 128-byte L2 lines that lie entirely inside [ptr, ptr + bytes) WITHOUT writing them back to DRAM (discard.global.L2);
- * the contents of the range are undefined afterwards.  The engine calls it on the processed windows once F3 and F4 have
- * consumed them, so that ~80 MB of dead dirty lines per step do not compete with the next step's ROI sampling for DRAM.
- */
-int bpv_scratch_discard(void* ptr, int64_t bytes, void* stream);
-
-/* ---------------------------------------------------------------------------------------------
  * Tensor-core building block of the spectra: 256-point DFT of `rows` real segments as one dense contraction on the
  * 5th-generation tensor cores (tcgen05.mma kind::tf32 with hi/lo split operands, fp32 accumulators in TMEM) — the
  * transform inside scipy.signal.welch(y, fs) as the reference calls it (signal_processor.py:260, nperseg = 256).

@@ -202,34 +202,6 @@ def test_overlapped_schedules_equal_the_serial_one(methods, transform):
         assert all(_same(x, y) for x, y in zip(outs[0], outs[ov])), ov
 
 
-def test_scratch_discard_changes_no_result():
-    """bpv_scratch_discard (include/bpv.h) drops the dead window scratch from L2 after F3 / F4: a run with it equals a run
-    without it bit for bit, full and partial steps; and the entry point rejects bad arguments."""
-    from bpv import synth, ops, _cabi
-    S, T, H, W = 4, 3, 48, 64
-    rng = np.random.default_rng(22)
-    frames = torch.from_numpy(rng.integers(0, 256, (S, T, H, W, 3), dtype=np.uint8)).cuda()
-    boxes = torch.from_numpy(np.stack([synth.roi_boxes(rng, T, H, W) for _ in range(S)])).cuda()
-    outs = []
-    for discard in (False, True):
-        eng = _engine(S, 40, T, processing_methods=[orc.DETREND_LINEAR, orc.FILTER_FIR], spectrum_transform=orc.PGRAM_WELCH)
-        eng.discard_scratch = discard
-        run = []
-        for k in range(14):
-            Tn = T if k % 5 else T - 1                                   # a partial step takes the two-launch form
-            ts = torch.from_numpy(np.tile((np.arange(Tn) + 1 + k * T) / 30.0, (S, 1))).cuda()
-            run.append(_snap(eng.step(frames.roll(k, dims=1)[:, :Tn].contiguous(), boxes[:, :Tn].contiguous(), ts)))
-        torch.cuda.synchronize()
-        outs.append(run)
-    assert all(_same(x, y) for x, y in zip(outs[0], outs[1]))
-    buf = torch.ones(1000, dtype=torch.float64, device='cuda')
-    ops.scratch_discard(buf[3:900])                                      # unaligned range: only whole 128-byte lines inside it
-    torch.cuda.synchronize()
-    assert float(buf[:3].sum()) == 3.0 and float(buf[900:].sum()) == 100.0
-    assert _cabi.lib().bpv_scratch_discard(None, 16, None) == -1
-    assert _cabi.lib().bpv_scratch_discard(None, 0, None) == 0
-
-
 def test_split_design_and_filter_equal_preprocess():
     from tests.test_window_gpu import make_windows, to_ring, params
     from bpv import ops, _cabi

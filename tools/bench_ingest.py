@@ -55,6 +55,6 @@ ok = b720[..., 0] != synth.NO_BOX
 b720[ok] = np.rint(b720[ok] * (dw / W)).astype(np.int32)
 b720_d = torch.from_numpy(b720).cuda()
 t = timeit(lambda: ops.roi_sample_resized(bgr, dh, dw, b720_d, 1))
-print(f'resized  {N} frames (1080p -> 720p boxes): {t*1e3:8.1f} us  {N/t*1e3/1e6:6.2f} M frames/s  = {t/t_bgr:.2f} x the BGR kernel per frame  (variant {os.environ.get("BPV_RESIZE_VARIANT", "default")})')
+print(f'resized  {N} frames (1080p -> 720p boxes): {t*1e3:8.1f} us  {N/t*1e3/1e6:6.2f} M frames/s  = {t/t_bgr:.2f} x the BGR kernel per frame')
 t = timeit(lambda: ops.roi_sample_resized(bgr, dh, dw, b720_d, 0))
 print(f'resized GREEN {N} frames: {t*1e3:8.1f} us  = {t/t_bgr:.2f} x the BGR kernel per frame')
